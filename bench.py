@@ -25,6 +25,9 @@ chain per GPU (weak scaling, no data-path collective: "replicas only", as parall
           the 120 (frequency, mode) systems sharded over the N GPUs, one ncclAllReduce of [gradient | misfit] per step issued by
           the library on its own stream) with its own value / e2e / roofline / clocks, so that the driver's 1/2/4/8-GPU runs hold
           a strong-scaling curve next to the weak-scaling one.   `--config cfg4` prints that record as the main line instead.
+`--dump-outputs DIR` : after the run, the chain state the last timed step of the main line left on the device (what
+          hmcmt_get_state hands a caller of hmcmt_leapfrog_steps_device), rank 0's, as DIR/model.npy and DIR/momentum.npy (float64,
+          [chains, active cells]).  The inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -472,11 +475,11 @@ def run_cfg2(args, D, local_rank):
                                 final_state_device_vs_host_rel=final_diff, steps_compared=W + K,
                                 observations="forward(true model) x (1 + 0.05 N), err = 0.05 |Z| (SURVEY.md 8d)"))
     pl.close()
-    return line
+    return line, dict(model=m_dev, momentum=p_dev)
 
 
-def run_cfg4(args, D, local_rank, nfreq=0):
-    """Strong scaling: one chain of the cfg4 workload, its (frequency, mode) systems sharded over the ranks."""
+def run_cfg4(args, D, local_rank, K, nfreq=0):
+    """Strong scaling: one chain of the cfg4 workload, its (frequency, mode) systems sharded over the ranks, K timed steps."""
     from hmcmt2d_b200 import api, synthetic
     rank, world = D.rank, D.world
     cfg = dict(CFG4)
@@ -489,7 +492,7 @@ def run_cfg4(args, D, local_rank, nfreq=0):
     m0 = synthetic.stress_model(inv, seed=1)                                   # the same chain state on every rank
     p0 = np.clip(np.random.default_rng(100).standard_normal(len(m0)), -2.5, 2.5)
     dt = prior.dt
-    K, W = max(3, min(args.steps, 10)), 3
+    W = 3
 
     sampler = ClockSampler(local_rank)
     sampler.start()
@@ -544,7 +547,7 @@ def run_cfg4(args, D, local_rank, nfreq=0):
                 gpu_launches=int(launches), clocks=clocks, roofline=roofline, validated=validated,
                 validation=dict(device_status=int(status), states_finite=finite, observations="analytic half-space + 5 % noise"))
     sp.close()
-    return line
+    return line, dict(model=m_end, momentum=p_end)
 
 
 def main():
@@ -557,7 +560,10 @@ def main():
     ap.add_argument("--no-strong-scaling", action="store_true", help="skip the cfg4 record appended to the cfg2 line")
     ap.add_argument("--config", default="cfg2", choices=["cfg2", "cfg4"])
     ap.add_argument("--nfreq", type=int, default=0, help="cfg4 only: reduced number of frequencies (testing)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the chain state left by the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -570,15 +576,17 @@ def main():
                "--master-port", "29511", os.path.abspath(__file__), "--gpus", str(args.gpus), "--steps", str(args.steps),
                "--warmup", str(args.warmup), "--config", args.config, "--nfreq", str(args.nfreq)]
         cmd += ["--no-strong-scaling"] if args.no_strong_scaling else []
+        cmd += ["--dump-outputs", args.dump_outputs] if args.dump_outputs else []
         raise SystemExit(subprocess.call(cmd))
     D = Dist(rank, world, local_rank)
     if args.config == "cfg4":
-        line = run_cfg4(args, D, local_rank, args.nfreq)
+        line, outputs = run_cfg4(args, D, local_rank, args.steps, args.nfreq)
     else:
-        line = run_cfg2(args, D, local_rank)
+        line, outputs = run_cfg2(args, D, local_rank)
         if not args.no_strong_scaling:
             try:
-                line["strong_scaling"] = run_cfg4(args, D, local_rank, args.nfreq)
+                # a short record next to the headline: 3 to 10 timed steps whatever --steps says
+                line["strong_scaling"] = run_cfg4(args, D, local_rank, max(3, min(args.steps, 10)), args.nfreq)[0]
             except Exception as e:                                   # never lose the headline line to the second workload
                 line["strong_scaling"] = dict(error=repr(e))
     if rank == 0 and world == 1 and not args.no_cpu_baseline:
@@ -588,6 +596,10 @@ def main():
                                     sample=f"1 of {cfg['nfreq']} frequencies (TE+TM forward+adjoint, {wall1:.2f} s) on one host core, "
                                            f"multiplied by {cfg['nfreq']}; restated CPU path (oracle, SciPy SuperLU symmetric-mode MMD), not MUMPS. "
                                            f"All-core figure: `bench.py --impl reference` ({os.cpu_count()} cores on this box)")
+    if rank == 0 and args.dump_outputs:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in outputs.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), np.ascontiguousarray(a, dtype=np.float64))
     if rank == 0:
         print(json.dumps(line), flush=True)
     D.close()

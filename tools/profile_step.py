@@ -1,6 +1,7 @@
 """Short driver for ncu: a couple of device-resident leapfrog steps of the cfg2 workload."""
+import os
 import sys
-sys.path.insert(0, '/root/repo')
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np
 from hmcmt2d_b200 import api, synthetic
 ny, nz, nf = (int(a) for a in sys.argv[1:4]) if len(sys.argv) > 3 else (200, 100, 30)

@@ -127,29 +127,42 @@ def readstartupFile(startupfile: str):
 # plan management
 
 
+# DataComp of "Rho_Pha" surveys, in the row order of MT2DFwdSolver.jl:191-205, and the modes they select
+_RHO_PHA_COMPS = {("RhoXY", "PhsXY"): [0], ("RhoYX", "PhsYX"): [1], ("RhoXY", "PhsXY", "RhoYX", "PhsYX"): [0, 1]}
+
+
 class Plan:
-    """Owns one `hmcmt_plan` (device-resident problem: mesh, survey, weights, factors, chain state)."""
+    """Owns one `hmcmt_plan` (device-resident problem: mesh, survey, weights, factors, chain state).
+    DataType "Impedance": packed data arrays are complex.  DataType "Rho_Pha": one real apparent resistivity or phase per row
+    (dtID = 2 mode + 1 / 2), and every packed data array (predictions, J^T v input, Jacobian rows, chain samples) is real."""
 
     def __init__(self, mtMesh: TensorMesh2D, mtData: MTData, invParam: InvDataModel, hmcprior: HMCPrior,
                  nChains: int = 1, device: int = 0):
-        if "Impedance" not in mtData.dataType:
-            raise NotImplementedError("only DataType Impedance reaches the gradient in the reference "
-                                      "('Rho_Pha' vs 'Rho_Phs', compJacTMatVec.jl:104)")
+        self.rho_phase = "Rho_Pha" in mtData.dataType
+        if not self.rho_phase and "Impedance" not in mtData.dataType:
+            raise NotImplementedError(f"DataType {mtData.dataType}")
         self.L = _lib.load()
         self.generation = 0
         ny, nz = mtMesh.gridSize
         self.ny, self.nz = int(ny), int(nz)
         self.nChains = int(nChains)
-        comp_mode = []
-        for c in mtData.dataComp:
-            if "XY" in c:
-                comp_mode.append(0)
-            elif "YX" in c:
-                comp_mode.append(1)
-            else:
-                raise NotImplementedError(f"data component {c}")
-        if comp_mode not in ([0], [1], [0, 1]):
-            raise ValueError("DataComp must be [ZXY, ZYX] in that order (MT2DFwdSolver.jl:183-187)")
+        self.dtype = np.float64 if self.rho_phase else np.complex128
+        if self.rho_phase:
+            comp_mode = _RHO_PHA_COMPS.get(tuple(mtData.dataComp))
+            if comp_mode is None:
+                raise ValueError("DataComp must be [RhoXY, PhsXY, RhoYX, PhsYX] in that order, or the two of one mode "
+                                 "(MT2DFwdSolver.jl:191-205)")
+        else:
+            comp_mode = []
+            for c in mtData.dataComp:
+                if "XY" in c:
+                    comp_mode.append(0)
+                elif "YX" in c:
+                    comp_mode.append(1)
+                else:
+                    raise NotImplementedError(f"data component {c}")
+            if comp_mode not in ([0], [1], [0, 1]):
+                raise ValueError("DataComp must be [ZXY, ZYX] in that order (MT2DFwdSolver.jl:183-187)")
         act = np.asarray(invParam.activeCell.tocsc().indices, dtype=np.int32)      # one row index per column
         Wm = invParam.Wm.tocsr()
         Wm.sort_indices()
@@ -158,7 +171,7 @@ class Plan:
             freqs=np.ascontiguousarray(mtData.freqs, dtype=np.float64), rx=np.ascontiguousarray(mtData.rxLoc, dtype=np.float64),
             comp=np.asarray(comp_mode, dtype=np.int32), fid=np.ascontiguousarray(mtData.freqID, dtype=np.int64),
             rid=np.ascontiguousarray(mtData.rxID, dtype=np.int64), did=np.ascontiguousarray(mtData.dtID, dtype=np.int64),
-            obs=np.ascontiguousarray(invParam.obsData, dtype=np.complex128),
+            obs=np.ascontiguousarray(invParam.obsData, dtype=self.dtype),
             err=np.ascontiguousarray(1.0 / invParam.dataW, dtype=np.float64), act=act,
             bg=np.ascontiguousarray(invParam.bgModel, dtype=np.float64),
             wp=np.ascontiguousarray(Wm.indptr, dtype=np.int32), wi=np.ascontiguousarray(Wm.indices, dtype=np.int32),
@@ -181,7 +194,8 @@ class Plan:
         pr.sigBounds[0], pr.sigBounds[1] = float(hmcprior.sigBounds[0]), float(hmcprior.sigBounds[1])
         pr.nChains, pr.device = self.nChains, int(device)
         h = C.c_void_p()
-        _lib.check(self.L.hmcmt_plan_create(C.byref(pr), C.byref(h)), "hmcmt_plan_create")
+        create = self.L.hmcmt_plan_create_rho_phase if self.rho_phase else self.L.hmcmt_plan_create
+        _lib.check(create(C.byref(pr), C.byref(h)), "hmcmt_plan_create")
         self.h = h
         self.nAC, self.nData, self.nFreq = len(act), pr.nData, pr.nFreq
         self.nNode = (self.ny + 1) * (self.nz + 1)
@@ -209,7 +223,7 @@ class Plan:
 
     def forward(self, m=None, sigma=None, fields=True):
         self.generation = getattr(self, "generation", 0) + 1       # MT2DFwdData handles of earlier evaluations become stale
-        pred = np.zeros((self.nChains, self.nData), dtype=np.complex128)
+        pred = np.zeros((self.nChains, self.nData), dtype=self.dtype)
         ex = np.zeros((self.nChains, self.nFreq, self.nNode), dtype=np.complex128) if (fields and self.compTE) else None
         hx = np.zeros((self.nChains, self.nFreq, self.nNode), dtype=np.complex128) if (fields and self.compTM) else None
         cp = lambda a: a.ctypes.data_as(C.POINTER(C.c_double)) if a is not None else None
@@ -222,14 +236,16 @@ class Plan:
         return pred, ex, hx
 
     def jtvec(self, v):
-        v = np.ascontiguousarray(v, dtype=np.complex128).reshape(self.nChains, self.nData)
+        """real(J^T conj(v)) w.r.t. the active-cell conductivities for the last forward evaluation (real v, J^T v, for Rho_Pha)."""
+        v = np.ascontiguousarray(v, dtype=self.dtype).reshape(self.nChains, self.nData)
         g = np.zeros((self.nChains, self.nAC))
         _lib.check(self.L.hmcmt_jtvec(self.h, v.ctypes.data_as(C.POINTER(C.c_double)), _lib.f64(g)), "hmcmt_jtvec")
         return g
 
     def jacobian(self):
-        """Explicit Jacobian dZ/dsigma_active of the last forward evaluation: [nChains, nData, nAC] complex."""
-        J = np.zeros((self.nChains, self.nData, self.nAC), dtype=np.complex128)
+        """Explicit Jacobian d pred / d sigma_active of the last forward evaluation: [nChains, nData, nAC], complex dZ/dsigma
+        (Impedance) or real d rho_a / d sigma, d phase / d sigma rows (Rho_Pha)."""
+        J = np.zeros((self.nChains, self.nData, self.nAC), dtype=self.dtype)
         _lib.check(self.L.hmcmt_jacobian(self.h, J.ctypes.data_as(C.POINTER(C.c_double))), "hmcmt_jacobian")
         return J
 
@@ -238,7 +254,7 @@ class Plan:
         model-norm part beta Wm (m - m_ref) on the device (m_ref from set_state), as proposeLeapfrog does right afterwards."""
         self.generation = getattr(self, "generation", 0) + 1
         mm = self._m(m)
-        pred = np.zeros((self.nChains, self.nData), dtype=np.complex128)
+        pred = np.zeros((self.nChains, self.nData), dtype=self.dtype)
         phi = np.zeros(self.nChains)
         g = np.zeros((self.nChains, self.nAC))
         fn = self.L.hmcmt_forward_gradient_total if total else self.L.hmcmt_forward_gradient
@@ -259,7 +275,7 @@ class Plan:
     def leapfrog_trajectory(self, dt, intstep, want_pred=True):
         L = np.ascontiguousarray(np.broadcast_to(np.asarray(intstep, dtype=np.int32), (self.nChains,)))
         stats = np.zeros((self.nChains, 4))
-        pred = np.zeros((self.nChains, self.nData), dtype=np.complex128) if want_pred else None
+        pred = np.zeros((self.nChains, self.nData), dtype=self.dtype) if want_pred else None
         _lib.check(self.L.hmcmt_leapfrog_trajectory(self.h, float(dt), _lib.i32(L), _lib.f64(stats),
                                                     None if pred is None else pred.ctypes.data_as(C.POINTER(C.c_double))),
                    "hmcmt_leapfrog_trajectory")
@@ -303,7 +319,7 @@ class Plan:
         model = np.zeros((nc, nsamples, self.nAC))
         stats = np.zeros((nc, nsamples + 1, 4))
         acc = np.zeros((nc, nsamples), dtype=np.int32)
-        data = np.zeros((nc, nsamples + 1, self.nData), dtype=np.complex128)
+        data = np.zeros((nc, nsamples + 1, self.nData), dtype=self.dtype)
         ms = None if m_start is None else np.ascontiguousarray(m_start, dtype=np.float64).reshape(nc, self.nAC)
         _lib.check(self.L.hmcmt_run_chain(self.h, float(dt), int(nsamples), float(rhoref), None if ms is None else _lib.f64(ms),
                                           _lib.f64(z_init), _lib.i32(intsteps),
@@ -373,7 +389,9 @@ def shard_systems(mtData: MTData, invParam: InvDataModel, rank: int, world: int)
     the ranks takes the TE systems and the second half the TM systems, frequencies round-robin inside each half (120 systems
     over 8 ranks = 15 each at cfg4, instead of 8 / 7 frequencies x 2 modes).  Otherwise falls back to `shard_frequencies`.
     -> (MTData of this rank, InvDataModel with its observation rows, `rows` = their positions in the full data vector)."""
-    two_modes = bool(mtData.compTE and mtData.compTM) and len(mtData.dataComp) == 2
+    # rows per mode: one impedance component, or the rho_a and phase rows of a "Rho_Pha" survey (dtID = 2 mode + 1 / 2)
+    per_mode = 2 if "Rho_Pha" in mtData.dataType else 1
+    two_modes = bool(mtData.compTE and mtData.compTM) and len(mtData.dataComp) == 2 * per_mode
     if world < 2 or world % 2 or not two_modes:
         return shard_frequencies(mtData, invParam, rank, world)
     half = world // 2
@@ -385,11 +403,12 @@ def shard_systems(mtData: MTData, invParam: InvDataModel, rank: int, world: int)
     newid = np.zeros(nF + 1, dtype=np.int64)
     newid[mine + 1] = np.arange(1, len(mine) + 1)
     fid, did = np.asarray(mtData.freqID), np.asarray(mtData.dtID)
-    rows = np.nonzero((newid[fid] > 0) & (did == mode + 1))[0]
+    comps = slice(mode * per_mode, (mode + 1) * per_mode)
+    rows = np.nonzero((newid[fid] > 0) & ((did - 1) // per_mode == mode))[0]
     nRx, nDt = np.asarray(mtData.rxLoc).shape[0], len(mtData.dataComp)
-    mask = np.asarray(mtData.dataID, dtype=bool).reshape(nF, nRx, nDt)[mine][:, :, mode].reshape(-1)
-    sub = MTData(np.array(mtData.rxLoc), np.array(mtData.freqs)[mine], mtData.dataType, [mtData.dataComp[mode]],
-                 np.asarray(mtData.rxID)[rows], newid[fid[rows]], np.ones(len(rows), dtype=np.int64), mask, mode == 0, mode == 1)
+    mask = np.asarray(mtData.dataID, dtype=bool).reshape(nF, nRx, nDt)[mine][:, :, comps].reshape(-1)
+    sub = MTData(np.array(mtData.rxLoc), np.array(mtData.freqs)[mine], mtData.dataType, list(mtData.dataComp[comps]),
+                 np.asarray(mtData.rxID)[rows], newid[fid[rows]], did[rows] - mode * per_mode, mask, mode == 0, mode == 1)
     dataW = np.asarray(invParam.dataW)[rows]
     inv = InvDataModel(np.asarray(invParam.obsData)[rows], dataW, np.array(invParam.strModel), np.array(invParam.refModel),
                        invParam.activeCell, np.array(invParam.bgModel), invParam.Wm, 1.0 / dataW)
@@ -405,6 +424,7 @@ class FreqShardedPlan:
     def __init__(self, mtMesh, mtData, invParam, hmcprior, rank: int, world: int, device: int = 0, group=None, balance="systems"):
         self.rank, self.world, self.group = int(rank), int(world), group
         self.nDataFull = len(np.asarray(invParam.obsData))
+        self.rho_phase = "Rho_Pha" in mtData.dataType              # real predictions
         shard = shard_systems if balance == "systems" else shard_frequencies
         sub, inv, self.rows = shard(mtData, invParam, rank, world)
         self.plan = Plan(mtMesh, sub, inv, hmcprior, nChains=1, device=device)
@@ -427,7 +447,7 @@ class FreqShardedPlan:
         import torch
         import torch.distributed as dist
         pred, phi, g = self.plan.forward_gradient(m)
-        full = np.zeros(self.nDataFull, dtype=np.complex128)
+        full = np.zeros(self.nDataFull, dtype=np.float64 if self.rho_phase else np.complex128)
         full[self.rows] = pred[0]
         packed = np.concatenate([g[0], phi, full.view(np.float64)])
         if self.world > 1:
@@ -437,7 +457,8 @@ class FreqShardedPlan:
             dist.all_reduce(t, op=dist.ReduceOp.SUM, group=self.group)
             packed = t.cpu().numpy()
         nAC = self.nAC
-        return packed[nAC + 1:].view(np.complex128), float(packed[nAC]), packed[:nAC]
+        data = packed[nAC + 1:]
+        return (data if self.rho_phase else data.view(np.complex128)), float(packed[nAC]), packed[:nAC]
 
     # device-resident leapfrog steps with one all-reduce per step
     def _exchange_tensor(self):

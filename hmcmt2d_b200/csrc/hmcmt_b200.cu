@@ -68,11 +68,14 @@ struct hmcmt_plan {
     int64_t launches = 0, factorLaunches = 0;
     bool haveForward = false, haveSens = false, sigmaDirect = false, useMf = false, timeFactor = false;
     int respKind = 0;                               // 0 impedance, 1 apparent resistivity / phase (forward only)
+    int dataKind = 0;                               // data of the plan: 0 impedance, 1 apparent resistivity / phase (rows real)
     // host copies
     std::vector<double> h_yLen, h_zLen, h_freqs;
-    std::vector<int> h_packed2full;      // [nData] full index (without chain) of each packed datum
+    std::vector<int> h_packed2full;      // [nData] full index (without chain) of each packed datum; rho / phase plans: index into
+                                         // the real view [nFull][2] (rho, phase) of the full arrays
     // device buffers
     DevBuf<double> yLen, zLen, zNode, freqs, fdy1, fdy2, wL, wR, bg, wmVal, wd, m, p, mref, sigma, meanSig, planes;
+    DevBuf<double> wdPha;                           // phase weights of a rho / phase plan (wd holds the rho weights)
     DevBuf<double> driftPart;                       // block maxima of the drift (k_drift_max)
     DevBuf<double> xbuf, Gpart, phiPart, phi, gsig, gdata, gtotal, energies, panels, curM, curP, chainScal, zmom;
     DevBuf<int> fid, iL, iR, cell2act, act2cell, wmPtr, wmIdx, status, driftFlag, packed2full, full2packed, Lsteps;
@@ -253,6 +256,12 @@ __global__ void k_pack_pred(int nData, int nFull, const int* __restrict__ packed
     int i = blockIdx.x * blockDim.x + threadIdx.x, ch = blockIdx.y;
     if (i < nData) out[(size_t)ch * nData + i] = predFull[(size_t)ch * nFull + packed2full[i]];
 }
+// rho / phase plans: the packed real data from the (rho_a, phase) pairs of respFull, viewed as [nChains][2 nFull] doubles
+__global__ void k_pack_pred_real(int nData, int nFull, const int* __restrict__ packed2full, const double* __restrict__ respFull,
+                                 double* __restrict__ out) {
+    int i = blockIdx.x * blockDim.x + threadIdx.x, ch = blockIdx.y;
+    if (i < nData) out[(size_t)ch * nData + i] = respFull[(size_t)ch * 2 * nFull + packed2full[i]];
+}
 __global__ void k_kick_masked(int nAC, double dt, int kstep, const int* __restrict__ L, const double* __restrict__ grad,
                               double* __restrict__ p) {
     int ch = blockIdx.y, a = blockIdx.x * blockDim.x + threadIdx.x;
@@ -273,11 +282,13 @@ __global__ void k_clip_momentum(int nAC, const double* __restrict__ z, double* _
     p[(size_t)ch * nAC + a] = v;
 }
 // Metropolis accept on the device (HMCSampler.jl:149-186).  chainScal[ch] = {startD, startM, startK, startH}
+// DT: element type of the packed data (cplx impedances, double for rho / phase plans)
+template <typename DT>
 __global__ void __launch_bounds__(kHmcThreads)
 k_accept(int nAC, int nData, int it, int nsamples, const double* __restrict__ uacc, const double* __restrict__ phi,
          const double* __restrict__ energies, const double* __restrict__ znew, double* __restrict__ m, double* __restrict__ p,
-         double* __restrict__ curM, double* __restrict__ chainScal, const cplx* __restrict__ predPacked,
-         double* __restrict__ hmcmodel, double* __restrict__ hmstats, int* __restrict__ accept, cplx* __restrict__ hmcdata) {
+         double* __restrict__ curM, double* __restrict__ chainScal, const DT* __restrict__ predPacked,
+         double* __restrict__ hmcmodel, double* __restrict__ hmstats, int* __restrict__ accept, DT* __restrict__ hmcdata) {
     __shared__ double sh[32];
     __shared__ int accSh;
     const int ch = blockIdx.x;
@@ -308,9 +319,9 @@ k_accept(int nAC, int nData, int it, int nsamples, const double* __restrict__ ua
         k += z * z;
     }
     k = block_reduce(k, false, sh);
-    cplx* dout = hmcdata + ((size_t)ch * (nsamples + 1) + it) * nData;
-    const cplx* dprev = dout - nData;
-    const cplx* dnew = predPacked + (size_t)ch * nData;
+    DT* dout = hmcdata + ((size_t)ch * (nsamples + 1) + it) * nData;
+    const DT* dprev = dout - nData;
+    const DT* dnew = predPacked + (size_t)ch * nData;
     for (int i = threadIdx.x; i < nData; i += blockDim.x) dout[i] = acc ? dnew[i] : dprev[i];
     if (threadIdx.x == 0) {
         sc[2] = 0.5 * k;
@@ -360,6 +371,19 @@ __global__ void k_jac_rows(int nAC, int nCell, int nFreq, int nRx, int nModes, i
     const int d = full2packed[(f * nRx + r) * nModes + mi];
     if (d < 0) return;
     J[(((size_t)ch * nData + d) * nAC + a) * 2 + part] = Gpart[(size_t)sys * nCell + act2cell[a]];
+}
+
+// rho / phase plans: v = e_d carries v_rho = 1 (part 0) or v_phi = 1 (part 1), the real rows d rho_a / d sigma and
+// d phase / d sigma of the datum, J [nChains][nData][nAC] doubles; full2packed indexes the real view [nFull][2]
+__global__ void k_jac_rows_real(int nAC, int nCell, int nFreq, int nRx, int nModes, int nData, int r, int part,
+                                const int* __restrict__ act2cell, const int* __restrict__ full2packed, const double* __restrict__ Gpart,
+                                double* __restrict__ J) {
+    const int a = blockIdx.x * blockDim.x + threadIdx.x, sys = blockIdx.y;
+    if (a >= nAC) return;
+    const int f = sys % nFreq, t = sys / nFreq, mi = t % nModes, ch = t / nModes;
+    const int d = full2packed[2 * ((f * nRx + r) * nModes + mi) + part];
+    if (d < 0) return;
+    J[((size_t)ch * nData + d) * nAC + a] = Gpart[(size_t)sys * nCell + act2cell[a]];
 }
 
 int ensure_pin(hmcmt_plan* pl, size_t bytes) {
@@ -507,9 +531,10 @@ int rx_range(hmcmt_plan* pl, const SysRange& r, bool wantAdjoint, const cplx* vi
     const MeshDev& M = pl->M;
     size_t rxSmem = (size_t)(6 * (M.ny + 1) + 3 * M.ny) * sizeof(cplx);
     if (wantAdjoint) HMCMT_CUDA_TRY(cudaMemsetAsync(pl->lam.p + (size_t)r.s0 * M.N, 0, sizeof(cplx) * (size_t)r.n * M.N, r.st));
-    k_rx_adjoint<<<r.n, kRxThreads, rxSmem, r.st>>>(M, pl->rx, pl->sm, pl->freqs.p, pl->sigma.p, pl->F.p, pl->obs.p, pl->wd.p, vin,
-                                                    pl->predFull.p, pl->phiPart.p, pl->srows.p, pl->qrow.p, pl->lam.p, wantAdjoint ? 1 : 0,
-                                                    pl->respKind, pl->respFull.p, r.s0);
+    auto kern = pl->dataKind ? k_rx_adjoint<true> : k_rx_adjoint<false>;
+    kern<<<r.n, kRxThreads, rxSmem, r.st>>>(M, pl->rx, pl->sm, pl->freqs.p, pl->sigma.p, pl->F.p, pl->obs.p, pl->wd.p, pl->wdPha.p, vin,
+                                            pl->predFull.p, pl->phiPart.p, pl->srows.p, pl->qrow.p, pl->lam.p, wantAdjoint ? 1 : 0,
+                                            pl->respKind, pl->respFull.p, r.s0);
     LAUNCH_CHECK(pl);
     return kOk;
 }
@@ -648,7 +673,8 @@ int compute_step_graph(hmcmt_plan* pl) {
 //   forward (all chains x modes x freqs) [+ adjoint gradient + prior gradient].
 int compute_step(hmcmt_plan* pl, bool wantAdjoint, const cplx* vin) {
     if (wantAdjoint && !vin && !pl->timeFactor) {
-        // the graph holds the standard evaluation (sigma = exp(m), impedance responses); anything else is launched eagerly
+        // the graph holds the standard evaluation (sigma = exp(m), the plan's own data type); the forward-only response toggle and
+        // direct conductivities are launched eagerly
         const bool standard = !pl->sigmaDirect && pl->respKind == 0;
         return pl->graphState >= 0 && standard ? compute_step_graph(pl) : compute_step_eager(pl);
     }
@@ -777,7 +803,8 @@ extern "C" {
 
 const char* hmcmt_version(void) { return "hmcmt_b200 0.1 (sm_100a; DMMA.8x8x4 tile-window band LDL^T; no CPU fallback)"; }
 
-int hmcmt_plan_create(const hmcmt_problem* pr, hmcmt_plan** out) {
+// dataKind 0: impedance data (hmcmt_plan_create), 1: apparent resistivity / phase rows (hmcmt_plan_create_rho_phase)
+static int plan_create(const hmcmt_problem* pr, hmcmt_plan** out, int dataKind) {
     if (!pr || !out) return kErrArg;
     *out = nullptr;
     int ndev = 0;
@@ -796,7 +823,7 @@ int hmcmt_plan_create(const hmcmt_problem* pr, hmcmt_plan** out) {
         if (cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, pr->device) == cudaSuccess && nsm > 0) pl->numSMs = nsm;
     }
     pl->ny = pr->ny; pl->nz = pr->nz; pl->nFreq = pr->nFreq; pl->nRx = pr->nRx; pl->nData = pr->nData; pl->nAC = pr->nAC;
-    pl->nChains = pr->nChains; pl->nComp = pr->nComp; pl->nModes = pr->nComp;
+    pl->nChains = pr->nChains; pl->nComp = pr->nComp; pl->nModes = pr->nComp; pl->dataKind = dataKind;
     for (int c = 0; c < pr->nComp; ++c) pl->modeList[c] = pr->compMode[c];
     pl->beta = pr->regParam;
     pl->lo = std::log(pr->sigBounds[0]);
@@ -860,15 +887,20 @@ int hmcmt_plan_create(const hmcmt_problem* pr, hmcmt_plan** out) {
         fid[r] = id; d1[r] = y - yNode[id - 1]; d2[r] = yNode[id] - y;
         linear_interp(y, yNode, iL[r], iR[r], wL[r], wR[r]);
     }
-    // data layout: full index ((f*nRx + r)*nModes + mi), rows must be sorted (freq, rx, comp)
-    std::vector<double> wdFull(pl->nFull, 0.0);
+    // data layout: full slot ((f*nRx + r)*nModes + mi), rows must be sorted (freq, rx, comp).  Rho / phase plans: dtID =
+    // 2 mi + 1 (rho_a) or 2 mi + 2 (phase), real obsData; the slot keeps the observed pair and both weights (0 where a row is absent)
+    // and a packed row maps to 2 slot + part of the real view of the full arrays
+    std::vector<double> wdFull(pl->nFull, 0.0), wpFull(dataKind ? pl->nFull : 0, 0.0);
     std::vector<cplx> obsFull(pl->nFull, mk(0.0, 0.0));
     pl->h_packed2full.resize(pr->nData);
+    const long nDt = dataKind ? 2 * pr->nComp : pr->nComp;
     long prev = -1;
     for (int i = 0; i < pr->nData; ++i) {
         long f = pr->freqID[i] - 1, r = pr->rxID[i] - 1, c = pr->dtID[i] - 1;
-        if (f < 0 || f >= pr->nFreq || r < 0 || r >= pr->nRx || c < 0 || c >= pr->nComp) { delete pl; return kErrArg; }
-        long full = (f * pr->nRx + r) * pl->nModes + c;
+        if (f < 0 || f >= pr->nFreq || r < 0 || r >= pr->nRx || c < 0 || c >= nDt) { delete pl; return kErrArg; }
+        const long mi = dataKind ? c / 2 : c, part = dataKind ? c % 2 : 0;
+        const long slot = (f * pr->nRx + r) * pl->nModes + mi;
+        const long full = dataKind ? 2 * slot + part : slot;
         if (full <= prev) {
             fprintf(stderr, "[hmcmt_b200] data rows must be sorted by (freq, rx, comp) without duplicates\n");
             delete pl;
@@ -876,8 +908,17 @@ int hmcmt_plan_create(const hmcmt_problem* pr, hmcmt_plan** out) {
         }
         prev = full;
         pl->h_packed2full[i] = (int)full;
-        wdFull[full] = 1.0 / std::fabs(pr->dataErr[i]);
-        obsFull[full] = mk(pr->obsData[2 * i], pr->obsData[2 * i + 1]);
+        const double w = 1.0 / std::fabs(pr->dataErr[i]);
+        if (!dataKind) {
+            wdFull[slot] = w;
+            obsFull[slot] = mk(pr->obsData[2 * i], pr->obsData[2 * i + 1]);
+        } else if (part == 0) {
+            wdFull[slot] = w;
+            obsFull[slot].x = pr->obsData[i];
+        } else {
+            wpFull[slot] = w;
+            obsFull[slot].y = pr->obsData[i];
+        }
     }
     std::vector<int> cell2act(M.nCell, -1);
     for (int a = 0; a < pr->nAC; ++a) {
@@ -898,9 +939,10 @@ int hmcmt_plan_create(const hmcmt_problem* pr, hmcmt_plan** out) {
     int nnzWm = pr->wmRowPtr[pr->nAC];
     ok(pl->wmIdx.upload(pr->wmColIdx, nnzWm)); ok(pl->wmVal.upload(pr->wmVal, nnzWm));
     ok(pl->wd.upload(wdFull.data(), pl->nFull)); ok(pl->obs.upload(obsFull.data(), pl->nFull));
+    ok(pl->wdPha.upload(wpFull.data(), wpFull.size()));
     ok(pl->packed2full.upload(pl->h_packed2full.data(), pr->nData));
     {
-        std::vector<int> f2p(pl->nFull, -1);
+        std::vector<int> f2p((dataKind ? 2 : 1) * (size_t)pl->nFull, -1);
         for (int i = 0; i < pr->nData; ++i) f2p[pl->h_packed2full[i]] = i;
         ok(pl->full2packed.upload(f2p.data(), f2p.size()));
     }
@@ -987,7 +1029,8 @@ int hmcmt_plan_create(const hmcmt_problem* pr, hmcmt_plan** out) {
         }
         pl->conStaged = contract_cols_smem(M.ny, M.nz, 1) <= 200 * 1024 ? 1 : 0;
         const size_t cSmem = contract_cols_smem(M.ny, M.nz, pl->conStaged);
-        if ((rxSmem > 48 * 1024 && cudaFuncSetAttribute(k_rx_adjoint, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)rxSmem) != cudaSuccess) ||
+        if ((rxSmem > 48 * 1024 && cudaFuncSetAttribute(dataKind ? k_rx_adjoint<true> : k_rx_adjoint<false>,
+                                                        cudaFuncAttributeMaxDynamicSharedMemorySize, (int)rxSmem) != cudaSuccess) ||
             (cSmem > 48 * 1024 && cudaFuncSetAttribute(k_contract_cols, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cSmem) != cudaSuccess)) {
             hmcmt_destroy(pl);
             return kErrArg;
@@ -1051,6 +1094,9 @@ int hmcmt_plan_create(const hmcmt_problem* pr, hmcmt_plan** out) {
     return kOk;
 }
 
+int hmcmt_plan_create(const hmcmt_problem* pr, hmcmt_plan** out) { return plan_create(pr, out, 0); }
+int hmcmt_plan_create_rho_phase(const hmcmt_problem* pr, hmcmt_plan** out) { return plan_create(pr, out, 1); }
+
 void hmcmt_destroy(hmcmt_plan* pl) {
     if (!pl) return;
     cudaSetDevice(pl->device);
@@ -1073,7 +1119,7 @@ void hmcmt_destroy(hmcmt_plan* pl) {
     for (auto& e : pl->factorEvents) { cudaEventDestroy(e.first); cudaEventDestroy(e.second); }
     for (cudaEvent_t e : pl->factorMid) cudaEventDestroy(e);
     pl->yLen.release(); pl->zLen.release(); pl->zNode.release(); pl->freqs.release(); pl->fdy1.release(); pl->fdy2.release();
-    pl->wL.release(); pl->wR.release(); pl->bg.release(); pl->wmVal.release(); pl->wd.release(); pl->m.release(); pl->p.release();
+    pl->wL.release(); pl->wR.release(); pl->bg.release(); pl->wmVal.release(); pl->wd.release(); pl->wdPha.release(); pl->m.release(); pl->p.release();
     pl->mref.release(); pl->sigma.release(); pl->meanSig.release(); pl->planes.release(); pl->Gpart.release(); pl->phiPart.release();
     pl->phi.release(); pl->gsig.release(); pl->gdata.release(); pl->gtotal.release(); pl->energies.release(); pl->panels.release(); pl->curM.release();
     pl->curP.release(); pl->driftPart.release(); pl->chainScal.release(); pl->zmom.release(); pl->fid.release(); pl->iL.release(); pl->iR.release();
@@ -1201,7 +1247,7 @@ int hmcmt_set_response_kind(hmcmt_plan* pl, int32_t kind) {
 int hmcmt_get_responses(hmcmt_plan* pl, double* out) {
     if (!pl || !out || !pl->haveForward) return kErrArg;
     HMCMT_CUDA_TRY(cudaSetDevice(pl->device));
-    const cplx* src = pl->respKind == 1 ? pl->respFull.p : pl->predFull.p;
+    const cplx* src = (pl->respKind == 1 || pl->dataKind == 1) ? pl->respFull.p : pl->predFull.p;
     HMCMT_CUDA_TRY(cudaMemcpyAsync(out, src, sizeof(cplx) * (size_t)pl->nChains * pl->nFull, cudaMemcpyDeviceToHost, pl->stream));
     HMCMT_CUDA_TRY(cudaStreamSynchronize(pl->stream));
     return kOk;
@@ -1258,11 +1304,23 @@ static int upload_model(hmcmt_plan* pl, const double* m) {
     HMCMT_CUDA_TRY(cudaMemcpyAsync(pl->m.p, pl->pin, bytes, cudaMemcpyHostToDevice, pl->stream));
     return kOk;
 }
-static int download_pred(hmcmt_plan* pl, double* pred) {
-    k_pack_pred<<<dim3((pl->nData + 255) / 256, pl->nChains), 256, 0, pl->stream>>>(pl->nData, pl->nFull, pl->packed2full.p,
-                                                                                    pl->predFull.p, pl->predPacked.p);
+// bytes of one packed datum: complex impedance, or one real rho_a / phase row
+static size_t datum_bytes(const hmcmt_plan* pl) { return pl->dataKind ? sizeof(double) : sizeof(cplx); }
+// predictions of the last evaluation into predPacked [nChains][nData] (complex, or real for rho / phase plans)
+static int pack_pred(hmcmt_plan* pl) {
+    const dim3 grid((pl->nData + 255) / 256, pl->nChains);
+    if (pl->dataKind)
+        k_pack_pred_real<<<grid, 256, 0, pl->stream>>>(pl->nData, pl->nFull, pl->packed2full.p, reinterpret_cast<const double*>(pl->respFull.p),
+                                                       reinterpret_cast<double*>(pl->predPacked.p));
+    else
+        k_pack_pred<<<grid, 256, 0, pl->stream>>>(pl->nData, pl->nFull, pl->packed2full.p, pl->predFull.p, pl->predPacked.p);
     LAUNCH_CHECK(pl);
-    HMCMT_CUDA_TRY(cudaMemcpyAsync(pred, pl->predPacked.p, sizeof(cplx) * (size_t)pl->nChains * pl->nData, cudaMemcpyDeviceToHost, pl->stream));
+    return kOk;
+}
+static int download_pred(hmcmt_plan* pl, double* pred) {
+    int rc = pack_pred(pl);
+    if (rc) return rc;
+    HMCMT_CUDA_TRY(cudaMemcpyAsync(pred, pl->predPacked.p, datum_bytes(pl) * (size_t)pl->nChains * pl->nData, cudaMemcpyDeviceToHost, pl->stream));
     return kOk;
 }
 
@@ -1307,11 +1365,15 @@ int hmcmt_jtvec(hmcmt_plan* pl, const double* v, double* gsig) {
     if (!pl || !v || !gsig) return kErrArg;
     if (!pl->haveForward) return kErrArg;
     HMCMT_CUDA_TRY(cudaSetDevice(pl->device));
-    // scatter the packed data vector into the full layout
+    // scatter the packed data vector into the full layout (rho / phase plans: the real rows into the (v_rho, v_phi) pairs)
     std::vector<cplx> full((size_t)pl->nChains * pl->nFull, mk(0.0, 0.0));
+    double* fullD = reinterpret_cast<double*>(full.data());
     for (int ch = 0; ch < pl->nChains; ++ch)
-        for (int i = 0; i < pl->nData; ++i)
-            full[(size_t)ch * pl->nFull + pl->h_packed2full[i]] = mk(v[2 * ((size_t)ch * pl->nData + i)], v[2 * ((size_t)ch * pl->nData + i) + 1]);
+        for (int i = 0; i < pl->nData; ++i) {
+            const size_t src = (size_t)ch * pl->nData + i;
+            if (pl->dataKind) fullD[(size_t)ch * 2 * pl->nFull + pl->h_packed2full[i]] = v[src];
+            else full[(size_t)ch * pl->nFull + pl->h_packed2full[i]] = mk(v[2 * src], v[2 * src + 1]);
+        }
     HMCMT_CUDA_TRY(cudaMemcpyAsync(pl->vin.p, full.data(), sizeof(cplx) * full.size(), cudaMemcpyHostToDevice, pl->stream));
     HMCMT_CUDA_TRY(cudaStreamSynchronize(pl->stream));
     // the factors, fields and boundary values of the last forward evaluation are still on the device (the reference's AinvTE /
@@ -1333,7 +1395,7 @@ int hmcmt_jacobian(hmcmt_plan* pl, double* J) {
     HMCMT_CUDA_TRY(cudaSetDevice(pl->device));
     const MeshDev& M = pl->M;
     cudaStream_t st = pl->stream;
-    const size_t nJ = (size_t)pl->nChains * pl->nData * pl->nAC * 2;
+    const size_t nJ = (size_t)pl->nChains * pl->nData * pl->nAC * (pl->dataKind ? 1 : 2);
     DevBuf<double> dJ;
     int rc = dJ.alloc(nJ);
     if (rc) return rc;
@@ -1347,8 +1409,13 @@ int hmcmt_jacobian(hmcmt_plan* pl, double* J) {
             rc = rx_phase(pl, true, pl->vin.p);
             if (rc == kOk) rc = adjoint_phase(pl, false);
             if (rc != kOk) break;
-            k_jac_rows<<<dim3((pl->nAC + 255) / 256, pl->nSys), 256, 0, st>>>(pl->nAC, M.nCell, pl->nFreq, pl->nRx, pl->nModes, pl->nData, r, part,
-                                                                             pl->act2cell.p, pl->full2packed.p, pl->Gpart.p, dJ.p);
+            const dim3 grid((pl->nAC + 255) / 256, pl->nSys);
+            if (pl->dataKind)
+                k_jac_rows_real<<<grid, 256, 0, st>>>(pl->nAC, M.nCell, pl->nFreq, pl->nRx, pl->nModes, pl->nData, r, part, pl->act2cell.p,
+                                                      pl->full2packed.p, pl->Gpart.p, dJ.p);
+            else
+                k_jac_rows<<<grid, 256, 0, st>>>(pl->nAC, M.nCell, pl->nFreq, pl->nRx, pl->nModes, pl->nData, r, part, pl->act2cell.p,
+                                                 pl->full2packed.p, pl->Gpart.p, dJ.p);
             ++pl->launches;
         }
     if (rc == kOk && cudaGetLastError() != cudaSuccess) rc = kErrCuda;
@@ -1375,7 +1442,7 @@ static int forward_gradient_impl(hmcmt_plan* pl, const double* m, double* pred, 
     pl->sigmaDirect = false;
     // One pinned staging buffer for everything that crosses the bus: [model up | pred | phi | gradient | error flags down], one
     // stream synchronisation per call (device-to-host copies into pageable caller memory would be staged by the driver one by one).
-    const size_t nM = sizeof(double) * (size_t)pl->nChains * pl->nAC, nP = sizeof(cplx) * (size_t)pl->nChains * pl->nData;
+    const size_t nM = sizeof(double) * (size_t)pl->nChains * pl->nAC, nP = datum_bytes(pl) * (size_t)pl->nChains * pl->nData;
     const size_t nPhi = sizeof(double) * pl->nChains, nS = sizeof(int) * ((size_t)pl->nSys + 1);
     const size_t oP = (nM + 255) & ~(size_t)255, oPhi = oP + ((nP + 255) & ~(size_t)255), oG = oPhi + ((nPhi + 255) & ~(size_t)255);
     const size_t oS = oG + ((nM + 255) & ~(size_t)255), total = oS + nS;
@@ -1387,9 +1454,7 @@ static int forward_gradient_impl(hmcmt_plan* pl, const double* m, double* pred, 
     rc = compute_step(pl, true, nullptr);
     if (rc) return rc;
     if (pred) {
-        k_pack_pred<<<dim3((pl->nData + 255) / 256, pl->nChains), 256, 0, pl->stream>>>(pl->nData, pl->nFull, pl->packed2full.p,
-                                                                                        pl->predFull.p, pl->predPacked.p);
-        LAUNCH_CHECK(pl);
+        if ((rc = pack_pred(pl))) return rc;
         HMCMT_CUDA_TRY(cudaMemcpyAsync(pin + oP, pl->predPacked.p, nP, cudaMemcpyDeviceToHost, pl->stream));
     }
     if (phid) HMCMT_CUDA_TRY(cudaMemcpyAsync(pin + oPhi, pl->phi.p, nPhi, cudaMemcpyDeviceToHost, pl->stream));
@@ -1594,14 +1659,15 @@ int hmcmt_run_chain(hmcmt_plan* pl, double dt, int32_t nsamples, double rhoref, 
     const int chunk = (int)std::max<size_t>(1, std::min<size_t>((size_t)nsamples, ((size_t)64 << 20) / (nState * sizeof(double))));
     DevBuf<double> dModel, dStats, dUacc, dZ;
     DevBuf<int> dAcc, dL;
-    DevBuf<cplx> dData;
+    DevBuf<unsigned char> dData;                     // [nChains][nsamples+1][nData] packed data (complex, or real for rho / phase plans)
+    const size_t dsz = datum_bytes(pl);
     cudaStream_t copy = nullptr;
     cudaEvent_t evCopied[2] = {nullptr, nullptr}, evFree[2] = {nullptr, nullptr};
     int rc = kOk;
     auto ok = [&](int r) { if (r && !rc) rc = r; };
     ok(dModel.alloc((size_t)nCh * nsamples * nAC)); ok(dStats.alloc((size_t)nCh * (nsamples + 1) * 4));
     ok(dUacc.upload(u_accept, (size_t)nCh * nsamples)); ok(dAcc.alloc((size_t)nCh * nsamples));
-    ok(dData.alloc((size_t)nCh * (nsamples + 1) * nData));
+    ok(dData.alloc((size_t)nCh * (nsamples + 1) * nData * dsz));
     ok(dZ.alloc(2 * (size_t)chunk * nState));
     {
         std::vector<int> Lall((size_t)nsamples * nCh);
@@ -1635,8 +1701,7 @@ int hmcmt_run_chain(hmcmt_plan* pl, double dt, int32_t nsamples, double rhoref, 
     // Hamiltonian at the start (getHamiltonian HMCSampler.jl:113-115): forward for the homogeneous model, mnorm = 0
     RC_TRY(compute_step(pl, false, nullptr));
     RC_TRY(energies(pl));
-    k_pack_pred<<<dim3((nData + 255) / 256, nCh), 256, 0, st>>>(nData, pl->nFull, pl->packed2full.p, pl->predFull.p, pl->predPacked.p);
-    pl->launches += 1;
+    RC_TRY(pack_pred(pl));
     {
         std::vector<double> e(2 * nCh), ph(nCh), sc(4 * nCh);
         RC_CUDA(cudaMemcpyAsync(e.data(), pl->energies.p, sizeof(double) * e.size(), cudaMemcpyDeviceToHost, st));
@@ -1646,8 +1711,9 @@ int hmcmt_run_chain(hmcmt_plan* pl, double dt, int32_t nsamples, double rhoref, 
             sc[4 * ch + 0] = ph[ch]; sc[4 * ch + 1] = e[2 * ch + 1]; sc[4 * ch + 2] = e[2 * ch];
             sc[4 * ch + 3] = ph[ch] + e[2 * ch] + e[2 * ch + 1];
             RC_CUDA(cudaMemcpyAsync(dStats.p + (size_t)ch * (nsamples + 1) * 4, &sc[4 * ch], sizeof(double) * 4, cudaMemcpyHostToDevice, st));
-            RC_CUDA(cudaMemcpyAsync(dData.p + (size_t)ch * (nsamples + 1) * nData, pl->predPacked.p + (size_t)ch * nData,
-                                    sizeof(cplx) * nData, cudaMemcpyDeviceToDevice, st));
+            RC_CUDA(cudaMemcpyAsync(dData.p + (size_t)ch * (nsamples + 1) * nData * dsz,
+                                    reinterpret_cast<const unsigned char*>(pl->predPacked.p) + (size_t)ch * nData * dsz, dsz * nData,
+                                    cudaMemcpyDeviceToDevice, st));
         }
         RC_CUDA(cudaMemcpyAsync(pl->chainScal.p, sc.data(), sizeof(double) * sc.size(), cudaMemcpyHostToDevice, st));
         // the first trajectory starts from hmcParamCurrent.rhomodel = the model-file strModel, copied BEFORE strModel / refModel
@@ -1676,11 +1742,17 @@ int hmcmt_run_chain(hmcmt_plan* pl, double dt, int32_t nsamples, double rhoref, 
         RC_TRY(trajectory_device(pl, dt, L, dL.p + (size_t)(it - 1) * nCh));
         if (!reuse_last_forward) RC_TRY(compute_step(pl, false, nullptr));       // the reference's redundant forward sweep
         RC_TRY(energies(pl));
-        k_pack_pred<<<dim3((nData + 255) / 256, nCh), 256, 0, st>>>(nData, pl->nFull, pl->packed2full.p, pl->predFull.p, pl->predPacked.p);
+        RC_TRY(pack_pred(pl));
         const double* zsrc = dZ.p + ((size_t)slot * chunk + inChunk) * nState;
-        k_accept<<<nCh, kHmcThreads, 0, st>>>(nAC, nData, it, nsamples, dUacc.p, pl->phi.p, pl->energies.p, zsrc, pl->m.p, pl->p.p,
-                                              pl->curM.p, pl->chainScal.p, pl->predPacked.p, dModel.p, dStats.p, dAcc.p, dData.p);
-        pl->launches += 2;
+        if (pl->dataKind)
+            k_accept<double><<<nCh, kHmcThreads, 0, st>>>(nAC, nData, it, nsamples, dUacc.p, pl->phi.p, pl->energies.p, zsrc, pl->m.p, pl->p.p,
+                                                          pl->curM.p, pl->chainScal.p, reinterpret_cast<const double*>(pl->predPacked.p),
+                                                          dModel.p, dStats.p, dAcc.p, reinterpret_cast<double*>(dData.p));
+        else
+            k_accept<cplx><<<nCh, kHmcThreads, 0, st>>>(nAC, nData, it, nsamples, dUacc.p, pl->phi.p, pl->energies.p, zsrc, pl->m.p, pl->p.p,
+                                                        pl->curM.p, pl->chainScal.p, pl->predPacked.p, dModel.p, dStats.p, dAcc.p,
+                                                        reinterpret_cast<cplx*>(dData.p));
+        pl->launches += 1;
         if (cudaGetLastError() != cudaSuccess) { cleanup(); return kErrCuda; }
         RC_TRY(mass_sqrt_apply(pl));             // p = sqrtM clip(z); k_accept's kinetic energy 1/2 z^T z equals 1/2 p^T invM p
         if (inChunk == chunk - 1 || it == nsamples) RC_CUDA(cudaEventRecord(evFree[slot], st));
@@ -1688,7 +1760,7 @@ int hmcmt_run_chain(hmcmt_plan* pl, double dt, int32_t nsamples, double rhoref, 
     RC_CUDA(cudaMemcpyAsync(hmcmodel, dModel.p, sizeof(double) * dModel.n, cudaMemcpyDeviceToHost, st));
     RC_CUDA(cudaMemcpyAsync(hmstats, dStats.p, sizeof(double) * dStats.n, cudaMemcpyDeviceToHost, st));
     RC_CUDA(cudaMemcpyAsync(accept, dAcc.p, sizeof(int) * dAcc.n, cudaMemcpyDeviceToHost, st));
-    RC_CUDA(cudaMemcpyAsync(hmcdata, dData.p, sizeof(cplx) * dData.n, cudaMemcpyDeviceToHost, st));
+    RC_CUDA(cudaMemcpyAsync(hmcdata, dData.p, dData.n, cudaMemcpyDeviceToHost, st));
     RC_CUDA(cudaStreamSynchronize(st));
     cleanup();
 #undef RC_TRY

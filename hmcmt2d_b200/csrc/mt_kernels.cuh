@@ -287,13 +287,19 @@ struct RxDev {
 };
 // data arrays are "full": index ((ch*nFreq+f)*nRx + r)*nModes + mi ; wd = 0 where the datum is absent.
 // vin: optional externally supplied data vector (hmcmt_jtvec); if null v = wd^2 (Z - obs).
+// kRhoPhase (plans of hmcmt_plan_create_rho_phase): the data of a slot are rho_a = |Z|^2/(omega mu0) and phase
+// phi = atan2(Im Z, Re Z) 180/pi; obs holds the pair (rho, phi), wd / wdPha their weights, resp receives the predicted pair.
+// With v_rho = w_rho^2 (rho - rho_obs), v_phi = w_phi^2 (phi - phi_obs) (or the real pair (v_rho, v_phi) carried by vin) the
+// slot's adjoint weight on Z is V = v_rho 2/(omega mu0) Z + v_phi 180/pi i Z/|Z|^2: Re(J^T conj(V)) is the misfit gradient
+// (d rho/d sigma = 2/(omega mu0) Re(conj(Z) J), d phi/d sigma = 180/pi Im(J/Z)), and everything after it is the impedance path.
 constexpr int kRxThreads = 256;
+template <bool kRhoPhase>
 __global__ void __launch_bounds__(kRxThreads)
 k_rx_adjoint(MeshDev M, RxDev rx, SysMap sm, const double* __restrict__ freqs, const double* __restrict__ sigma,
              const cplx* __restrict__ F, const cplx* __restrict__ obs, const double* __restrict__ wd,
-             const cplx* __restrict__ vin, cplx* __restrict__ pred, double* __restrict__ phiPart,
-             cplx* __restrict__ srows, cplx* __restrict__ qrow, cplx* __restrict__ adjrhs, int wantAdjoint, int respKind,
-             cplx* __restrict__ resp, int sys0) {
+             const double* __restrict__ wdPha, const cplx* __restrict__ vin, cplx* __restrict__ pred,
+             double* __restrict__ phiPart, cplx* __restrict__ srows, cplx* __restrict__ qrow, cplx* __restrict__ adjrhs,
+             int wantAdjoint, int respKind, cplx* __restrict__ resp, int sys0) {
     extern __shared__ __align__(16) unsigned char smraw[];
     const int ny = M.ny;
     cplx* F0 = reinterpret_cast<cplx*>(smraw);        // ny+1
@@ -367,16 +373,31 @@ k_rx_adjoint(MeshDev M, RxDev rx, SysMap sm, const double* __restrict__ freqs, c
             cplx Z = numF / denF;
             size_t di = (((size_t)ch * nFreq + f) * rx.nRx + r) * sm.nModes + mi;
             pred[di] = Z;
-            // apparent resistivity and phase (compMTRespTE mt2DTE.jl:253-256, compMTRespTM mt2DTM.jl:236-239): forward only
-            if (respKind == 1) resp[di] = mk(cabs2(Z) / (omega * kMu0), atan2(Z.y, Z.x) * 180.0 / kPi);
             size_t dob = ((size_t)f * rx.nRx + r) * sm.nModes + mi;     // obs / weights are shared by all chains
-            double w = wd[dob];
-            cplx res = w * (Z - obs[dob]);
-            phi += 0.5 * cabs2(res);
-            if (!wantAdjoint) continue;
-            cplx v = vin ? vin[di] : w * res;
-            if (w == 0.0 && !vin) continue;
-            cplx d = cconj(v);
+            cplx d;
+            if constexpr (kRhoPhase) {
+                // apparent resistivity and phase (compMTRespTE mt2DTE.jl:253-256, compMTRespTM mt2DTM.jl:236-239)
+                const double rhoA = cabs2(Z) / (omega * kMu0), phs = atan2(Z.y, Z.x) * 180.0 / kPi;
+                resp[di] = mk(rhoA, phs);
+                const double wr = wd[dob], wp = wdPha[dob];
+                const double rr = wr * (rhoA - obs[dob].x), rp = wp * (phs - obs[dob].y);     // no phase wrapping
+                phi += 0.5 * (rr * rr + rp * rp);
+                if (!wantAdjoint) continue;
+                if (wr == 0.0 && wp == 0.0 && !vin) continue;
+                const double vr = vin ? vin[di].x : wr * rr, vp = vin ? vin[di].y : wp * rp;
+                const cplx V = (vr * 2.0 / (omega * kMu0)) * Z + (vp * 180.0 / kPi / cabs2(Z)) * mk(-Z.y, Z.x);
+                d = cconj(V);
+            } else {
+                // apparent resistivity and phase (compMTRespTE mt2DTE.jl:253-256, compMTRespTM mt2DTM.jl:236-239): forward only
+                if (respKind == 1) resp[di] = mk(cabs2(Z) / (omega * kMu0), atan2(Z.y, Z.x) * 180.0 / kPi);
+                double w = wd[dob];
+                cplx res = w * (Z - obs[dob]);
+                phi += 0.5 * cabs2(res);
+                if (!wantAdjoint) continue;
+                cplx v = vin ? vin[di] : w * res;
+                if (w == 0.0 && !vin) continue;
+                d = cconj(v);
+            }
             const int iL = rx.iL[r], iR = rx.iR[r];
             const double wl = rx.wL[r], wr = rx.wR[r];
             cplx numS, denS;     // normalised interpolation used by the sensitivities (dataFuncSens.jl:89-91)

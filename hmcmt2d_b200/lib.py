@@ -54,6 +54,7 @@ def load() -> C.CDLL:
     vp = C.c_void_p
     lib.hmcmt_version.restype = C.c_char_p
     lib.hmcmt_plan_create.argtypes = [C.POINTER(Problem), C.POINTER(vp)]
+    lib.hmcmt_plan_create_rho_phase.argtypes = [C.POINTER(Problem), C.POINTER(vp)]
     lib.hmcmt_destroy.argtypes = [vp]
     lib.hmcmt_destroy.restype = None
     lib.hmcmt_plan_info.argtypes = [vp, C.c_int]
@@ -109,7 +110,7 @@ def load() -> C.CDLL:
 EXPORTED_SYMBOLS = [
     "factor_mumps_cmplx_", "factor_mumps_", "solve_mumps_cmplx_", "solve_mumps_", "solve_mumps_sparse_rhs_",
     "solve_mumps_cmplx_sparse_rhs_", "destroy_mumps_", "destroy_mumps_cmplx_",
-    "hmcmt_plan_create", "hmcmt_destroy", "hmcmt_plan_info", "hmcmt_forward", "hmcmt_forward_sigma", "hmcmt_jtvec",
+    "hmcmt_plan_create", "hmcmt_plan_create_rho_phase", "hmcmt_destroy", "hmcmt_plan_info", "hmcmt_forward", "hmcmt_forward_sigma", "hmcmt_jtvec",
     "hmcmt_forward_gradient", "hmcmt_forward_gradient_total", "hmcmt_jacobian", "hmcmt_status", "hmcmt_set_mass_matrix", "hmcmt_set_response_kind", "hmcmt_get_responses",
     "hmcmt_set_state", "hmcmt_get_state", "hmcmt_leapfrog_trajectory", "hmcmt_leapfrog_steps_device", "hmcmt_sync",
     "hmcmt_step_partial", "hmcmt_exchange_buffer", "hmcmt_step_finish", "hmcmt_nccl_unique_id", "hmcmt_nccl_init",

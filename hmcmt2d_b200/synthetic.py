@@ -4,6 +4,8 @@ last 8 growing x2), log-spaced frequencies, receivers on the air/earth interface
 with a 10 Ohm-m block.  Sizes are totals including padding and air."""
 from __future__ import annotations
 
+import dataclasses
+
 import numpy as np
 
 from .api import InvDataModel, setupInverseDataModel
@@ -86,3 +88,22 @@ def true_model_data(data: MTData, pred_true, noise: float = 0.05, seed: int = 7)
     rng = np.random.default_rng(seed)
     z = np.asarray(pred_true)
     return z * (1.0 + noise * rng.standard_normal(len(z))), noise * np.abs(z)
+
+
+def rho_phase_problem(data: MTData, inv: InvDataModel, rho_err: float = 0.05, phase_err: float = 1.5):
+    """The same survey as "Rho_Pha" data: every impedance row becomes an apparent resistivity rho_a = |Z|^2/(omega mu0) row and a
+    phase atan2(Im Z, Re Z) row in degrees (DataComp RhoXY, PhsXY / RhoYX, PhsYX, the row order of MT2DFwdSolver.jl:191-205),
+    converted from the impedance observations; errors rho_err x rho_a and an absolute phase_err degrees.
+    -> (MTData, InvDataModel) with the model part of `inv` unchanged."""
+    mu0 = 4e-7 * np.pi
+    z = np.asarray(inv.obsData, dtype=np.complex128)
+    fid, rid, did = (np.asarray(a, dtype=np.int64) for a in (data.freqID, data.rxID, data.dtID))
+    rho = np.abs(z) ** 2 / (2 * np.pi * np.asarray(data.freqs)[fid - 1] * mu0)
+    obs = np.stack([rho, np.degrees(np.arctan2(z.imag, z.real))], axis=1).reshape(-1)
+    err = np.stack([rho_err * rho, np.full(len(z), phase_err)], axis=1).reshape(-1)
+    comps = [name + ("XY" if "XY" in c else "YX") for c in data.dataComp for name in ("Rho", "Phs")]
+    nF, nRx = len(data.freqs), np.asarray(data.rxLoc).shape[0]
+    mask = np.repeat(np.asarray(data.dataID, dtype=bool).reshape(nF, nRx, len(data.dataComp)), 2, axis=2).reshape(-1)
+    rp = MTData(np.array(data.rxLoc), np.array(data.freqs), "Rho_Pha", comps, np.repeat(rid, 2), np.repeat(fid, 2),
+                np.stack([2 * did - 1, 2 * did], axis=1).reshape(-1), mask, data.compTE, data.compTM)
+    return rp, dataclasses.replace(inv, obsData=obs, dataW=1.0 / err, dataErr=err)

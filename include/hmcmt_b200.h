@@ -103,6 +103,17 @@ typedef struct hmcmt_problem {
 } hmcmt_problem;
 
 int hmcmt_plan_create(const hmcmt_problem* prob, hmcmt_plan** out);
+/* The same plan for apparent resistivity / phase data ("DataType: Rho_Pha", readMT2DData.jl:87), the same struct read with:
+ *   obsData  [nData] real: rho_a = |Z|^2/(omega mu0) in Ohm m, or phase = atan2(Im Z, Re Z) in degrees;
+ *   dataErr  [nData], weights 1/|err| per row;
+ *   nComp / compMode the modes as above; dtID = 2 (mode index) + 1 for rho_a, 2 (mode index) + 2 for phase, i.e. the reference's
+ *            DataComp order [RhoXY, PhsXY, RhoYX, PhsYX] (or the two rows of one mode).
+ * The misfit is phi_d = 1/2 sum_i ((pred_i - obs_i)/|err_i|)^2 over the rows present, the phase difference taken literally (no
+ * wrapping), and the gradients are its exact derivatives.  For such a plan every packed data array of the entry points below is
+ * [..][nData] REAL (doubles): pred of hmcmt_forward / _sigma / _forward_gradient / _total / hmcmt_leapfrog_trajectory, v of
+ * hmcmt_jtvec (gsig = sum_i v_i d pred_i / d sigma), J of hmcmt_jacobian ([nChains][nData][nAC]: d rho_a / d sigma and
+ * d phase / d sigma rows) and hmcdata of hmcmt_run_chain.  hmcmt_get_responses returns the (rho_a, phase) pairs. */
+int hmcmt_plan_create_rho_phase(const hmcmt_problem* prob, hmcmt_plan** out);
 void hmcmt_destroy(hmcmt_plan* plan);
 /* sizes derived by the plan: n=0 N (unknowns/system), 1 nNode, 2 nCell, 3 nb, 4 half-bandwidth,
  * 5 tile-window T, 6 macro-steps S, 7 systems per chain, 8 receiver node row zid (0-based),
@@ -191,10 +202,10 @@ int hmcmt_status(hmcmt_plan* plan);
  * identical to the reference's dense L).  Affects drift (getKineticGradient), kinetic energy and the momentum draws of
  * hmcmt_run_chain.  -40 if Wm is not positive definite. */
 int hmcmt_set_mass_matrix(hmcmt_plan* plan, int32_t kind);
-/* Response type of the forward evaluation (compMTRespTE mt2DTE.jl:240-259, compMTRespTM mt2DTM.jl:224-242):
- * kind 0 = impedance, 1 = apparent resistivity rho_a = |Z|^2/(omega mu0) and phase atan2(Im Z, Re Z) in degrees
- * ("Rho_Pha" data).  Forward only: the reference's own sensitivity code never reaches that data type
- * ("Rho_Pha" in readMT2DData.jl:87 / MT2DFwdSolver.jl:191 vs "Rho_Phs" in compJacTMatVec.jl:104), so gradients stay impedance-only.
+/* Response type of the forward evaluation of an impedance plan (compMTRespTE mt2DTE.jl:240-259, compMTRespTM mt2DTM.jl:224-242):
+ * kind 0 = impedance, 1 = apparent resistivity rho_a = |Z|^2/(omega mu0) and phase atan2(Im Z, Re Z) in degrees.  A forward-only
+ * toggle: the misfit and gradients of such a plan stay those of its impedance data (evaluations with kind 1 are launched eagerly,
+ * outside the captured graph).  Gradients of rho / phase data come from a plan made by hmcmt_plan_create_rho_phase.
  * hmcmt_get_responses copies the responses of the last forward evaluation, unmasked:
  * out [nChains][nFreq][nRx][nComp][2] doubles = (Re Z, Im Z) or (rho_a, phase). */
 int hmcmt_set_response_kind(hmcmt_plan* plan, int32_t kind);

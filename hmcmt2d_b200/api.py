@@ -129,11 +129,19 @@ def readstartupFile(startupfile: str):
 
 # DataComp of "Rho_Pha" surveys, in the row order of MT2DFwdSolver.jl:191-205, and the modes they select
 _RHO_PHA_COMPS = {("RhoXY", "PhsXY"): [0], ("RhoYX", "PhsYX"): [1], ("RhoXY", "PhsXY", "RhoYX", "PhsYX"): [0, 1]}
+# DataComp entries of "Impedance" surveys and their hmcmt_problem.compMode: the impedances (MT2DFwdSolver.jl:183-187) and the TE
+# tipper TZY = Hz/Hy (include/hmcmt_b200.h), any of them in this order
+_IMPEDANCE_COMPS = {"ZXY": 0, "ZYX": 1, "TZY": 2}
+
+
+def _comp_mode(comp: str) -> int:
+    """System a DataComp entry is computed in: 0 TE (ZXY, TZY, RhoXY, PhsXY), 1 TM (ZYX, RhoYX, PhsYX)."""
+    return 0 if ("XY" in comp or comp == "TZY") else 1
 
 
 class Plan:
     """Owns one `hmcmt_plan` (device-resident problem: mesh, survey, weights, factors, chain state).
-    DataType "Impedance": packed data arrays are complex.  DataType "Rho_Pha": one real apparent resistivity or phase per row
+    DataType "Impedance": packed data arrays are complex; DataComp is ZXY, ZYX and the tipper TZY, or any of them in that order.  DataType "Rho_Pha": one real apparent resistivity or phase per row
     (dtID = 2 mode + 1 / 2), and every packed data array (predictions, J^T v input, Jacobian rows, chain samples) is real."""
 
     def __init__(self, mtMesh: TensorMesh2D, mtData: MTData, invParam: InvDataModel, hmcprior: HMCPrior,
@@ -155,14 +163,11 @@ class Plan:
         else:
             comp_mode = []
             for c in mtData.dataComp:
-                if "XY" in c:
-                    comp_mode.append(0)
-                elif "YX" in c:
-                    comp_mode.append(1)
-                else:
+                if c not in _IMPEDANCE_COMPS:
                     raise NotImplementedError(f"data component {c}")
-            if comp_mode not in ([0], [1], [0, 1]):
-                raise ValueError("DataComp must be [ZXY, ZYX] in that order (MT2DFwdSolver.jl:183-187)")
+                comp_mode.append(_IMPEDANCE_COMPS[c])
+            if comp_mode != sorted(set(comp_mode)):
+                raise ValueError("DataComp must be [ZXY, ZYX, TZY] or a part of it, in that order (MT2DFwdSolver.jl:183-187)")
         act = np.asarray(invParam.activeCell.tocsc().indices, dtype=np.int32)      # one row index per column
         Wm = invParam.Wm.tocsr()
         Wm.sort_indices()
@@ -200,7 +205,7 @@ class Plan:
         self.nAC, self.nData, self.nFreq = len(act), pr.nData, pr.nFreq
         self.nNode = (self.ny + 1) * (self.nz + 1)
         self.nCell = self.ny * self.nz
-        self.compTE, self.compTM = 0 in comp_mode, 1 in comp_mode
+        self.compTE, self.compTM = 0 in comp_mode or 2 in comp_mode, 1 in comp_mode
 
     def info(self, what: int) -> int:
         return int(self.L.hmcmt_plan_info(self.h, what))
@@ -388,10 +393,10 @@ def shard_systems(mtData: MTData, invParam: InvDataModel, rank: int, world: int)
     """Balanced partition of the (frequency, mode) SYSTEMS: with an even number of ranks and a TE + TM survey the first half of
     the ranks takes the TE systems and the second half the TM systems, frequencies round-robin inside each half (120 systems
     over 8 ranks = 15 each at cfg4, instead of 8 / 7 frequencies x 2 modes).  Otherwise falls back to `shard_frequencies`.
+    A rank takes every DataComp entry its mode computes: ZXY and TZY, or ZYX, or the rho_a and phase rows of one mode.
     -> (MTData of this rank, InvDataModel with its observation rows, `rows` = their positions in the full data vector)."""
-    # rows per mode: one impedance component, or the rho_a and phase rows of a "Rho_Pha" survey (dtID = 2 mode + 1 / 2)
-    per_mode = 2 if "Rho_Pha" in mtData.dataType else 1
-    two_modes = bool(mtData.compTE and mtData.compTM) and len(mtData.dataComp) == 2 * per_mode
+    comp_modes = np.array([_comp_mode(c) for c in mtData.dataComp])
+    two_modes = bool(mtData.compTE and mtData.compTM) and set(comp_modes.tolist()) == {0, 1}
     if world < 2 or world % 2 or not two_modes:
         return shard_frequencies(mtData, invParam, rank, world)
     half = world // 2
@@ -403,12 +408,14 @@ def shard_systems(mtData: MTData, invParam: InvDataModel, rank: int, world: int)
     newid = np.zeros(nF + 1, dtype=np.int64)
     newid[mine + 1] = np.arange(1, len(mine) + 1)
     fid, did = np.asarray(mtData.freqID), np.asarray(mtData.dtID)
-    comps = slice(mode * per_mode, (mode + 1) * per_mode)
-    rows = np.nonzero((newid[fid] > 0) & ((did - 1) // per_mode == mode))[0]
+    comps = np.nonzero(comp_modes == mode)[0]                   # DataComp entries of this mode, in order
+    newdid = np.zeros(len(comp_modes) + 1, dtype=np.int64)
+    newdid[comps + 1] = np.arange(1, len(comps) + 1)
+    rows = np.nonzero((newid[fid] > 0) & (newdid[did] > 0))[0]
     nRx, nDt = np.asarray(mtData.rxLoc).shape[0], len(mtData.dataComp)
     mask = np.asarray(mtData.dataID, dtype=bool).reshape(nF, nRx, nDt)[mine][:, :, comps].reshape(-1)
-    sub = MTData(np.array(mtData.rxLoc), np.array(mtData.freqs)[mine], mtData.dataType, list(mtData.dataComp[comps]),
-                 np.asarray(mtData.rxID)[rows], newid[fid[rows]], did[rows] - mode * per_mode, mask, mode == 0, mode == 1)
+    sub = MTData(np.array(mtData.rxLoc), np.array(mtData.freqs)[mine], mtData.dataType, [mtData.dataComp[k] for k in comps],
+                 np.asarray(mtData.rxID)[rows], newid[fid[rows]], newdid[did[rows]], mask, mode == 0, mode == 1)
     dataW = np.asarray(invParam.dataW)[rows]
     inv = InvDataModel(np.asarray(invParam.obsData)[rows], dataW, np.array(invParam.strModel), np.array(invParam.refModel),
                        invParam.activeCell, np.array(invParam.bgModel), invParam.Wm, 1.0 / dataW)

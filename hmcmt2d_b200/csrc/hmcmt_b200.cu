@@ -46,7 +46,9 @@ struct hmcmt_plan {
     // sizes
     int ny = 0, nz = 0, nFreq = 0, nRx = 0, nData = 0, nAC = 0, nChains = 1, nModes = 0, nComp = 0;
     int modeList[2] = {0, 1};
-    int nSysPerChain = 0, nSys = 0, nFull = 0;      // nFull = nFreq*nRx*nModes per chain
+    int nSysPerChain = 0, nSys = 0, nFull = 0;      // nFull = nFreq*nRx*nComp per chain
+    bool tipper = false;                            // an impedance plan with a TZY component (compMode 2)
+    CompMap cm{};                                   // component <-> system of a tipper plan (k_rx_adjoint<false, true>)
     int T = 0, S = 0, b = 0, device = 0, conStaged = 0, numSMs = 148;
     BandDom dom{};
     int steps0 = 0, steps1 = 0;                     // macro-steps of half 0 (own lines + separator) / half 1 (0 when not split)
@@ -74,11 +76,11 @@ struct hmcmt_plan {
     std::vector<int> h_packed2full;      // [nData] full index (without chain) of each packed datum; rho / phase plans: index into
                                          // the real view [nFull][2] (rho, phase) of the full arrays
     // device buffers
-    DevBuf<double> yLen, zLen, zNode, freqs, fdy1, fdy2, wL, wR, bg, wmVal, wd, m, p, mref, sigma, meanSig, planes;
+    DevBuf<double> yLen, zLen, zNode, freqs, fdy1, fdy2, wL, wR, twL, twR, bg, wmVal, wd, m, p, mref, sigma, meanSig, planes;
     DevBuf<double> wdPha;                           // phase weights of a rho / phase plan (wd holds the rho weights)
     DevBuf<double> driftPart;                       // block maxima of the drift (k_drift_max)
     DevBuf<double> xbuf, Gpart, phiPart, phi, gsig, gdata, gtotal, energies, panels, curM, curP, chainScal, zmom;
-    DevBuf<int> fid, iL, iR, cell2act, act2cell, wmPtr, wmIdx, status, driftFlag, packed2full, full2packed, Lsteps;
+    DevBuf<int> fid, iL, iR, tjL, tjR, cell2act, act2cell, wmPtr, wmIdx, status, driftFlag, packed2full, full2packed, Lsteps;
     DevBuf<cplx> obs, bc, bcs, rhs, x, F, lam, Lam, srows, qrow, scratch, predFull, ainvz, zadj, vin, predPacked, wexp, conCols, respFull;
     DevBuf<BandSys> sysDesc;
     DevBuf<SolveJob> jobs, fwdJobs;                 // fwdJobs: back-substitution sweeps of the fused forward systems (split systems)
@@ -357,18 +359,23 @@ __global__ void k_unpack_exchange(int nAC, const double* __restrict__ xbuf, cons
 // Explicit Jacobian (compJacMat.jl:7-381 / compJacTMat.jl:9-406): one pass of the adjoint machinery per (receiver, real /
 // imaginary part) yields, in every (frequency, mode) system, the row of that system's datum at this receiver.
 //   v = e_d   -> real(J^T conj(v)) = Re J[d,:]  ;   v = i e_d -> Im J[d,:]
-__global__ void k_jac_vin(int nFull, int nRx, int nModes, int r, cplx val, cplx* __restrict__ vin) {
+// Components that share a system (ZXY and TZY) need passes of their own: a pass covers the components of compMask, comp[mi] being
+// the one of them that system mi holds (-1: none).
+__global__ void k_jac_vin(int nFull, int nRx, int nComp, unsigned compMask, int r, cplx val, cplx* __restrict__ vin) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x, ch = blockIdx.y;
     if (i >= nFull) return;
-    const int rx = (i / nModes) % nRx;
-    vin[(size_t)ch * nFull + i] = rx == r ? val : mk(0.0, 0.0);
+    const int rx = (i / nComp) % nRx, c = i % nComp;
+    vin[(size_t)ch * nFull + i] = (rx == r && ((compMask >> c) & 1u)) ? val : mk(0.0, 0.0);
 }
-__global__ void k_jac_rows(int nAC, int nCell, int nFreq, int nRx, int nModes, int nData, int r, int part, const int* __restrict__ act2cell,
-                           const int* __restrict__ full2packed, const double* __restrict__ Gpart, double* __restrict__ J) {
+__global__ void k_jac_rows(int nAC, int nCell, int nFreq, int nRx, int nModes, int nComp, int2 comp, int nData, int r, int part,
+                           const int* __restrict__ act2cell, const int* __restrict__ full2packed, const double* __restrict__ Gpart,
+                           double* __restrict__ J) {
     const int a = blockIdx.x * blockDim.x + threadIdx.x, sys = blockIdx.y;
     if (a >= nAC) return;
     const int f = sys % nFreq, t = sys / nFreq, mi = t % nModes, ch = t / nModes;
-    const int d = full2packed[(f * nRx + r) * nModes + mi];
+    const int c = mi == 0 ? comp.x : comp.y;
+    if (c < 0) return;
+    const int d = full2packed[(f * nRx + r) * nComp + c];
     if (d < 0) return;
     J[(((size_t)ch * nData + d) * nAC + a) * 2 + part] = Gpart[(size_t)sys * nCell + act2cell[a]];
 }
@@ -525,16 +532,20 @@ int forward_phase(hmcmt_plan* pl, bool wantAdjoint) {
     return kOk;
 }
 
+// the receiver-functional instance of the plan's data (fixed when the plan is created)
+decltype(&k_rx_adjoint<false, false>) rx_kernel(const hmcmt_plan* pl) {
+    if (pl->dataKind) return k_rx_adjoint<true, false>;
+    return pl->tipper ? k_rx_adjoint<false, true> : k_rx_adjoint<false, false>;
+}
 // receiver functional: responses, residual, misfit partial and (wantAdjoint) the adjoint sources for the data vector vin
 // (null: v = Wd^2 (pred - obs))
 int rx_range(hmcmt_plan* pl, const SysRange& r, bool wantAdjoint, const cplx* vin) {
     const MeshDev& M = pl->M;
     size_t rxSmem = (size_t)(6 * (M.ny + 1) + 3 * M.ny) * sizeof(cplx);
     if (wantAdjoint) HMCMT_CUDA_TRY(cudaMemsetAsync(pl->lam.p + (size_t)r.s0 * M.N, 0, sizeof(cplx) * (size_t)r.n * M.N, r.st));
-    auto kern = pl->dataKind ? k_rx_adjoint<true> : k_rx_adjoint<false>;
-    kern<<<r.n, kRxThreads, rxSmem, r.st>>>(M, pl->rx, pl->sm, pl->freqs.p, pl->sigma.p, pl->F.p, pl->obs.p, pl->wd.p, pl->wdPha.p, vin,
-                                            pl->predFull.p, pl->phiPart.p, pl->srows.p, pl->qrow.p, pl->lam.p, wantAdjoint ? 1 : 0,
-                                            pl->respKind, pl->respFull.p, r.s0);
+    rx_kernel(pl)<<<r.n, kRxThreads, rxSmem, r.st>>>(M, pl->rx, pl->sm, pl->cm, pl->freqs.p, pl->sigma.p, pl->F.p, pl->obs.p, pl->wd.p,
+                                                     pl->wdPha.p, vin, pl->predFull.p, pl->phiPart.p, pl->srows.p, pl->qrow.p, pl->lam.p,
+                                                     wantAdjoint ? 1 : 0, pl->respKind, pl->respFull.p, r.s0);
     LAUNCH_CHECK(pl);
     return kOk;
 }
@@ -812,8 +823,19 @@ static int plan_create(const hmcmt_problem* pr, hmcmt_plan** out, int dataKind) 
         fprintf(stderr, "[hmcmt_b200] no CUDA device: this library has no CPU fallback\n");
         return kErrNoDevice;
     }
-    if (pr->ny < 3 || pr->nz < 3 || pr->nFreq < 1 || pr->nRx < 1 || pr->nComp < 1 || pr->nComp > 2 || pr->nChains < 1 || pr->nAC < 1)
+    if (pr->ny < 3 || pr->nz < 3 || pr->nFreq < 1 || pr->nRx < 1 || pr->nComp < 1 || pr->nComp > 3 || pr->nChains < 1 || pr->nAC < 1)
         return kErrArg;
+    // compMode 2 (TZY, the TE tipper): at most once, as the last component, impedance plans only; the impedance components before
+    // it are one or two as without it
+    const bool tipper = pr->compMode[pr->nComp - 1] == 2;
+    const int nZ = pr->nComp - (tipper ? 1 : 0);
+    if (nZ > 2 || (tipper && dataKind)) return kErrArg;
+    for (int c = 0; c < nZ; ++c)
+        if (pr->compMode[c] == 2) return kErrArg;
+    int teSys = -1;                                  // the system the tipper shares (the first TE one), or a TE system of its own
+    for (int c = 0; c < nZ && teSys < 0; ++c)
+        if (pr->compMode[c] == 0) teSys = c;
+    if (tipper && teSys < 0 && nZ == 2) return kErrArg;
     HMCMT_CUDA_TRY(cudaSetDevice(pr->device));
     hmcmt_plan* pl = new (std::nothrow) hmcmt_plan();
     if (!pl) return kErrAlloc;
@@ -823,8 +845,12 @@ static int plan_create(const hmcmt_problem* pr, hmcmt_plan** out, int dataKind) 
         if (cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, pr->device) == cudaSuccess && nsm > 0) pl->numSMs = nsm;
     }
     pl->ny = pr->ny; pl->nz = pr->nz; pl->nFreq = pr->nFreq; pl->nRx = pr->nRx; pl->nData = pr->nData; pl->nAC = pr->nAC;
-    pl->nChains = pr->nChains; pl->nComp = pr->nComp; pl->nModes = pr->nComp; pl->dataKind = dataKind;
-    for (int c = 0; c < pr->nComp; ++c) pl->modeList[c] = pr->compMode[c];
+    pl->nChains = pr->nChains; pl->nComp = pr->nComp; pl->nModes = nZ; pl->dataKind = dataKind; pl->tipper = tipper;
+    for (int c = 0; c < nZ; ++c) pl->modeList[c] = pr->compMode[c];
+    if (tipper) {
+        if (teSys < 0) { teSys = nZ; pl->modeList[pl->nModes++] = 0; }
+        pl->cm = CompMap{pl->nComp, {nZ > 0 ? 0 : -1, nZ > 1 ? 1 : -1}, pl->nComp - 1, teSys};
+    }
     pl->beta = pr->regParam;
     pl->lo = std::log(pr->sigBounds[0]);
     pl->hi = std::log(pr->sigBounds[1]);
@@ -861,7 +887,7 @@ static int plan_create(const hmcmt_problem* pr, hmcmt_plan** out, int dataKind) 
     }
     pl->nSysPerChain = pl->nModes * pl->nFreq;
     pl->nSys = pl->nSysPerChain * pl->nChains;
-    pl->nFull = pl->nFreq * pl->nRx * pl->nModes;
+    pl->nFull = pl->nFreq * pl->nRx * pl->nComp;
     pl->sm = SysMap{pl->nFreq, pl->nModes, pl->modeList[0], pl->modeList[1]};
     pl->h_yLen.assign(pr->yLen, pr->yLen + ny);
     pl->h_zLen.assign(pr->zLen, pr->zLen + nz);
@@ -877,8 +903,10 @@ static int plan_create(const hmcmt_problem* pr, hmcmt_plan** out, int dataKind) 
     for (int k = 0; k <= nz; ++k) if (std::fabs(zNode[k] - pr->rxLoc[1]) < 0.1) { zid = k; break; }
     if (zid < 0 || zid >= nz) { delete pl; return kErrArg; }
     M.zid = zid;
-    std::vector<int> fid(pr->nRx), iL(pr->nRx), iR(pr->nRx);
-    std::vector<double> d1(pr->nRx), d2(pr->nRx), wL(pr->nRx), wR(pr->nRx);
+    std::vector<double> yCen(ny);
+    for (int j = 0; j < ny; ++j) yCen[j] = 0.5 * (yNode[j] + yNode[j + 1]);
+    std::vector<int> fid(pr->nRx), iL(pr->nRx), iR(pr->nRx), tjL(pr->nRx), tjR(pr->nRx);
+    std::vector<double> d1(pr->nRx), d2(pr->nRx), wL(pr->nRx), wR(pr->nRx), twL(pr->nRx), twR(pr->nRx);
     for (int r = 0; r < pr->nRx; ++r) {
         double y = pr->rxLoc[2 * r];
         int id = -1;
@@ -886,10 +914,11 @@ static int plan_create(const hmcmt_problem* pr, hmcmt_plan** out, int dataKind) 
         if (id <= 0) { delete pl; return kErrArg; }       // "receiver location seems to be out of range"
         fid[r] = id; d1[r] = y - yNode[id - 1]; d2[r] = yNode[id] - y;
         linear_interp(y, yNode, iL[r], iR[r], wL[r], wR[r]);
+        linear_interp(y, yCen, tjL[r], tjR[r], twL[r], twR[r]);
     }
-    // data layout: full slot ((f*nRx + r)*nModes + mi), rows must be sorted (freq, rx, comp).  Rho / phase plans: dtID =
-    // 2 mi + 1 (rho_a) or 2 mi + 2 (phase), real obsData; the slot keeps the observed pair and both weights (0 where a row is absent)
-    // and a packed row maps to 2 slot + part of the real view of the full arrays
+    // data layout: full slot ((f*nRx + r)*nComp + c), one per DataComp entry, rows must be sorted (freq, rx, comp).  Rho / phase
+    // plans (nComp = nModes): dtID = 2 mi + 1 (rho_a) or 2 mi + 2 (phase), real obsData; the slot keeps the observed pair and both
+    // weights (0 where a row is absent) and a packed row maps to 2 slot + part of the real view of the full arrays
     std::vector<double> wdFull(pl->nFull, 0.0), wpFull(dataKind ? pl->nFull : 0, 0.0);
     std::vector<cplx> obsFull(pl->nFull, mk(0.0, 0.0));
     pl->h_packed2full.resize(pr->nData);
@@ -898,8 +927,8 @@ static int plan_create(const hmcmt_problem* pr, hmcmt_plan** out, int dataKind) 
     for (int i = 0; i < pr->nData; ++i) {
         long f = pr->freqID[i] - 1, r = pr->rxID[i] - 1, c = pr->dtID[i] - 1;
         if (f < 0 || f >= pr->nFreq || r < 0 || r >= pr->nRx || c < 0 || c >= nDt) { delete pl; return kErrArg; }
-        const long mi = dataKind ? c / 2 : c, part = dataKind ? c % 2 : 0;
-        const long slot = (f * pr->nRx + r) * pl->nModes + mi;
+        const long ci = dataKind ? c / 2 : c, part = dataKind ? c % 2 : 0;     // DataComp entry (rho / phase: its mode)
+        const long slot = (f * pr->nRx + r) * pl->nComp + ci;
         const long full = dataKind ? 2 * slot + part : slot;
         if (full <= prev) {
             fprintf(stderr, "[hmcmt_b200] data rows must be sorted by (freq, rx, comp) without duplicates\n");
@@ -933,6 +962,8 @@ static int plan_create(const hmcmt_problem* pr, hmcmt_plan** out, int dataKind) 
     ok(pl->fid.upload(fid.data(), pr->nRx)); ok(pl->iL.upload(iL.data(), pr->nRx)); ok(pl->iR.upload(iR.data(), pr->nRx));
     ok(pl->fdy1.upload(d1.data(), pr->nRx)); ok(pl->fdy2.upload(d2.data(), pr->nRx));
     ok(pl->wL.upload(wL.data(), pr->nRx)); ok(pl->wR.upload(wR.data(), pr->nRx));
+    ok(pl->tjL.upload(tjL.data(), pr->nRx)); ok(pl->tjR.upload(tjR.data(), pr->nRx));
+    ok(pl->twL.upload(twL.data(), pr->nRx)); ok(pl->twR.upload(twR.data(), pr->nRx));
     ok(pl->cell2act.upload(cell2act.data(), M.nCell)); ok(pl->act2cell.upload(pr->activeIdx, pr->nAC));
     ok(pl->bg.upload(pr->bgModel, M.nCell));
     ok(pl->wmPtr.upload(pr->wmRowPtr, pr->nAC + 1));
@@ -975,7 +1006,7 @@ static int plan_create(const hmcmt_problem* pr, hmcmt_plan** out, int dataKind) 
     cudaMemset(pl->p.p, 0, sizeof(double) * nCh * pr->nAC);
     cudaMemset(pl->mref.p, 0, sizeof(double) * nCh * pr->nAC);
     M.yLen = pl->yLen.p; M.zLen = pl->zLen.p; M.zNode = pl->zNode.p;
-    pl->rx = RxDev{pr->nRx, pl->fid.p, pl->fdy1.p, pl->fdy2.p, pl->iL.p, pl->iR.p, pl->wL.p, pl->wR.p};
+    pl->rx = RxDev{pr->nRx, pl->fid.p, pl->fdy1.p, pl->fdy2.p, pl->iL.p, pl->iR.p, pl->wL.p, pl->wR.p, pl->tjL.p, pl->tjR.p, pl->twL.p, pl->twR.p};
     // per-system descriptors
     std::vector<BandSys> sd(nSys);
     std::vector<SolveJob> jb(nSys), jfw(nSys);
@@ -1029,8 +1060,7 @@ static int plan_create(const hmcmt_problem* pr, hmcmt_plan** out, int dataKind) 
         }
         pl->conStaged = contract_cols_smem(M.ny, M.nz, 1) <= 200 * 1024 ? 1 : 0;
         const size_t cSmem = contract_cols_smem(M.ny, M.nz, pl->conStaged);
-        if ((rxSmem > 48 * 1024 && cudaFuncSetAttribute(dataKind ? k_rx_adjoint<true> : k_rx_adjoint<false>,
-                                                        cudaFuncAttributeMaxDynamicSharedMemorySize, (int)rxSmem) != cudaSuccess) ||
+        if ((rxSmem > 48 * 1024 && cudaFuncSetAttribute(rx_kernel(pl), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)rxSmem) != cudaSuccess) ||
             (cSmem > 48 * 1024 && cudaFuncSetAttribute(k_contract_cols, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cSmem) != cudaSuccess)) {
             hmcmt_destroy(pl);
             return kErrArg;
@@ -1119,7 +1149,7 @@ void hmcmt_destroy(hmcmt_plan* pl) {
     for (auto& e : pl->factorEvents) { cudaEventDestroy(e.first); cudaEventDestroy(e.second); }
     for (cudaEvent_t e : pl->factorMid) cudaEventDestroy(e);
     pl->yLen.release(); pl->zLen.release(); pl->zNode.release(); pl->freqs.release(); pl->fdy1.release(); pl->fdy2.release();
-    pl->wL.release(); pl->wR.release(); pl->bg.release(); pl->wmVal.release(); pl->wd.release(); pl->wdPha.release(); pl->m.release(); pl->p.release();
+    pl->wL.release(); pl->wR.release(); pl->twL.release(); pl->twR.release(); pl->tjL.release(); pl->tjR.release(); pl->bg.release(); pl->wmVal.release(); pl->wd.release(); pl->wdPha.release(); pl->m.release(); pl->p.release();
     pl->mref.release(); pl->sigma.release(); pl->meanSig.release(); pl->planes.release(); pl->Gpart.release(); pl->phiPart.release();
     pl->phi.release(); pl->gsig.release(); pl->gdata.release(); pl->gtotal.release(); pl->energies.release(); pl->panels.release(); pl->curM.release();
     pl->curP.release(); pl->driftPart.release(); pl->chainScal.release(); pl->zmom.release(); pl->fid.release(); pl->iL.release(); pl->iR.release();
@@ -1401,23 +1431,33 @@ int hmcmt_jacobian(hmcmt_plan* pl, double* J) {
     if (rc) return rc;
     HMCMT_CUDA_TRY(cudaMemsetAsync(dJ.p, 0, nJ * sizeof(double), st));
     if (!pl->haveSens) rc = launch_sens_side(pl);
-    for (int r = 0; r < pl->nRx && rc == kOk; ++r)
-        for (int part = 0; part < 2 && rc == kOk; ++part) {
-            k_jac_vin<<<dim3((pl->nFull + 255) / 256, pl->nChains), 256, 0, st>>>(pl->nFull, pl->nRx, pl->nModes, r,
-                                                                                 part == 0 ? mk(1.0, 0.0) : mk(0.0, 1.0), pl->vin.p);
-            ++pl->launches;
-            rc = rx_phase(pl, true, pl->vin.p);
-            if (rc == kOk) rc = adjoint_phase(pl, false);
-            if (rc != kOk) break;
-            const dim3 grid((pl->nAC + 255) / 256, pl->nSys);
-            if (pl->dataKind)
-                k_jac_rows_real<<<grid, 256, 0, st>>>(pl->nAC, M.nCell, pl->nFreq, pl->nRx, pl->nModes, pl->nData, r, part, pl->act2cell.p,
-                                                      pl->full2packed.p, pl->Gpart.p, dJ.p);
-            else
-                k_jac_rows<<<grid, 256, 0, st>>>(pl->nAC, M.nCell, pl->nFreq, pl->nRx, pl->nModes, pl->nData, r, part, pl->act2cell.p,
-                                                 pl->full2packed.p, pl->Gpart.p, dJ.p);
-            ++pl->launches;
-        }
+    // groups of components that share no system, one set of 2 nRx passes each: all components, or (tipper plans) the impedance
+    // components and then the tipper
+    struct Group { unsigned mask; int2 comp; };
+    std::vector<Group> groups;
+    const CompMap& cm = pl->cm;
+    if (!pl->tipper) groups.push_back(Group{(1u << pl->nComp) - 1u, make_int2(0, 1)});
+    else if (cm.zc[0] >= 0 || cm.zc[1] >= 0)
+        groups.push_back(Group{(cm.zc[0] >= 0 ? 1u << cm.zc[0] : 0u) | (cm.zc[1] >= 0 ? 1u << cm.zc[1] : 0u), make_int2(cm.zc[0], cm.zc[1])});
+    if (pl->tipper) groups.push_back(Group{1u << cm.tc, make_int2(cm.tmi == 0 ? cm.tc : -1, cm.tmi == 1 ? cm.tc : -1)});
+    for (const Group& grp : groups)
+        for (int r = 0; r < pl->nRx && rc == kOk; ++r)
+            for (int part = 0; part < 2 && rc == kOk; ++part) {
+                k_jac_vin<<<dim3((pl->nFull + 255) / 256, pl->nChains), 256, 0, st>>>(pl->nFull, pl->nRx, pl->nComp, grp.mask, r,
+                                                                                     part == 0 ? mk(1.0, 0.0) : mk(0.0, 1.0), pl->vin.p);
+                ++pl->launches;
+                rc = rx_phase(pl, true, pl->vin.p);
+                if (rc == kOk) rc = adjoint_phase(pl, false);
+                if (rc != kOk) break;
+                const dim3 grid((pl->nAC + 255) / 256, pl->nSys);
+                if (pl->dataKind)
+                    k_jac_rows_real<<<grid, 256, 0, st>>>(pl->nAC, M.nCell, pl->nFreq, pl->nRx, pl->nModes, pl->nData, r, part, pl->act2cell.p,
+                                                          pl->full2packed.p, pl->Gpart.p, dJ.p);
+                else
+                    k_jac_rows<<<grid, 256, 0, st>>>(pl->nAC, M.nCell, pl->nFreq, pl->nRx, pl->nModes, pl->nComp, grp.comp, pl->nData, r,
+                                                     part, pl->act2cell.p, pl->full2packed.p, pl->Gpart.p, dJ.p);
+                ++pl->launches;
+            }
     if (rc == kOk && cudaGetLastError() != cudaSuccess) rc = kErrCuda;
     if (rc == kOk && cudaMemcpyAsync(J, dJ.p, nJ * sizeof(double), cudaMemcpyDeviceToHost, st) != cudaSuccess) rc = kErrCuda;
     if (cudaStreamSynchronize(st) != cudaSuccess && rc == kOk) rc = kErrCuda;

@@ -284,18 +284,32 @@ struct RxDev {
     const int* iR;
     const double* wL;
     const double* wR;
+    const int* tjL;        // the same weights on the cell centres (linRxMap2, sensUtils.jl:17-52): Hz of the tipper
+    const int* tjR;
+    const double* twL;
+    const double* twR;
 };
-// data arrays are "full": index ((ch*nFreq+f)*nRx + r)*nModes + mi ; wd = 0 where the datum is absent.
+// Data components of an impedance plan with a tipper (kTipper): system mi holds the impedance component zc[mi] (-1: none, a
+// [TZY]-only plan) and system tmi also the tipper component tc.  Without a tipper nComp = nModes and component = system.
+struct CompMap {
+    int nComp, zc[2], tc, tmi;
+};
+// data arrays are "full": index ((ch*nFreq+f)*nRx + r)*nComp + c ; wd = 0 where the datum is absent.
 // vin: optional externally supplied data vector (hmcmt_jtvec); if null v = wd^2 (Z - obs).
 // kRhoPhase (plans of hmcmt_plan_create_rho_phase): the data of a slot are rho_a = |Z|^2/(omega mu0) and phase
 // phi = atan2(Im Z, Re Z) 180/pi; obs holds the pair (rho, phi), wd / wdPha their weights, resp receives the predicted pair.
 // With v_rho = w_rho^2 (rho - rho_obs), v_phi = w_phi^2 (phi - phi_obs) (or the real pair (v_rho, v_phi) carried by vin) the
 // slot's adjoint weight on Z is V = v_rho 2/(omega mu0) Z + v_phi 180/pi i Z/|Z|^2: Re(J^T conj(V)) is the misfit gradient
 // (d rho/d sigma = 2/(omega mu0) Re(conj(Z) J), d phi/d sigma = 180/pi Im(J/Z)), and everything after it is the impedance path.
+// kTipper (impedance plans with a TZY component): the TE system tmi also forms, per receiver, the tipper
+//   Hz0_j = (F0_{j+1} - F0_j)/(yLen_j i omega mu0) at the cell centres, Hzr = twL Hz0_{tjL} + twR Hz0_{tjR},
+//   Hyr = wL Hy0_{iL} + wR Hy0_{iR} (G0, the normalised node weights), T = Hzr/Hyr,
+// and with d = conj(v_T) adds the reverse mode d/Hyr (onto F0 through the two-point difference of each cell) and -d T/Hyr (onto
+// G0 with the node weights) to the impedance adjoints; everything after that is the impedance path.
 constexpr int kRxThreads = 256;
-template <bool kRhoPhase>
+template <bool kRhoPhase, bool kTipper>
 __global__ void __launch_bounds__(kRxThreads)
-k_rx_adjoint(MeshDev M, RxDev rx, SysMap sm, const double* __restrict__ freqs, const double* __restrict__ sigma,
+k_rx_adjoint(MeshDev M, RxDev rx, SysMap sm, CompMap cm, const double* __restrict__ freqs, const double* __restrict__ sigma,
              const cplx* __restrict__ F, const cplx* __restrict__ obs, const double* __restrict__ wd,
              const double* __restrict__ wdPha, const cplx* __restrict__ vin, cplx* __restrict__ pred,
              double* __restrict__ phiPart, cplx* __restrict__ srows, cplx* __restrict__ qrow, cplx* __restrict__ adjrhs,
@@ -362,18 +376,21 @@ k_rx_adjoint(MeshDev M, RxDev rx, SysMap sm, const double* __restrict__ freqs, c
     __syncthreads();
     // ---- responses, residual, misfit, receiver adjoints (serial over receivers: deterministic) ----
     __shared__ double phiSh;
+    const int nC = kTipper ? cm.nComp : sm.nModes;                 // data slots per (frequency, receiver)
+    const int zc = kTipper ? (mi == 0 ? cm.zc[0] : cm.zc[1]) : mi;    // this system's impedance component
     if (tid == 0) {
         double phi = 0.0;
-        for (int r = 0; r < rx.nRx; ++r) {
+        const int nRxZ = (kTipper && zc < 0) ? 0 : rx.nRx;
+        for (int r = 0; r < nRxZ; ++r) {
             const int id = rx.fid[r];
             const double d1 = rx.fdy1[r], d2 = rx.fdy2[r];
             cplx numF, denF;     // un-normalised interpolation used by the forward (mt2DTE.jl:196-207)
             if (mode == 0) { numF = F0[id - 1] * d2 + F0[id] * d1; denF = G0[id - 1] * d2 + G0[id] * d1; }
             else           { numF = G0[id - 1] * d2 + G0[id] * d1; denF = F0[id - 1] * d2 + F0[id] * d1; }
             cplx Z = numF / denF;
-            size_t di = (((size_t)ch * nFreq + f) * rx.nRx + r) * sm.nModes + mi;
+            size_t di = (((size_t)ch * nFreq + f) * rx.nRx + r) * nC + zc;
             pred[di] = Z;
-            size_t dob = ((size_t)f * rx.nRx + r) * sm.nModes + mi;     // obs / weights are shared by all chains
+            size_t dob = ((size_t)f * rx.nRx + r) * nC + zc;     // obs / weights are shared by all chains
             cplx d;
             if constexpr (kRhoPhase) {
                 // apparent resistivity and phase (compMTRespTE mt2DTE.jl:253-256, compMTRespTM mt2DTM.jl:236-239)
@@ -411,6 +428,32 @@ k_rx_adjoint(MeshDev M, RxDev rx, SysMap sm, const double* __restrict__ freqs, c
             } else {             // num <- Ey0, den <- F0
                 aG0[iL] += wl * nbar; aG0[iR] += wr * nbar;
                 aF0[iL] += wl * dbar; aF0[iR] += wr * dbar;
+            }
+        }
+        if constexpr (kTipper) {
+            const int tc = mi == cm.tmi ? cm.tc : -1;
+            for (int r = 0; tc >= 0 && r < rx.nRx; ++r) {
+                const int jL = rx.tjL[r], jR = rx.tjR[r], iL = rx.iL[r], iR = rx.iR[r];
+                const double vl = rx.twL[r], vr = rx.twR[r], wl = rx.wL[r], wr = rx.wR[r];
+                const cplx hzr = vl * ((F0[jL + 1] - F0[jL]) / M.yLen[jL] / iwmu) + vr * ((F0[jR + 1] - F0[jR]) / M.yLen[jR] / iwmu);
+                const cplx hyr = wl * G0[iL] + wr * G0[iR];
+                const cplx T = hzr / hyr;
+                const size_t di = (((size_t)ch * nFreq + f) * rx.nRx + r) * nC + tc;
+                pred[di] = T;
+                if (respKind == 1) resp[di] = T;                  // the response toggle keeps the tipper complex
+                const size_t dob = ((size_t)f * rx.nRx + r) * nC + tc;
+                const double w = wd[dob];
+                const cplx res = w * (T - obs[dob]);
+                phi += 0.5 * cabs2(res);
+                if (!wantAdjoint) continue;
+                if (w == 0.0 && !vin) continue;
+                const cplx d = cconj(vin ? vin[di] : w * res);
+                const cplx hzbar = d / hyr / iwmu;
+                const cplx aL = (vl / M.yLen[jL]) * hzbar, aR = (vr / M.yLen[jR]) * hzbar;
+                aF0[jL + 1] += aL; aF0[jL] -= aL;
+                aF0[jR + 1] += aR; aF0[jR] -= aR;
+                const cplx hybar = -(d * T / hyr);
+                aG0[iL] += wl * hybar; aG0[iR] += wr * hybar;
             }
         }
         phiSh = phi;

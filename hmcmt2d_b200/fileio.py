@@ -147,7 +147,7 @@ def readMT2DData(datafile: str):
             else:
                 obs = np.array([float(r[3]) for r in rows])
                 err = np.array([float(r[4]) for r in rows])
-    te = any("XY" in c for c in comps)
+    te = any("XY" in c or c == "TZY" for c in comps)            # the tipper TZY = Hz/Hy is a TE response
     tm = any("YX" in c for c in comps)
     mask = np.zeros((len(freqs), rx.shape[0], len(comps)), dtype=bool)      # vec(Bool[nDt,nRx,nFreq]) :165-172
     mask[fid - 1, rid - 1, did - 1] = True

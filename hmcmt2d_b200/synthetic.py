@@ -107,3 +107,24 @@ def rho_phase_problem(data: MTData, inv: InvDataModel, rho_err: float = 0.05, ph
     rp = MTData(np.array(data.rxLoc), np.array(data.freqs), "Rho_Pha", comps, np.repeat(rid, 2), np.repeat(fid, 2),
                 np.stack([2 * did - 1, 2 * did], axis=1).reshape(-1), mask, data.compTE, data.compTM)
     return rp, dataclasses.replace(inv, obsData=obs, dataW=1.0 / err, dataErr=err)
+
+
+def tipper_problem(data: MTData, inv: InvDataModel, tipper_obs, tipper_err: float = 0.02):
+    """The impedance survey `data` with tipper rows TZY = Hz/Hy added at every (frequency, receiver): `tipper_obs` [nFreq * nRx]
+    complex, frequency-major, and an absolute error `tipper_err` per row (the tipper vanishes over a layered earth, so an error
+    relative to |T| would give the rows of laterally uniform ground unbounded weights).  Rows in (freq, rx, comp) order.
+    -> (MTData with DataComp + [TZY], InvDataModel with the merged observations) with the model part of `inv` unchanged."""
+    if "Impedance" not in data.dataType or "TZY" in data.dataComp:
+        raise ValueError("tipper rows are added to an impedance survey without them")
+    nF, nRx, nC = len(data.freqs), np.asarray(data.rxLoc).shape[0], len(data.dataComp)
+    t = np.asarray(tipper_obs, dtype=np.complex128).reshape(nF * nRx)
+    fid = np.concatenate([data.freqID, np.repeat(np.arange(1, nF + 1), nRx)]).astype(np.int64)
+    rid = np.concatenate([data.rxID, np.tile(np.arange(1, nRx + 1), nF)]).astype(np.int64)
+    did = np.concatenate([data.dtID, np.full(nF * nRx, nC + 1)]).astype(np.int64)
+    obs = np.concatenate([np.asarray(inv.obsData, dtype=np.complex128), t])
+    err = np.concatenate([1.0 / np.asarray(inv.dataW, dtype=np.float64), np.full(nF * nRx, float(tipper_err))])
+    order = np.lexsort((did, rid, fid))
+    mask = np.concatenate([np.asarray(data.dataID, dtype=bool).reshape(nF, nRx, nC), np.ones((nF, nRx, 1), dtype=bool)], axis=2)
+    td = MTData(np.array(data.rxLoc), np.array(data.freqs), "Impedance", list(data.dataComp) + ["TZY"], rid[order], fid[order],
+                did[order], mask.reshape(-1), True, data.compTM)
+    return td, dataclasses.replace(inv, obsData=obs[order], dataW=1.0 / err[order], dataErr=err[order])

@@ -80,8 +80,10 @@ typedef struct hmcmt_problem {
     const double* freqs;      /* [nFreq] Hz */
     int32_t nRx;
     const double* rxLoc;      /* [nRx][2] row-major (y, z) */
-    int32_t nComp;            /* number of DataComp entries (1 or 2) */
-    const int32_t* compMode;  /* [nComp] 0 = ZXY (TE), 1 = ZYX (TM); reference order is [ZXY, ZYX] */
+    int32_t nComp;            /* number of DataComp entries (1 to 3) */
+    const int32_t* compMode;  /* [nComp] 0 = ZXY (TE), 1 = ZYX (TM), 2 = TZY (TE tipper, below); reference order is [ZXY, ZYX].
+                                 2 may appear once, as the last entry, after at most two impedance entries, and only in a plan of
+                                 hmcmt_plan_create; anything else returns -3 */
     int32_t nData;
     const int64_t* freqID;    /* [nData] 1-based, rows sorted by (freq, rx, comp) as the reference requires */
     const int64_t* rxID;      /* [nData] 1-based */
@@ -103,6 +105,20 @@ typedef struct hmcmt_problem {
 } hmcmt_problem;
 
 int hmcmt_plan_create(const hmcmt_problem* prob, hmcmt_plan** out);
+/* compMode 2 (TZY) is the vertical magnetic transfer function of the TE system, T = Hz/Hy, with the reference's conventions
+ * (e^{+i omega t}, z down, the Faraday sign of its Bz and Hy).  For frequency f and receiver r, with F0 = Ex on the receiver node
+ * row (the air/earth interface), yc_j the cell-centre y coordinates and Hy0 the surface field the impedance ZXY is formed from
+ * (compFieldsAtRxTE mt2DTE.jl:153-210, copied end values):
+ *   Hz0_j = (F0_{j+1} - F0_j) / (yLen_j i omega mu0)                  j = 0..ny-1, at yc_j    (Bz_0/mu0 of mt2DTE.jl)
+ *   Hzr   = wzL Hz0_{jL} + wzR Hz0_{jR},  (jL, jR, wzL, wzR) = linearInterp(y_r, yc)          (sensUtils.jl:133-161)
+ *   Hyr   = wL Hy0_{iL} + wR Hy0_{iR},    (iL, iR, wL, wR) = linearInterp(y_r, yNode)        (the normalised weights of the
+ *                                                                                             impedance sensitivities)
+ *   T     = Hzr / Hyr.
+ * ZXY and ZYX are computed exactly as without it.  A tipper row is a complex datum like an impedance: its misfit
+ * 1/2 |(T - T_obs)/|err||^2 is summed into phi_d, and its gradient is the derivative through the same adjoint solve, with the same
+ * boundary-condition approximations as the impedance gradient.  Every packed data array keeps its complex rows in place; the
+ * explicit Jacobian takes 2 nRx adjoint passes for the impedance components and 2 nRx more for the tipper (they share the TE
+ * system).  [TZY] alone or [ZYX, TZY] still solve the TE system, which then carries no impedance datum. */
 /* The same plan for apparent resistivity / phase data ("DataType: Rho_Pha", readMT2DData.jl:87), the same struct read with:
  *   obsData  [nData] real: rho_a = |Z|^2/(omega mu0) in Ohm m, or phase = atan2(Im Z, Re Z) in degrees;
  *   dataErr  [nData], weights 1/|err| per row;
@@ -113,7 +129,7 @@ int hmcmt_plan_create(const hmcmt_problem* prob, hmcmt_plan** out);
  * [..][nData] REAL (doubles): pred of hmcmt_forward / _sigma / _forward_gradient / _total / hmcmt_leapfrog_trajectory, v of
  * hmcmt_jtvec (gsig = sum_i v_i d pred_i / d sigma), J of hmcmt_jacobian ([nChains][nData][nAC]: d rho_a / d sigma and
  * d phase / d sigma rows) and hmcdata of hmcmt_run_chain.  hmcmt_get_responses returns the (rho_a, phase) pairs. */
-int hmcmt_plan_create_rho_phase(const hmcmt_problem* prob, hmcmt_plan** out);
+int hmcmt_plan_create_rho_phase(const hmcmt_problem* prob, hmcmt_plan** out);      /* compMode 2 (complex tipper rows): -3 */
 void hmcmt_destroy(hmcmt_plan* plan);
 /* sizes derived by the plan: n=0 N (unknowns/system), 1 nNode, 2 nCell, 3 nb, 4 half-bandwidth,
  * 5 tile-window T, 6 macro-steps S, 7 systems per chain, 8 receiver node row zid (0-based),
@@ -203,7 +219,8 @@ int hmcmt_status(hmcmt_plan* plan);
  * hmcmt_run_chain.  -40 if Wm is not positive definite. */
 int hmcmt_set_mass_matrix(hmcmt_plan* plan, int32_t kind);
 /* Response type of the forward evaluation of an impedance plan (compMTRespTE mt2DTE.jl:240-259, compMTRespTM mt2DTM.jl:224-242):
- * kind 0 = impedance, 1 = apparent resistivity rho_a = |Z|^2/(omega mu0) and phase atan2(Im Z, Re Z) in degrees.  A forward-only
+ * kind 0 = impedance, 1 = apparent resistivity rho_a = |Z|^2/(omega mu0) and phase atan2(Im Z, Re Z) in degrees (tipper slots keep
+ * (Re T, Im T)).  A forward-only
  * toggle: the misfit and gradients of such a plan stay those of its impedance data (evaluations with kind 1 are launched eagerly,
  * outside the captured graph).  Gradients of rho / phase data come from a plan made by hmcmt_plan_create_rho_phase.
  * hmcmt_get_responses copies the responses of the last forward evaluation, unmasked:

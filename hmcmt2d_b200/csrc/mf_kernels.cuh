@@ -704,15 +704,18 @@ __global__ void mf_mt_vals_kernel(int N, const MtValSys* __restrict__ sysv, cplx
 
 // ------------------------------------------------------------------------------------------------------------------------
 // solves.  One CTA per (front, right-hand side); vec = blockIdx.y indexes (system, rhs): sys = vec / nrhs.
-//   v   : [nvec][Np]  forward: pivot parts of the eliminated rhs; backward: overwritten by the solution (padded permuted numbering)
-//   upd : [nvec][updEntries] update vectors handed from the children to their parent
+//   v   : pivot parts of the eliminated rhs (forward), overwritten by the solution (backward), padded permuted numbering;
+//         vector `vec` at v + vec*vStride
+//   upd : update vectors handed from the children to their parent, vector `vec` at upd + vec*uStride
+// The solver's workspace holds maxRhs slots per system (Solver::solve_args): a call with one vector per system strides over
+// the other slots, so that a solve on slot 1 leaves the slot-0 vectors of the same systems intact.
 struct SolveArgs {
     const cplx* B;      // right-hand sides, original numbering, vector `vec` at B + vec*ldb
     cplx* X;            // solutions, same layout (may alias B)
     int64_t ldb, ldx;
     cplx* v;
     cplx* upd;
-    int64_t Np, updEntries;
+    int64_t vStride, uStride;
     int nrhs;
 };
 constexpr int kSolveMfThreads = 256;      // upper bound; launched with 128 threads where no front of the depth exceeds 144 rows
@@ -725,8 +728,8 @@ mf_fwd_kernel(Tables tb, SolveArgs sa, const int* __restrict__ list) {
     const int vec = blockIdx.y, sys = vec / sa.nrhs, tid = threadIdx.x, nthr = blockDim.x;
     const int fp = F.sp + F.up;
     const cplx* b = sa.B + (size_t)vec * sa.ldb;
-    cplx* v = sa.v + (size_t)vec * sa.Np;
-    cplx* upd = sa.upd + (size_t)vec * sa.updEntries;
+    cplx* v = sa.v + (size_t)vec * sa.vStride;
+    cplx* upd = sa.upd + (size_t)vec * sa.uStride;
     for (int i = tid; i < fp; i += nthr) {
         cplx x = mk(0.0, 0.0);
         if (i < F.s) x = b[tb.pos2orig[F.cbp + i]];
@@ -767,22 +770,26 @@ mf_fwd_kernel(Tables tb, SolveArgs sa, const int* __restrict__ list) {
     for (int i = tid; i < F.up; i += nthr) upd[F.updOff + i] = w[F.sp + i];
 }
 
-__global__ void __launch_bounds__(kSolveMfThreads)
-mf_bwd_kernel(Tables tb, SolveArgs sa, const int* __restrict__ list) {
-    extern __shared__ __align__(16) unsigned char mf_smem[];
-    const Front F = tb.fronts[list[blockIdx.x]];
-    const int vec = blockIdx.y, sys = vec / sa.nrhs, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nthr = blockDim.x;
+// Backward substitution of one front for NV vectors of the same system: every G / M element is loaded once and applied to all
+// of them, each vector with exactly the arithmetic of the single-vector sweep.  xf[t]: [fp] then the stage tmp[t]: [largest chunk].
+template <int NV>
+__device__ __forceinline__ void mf_bwd_front(const Tables& tb, const Front& F, int sys, cplx* const (&v)[NV], cplx* const (&x)[NV],
+                                             cplx* smem) {
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nthr = blockDim.x;
     const int fp = F.sp + F.up;
-    cplx* xf = reinterpret_cast<cplx*>(mf_smem);        // [fp]
-    cplx* tmp = xf + fp;                                 // [kChunkMax or sp]
-    cplx* v = sa.v + (size_t)vec * sa.Np;
-    cplx* x = sa.X + (size_t)vec * sa.ldx;
+    cplx* xf[NV];
+    cplx* tmp[NV];
+#pragma unroll
+    for (int t = 0; t < NV; ++t) { xf[t] = smem + t * fp; tmp[t] = smem + NV * fp + t * F.sp; }
     const int* rows = tb.rows + F.rowPtr;
     for (int i = tid; i < fp; i += nthr) {
-        cplx val = mk(0.0, 0.0);
-        if (i < F.sp) val = v[F.cbp + i];
-        else if (i - F.sp < F.u) val = v[rows[i - F.sp]];
-        xf[i] = val;
+#pragma unroll
+        for (int t = 0; t < NV; ++t) {
+            cplx val = mk(0.0, 0.0);
+            if (i < F.sp) val = v[t][F.cbp + i];
+            else if (i - F.sp < F.u) val = v[t][rows[i - F.sp]];
+            xf[t][i] = val;
+        }
     }
     __syncthreads();
     const double* fac = tb.fac + (size_t)sys * tb.facStride;
@@ -794,44 +801,91 @@ mf_bwd_kernel(Tables tb, SolveArgs sa, const int* __restrict__ list) {
         const double* M = fac + ch.mOff;
         // x1[k] = sum_j G[j][k] w1[j] - sum_i M[i][k] x2[i] : one warp per group of four k
         for (int kg = warp; kg < (sc >> 2); kg += NWS) {
-            cplx a0 = mk(0.0, 0.0), a1 = a0, a2 = a0, a3 = a0;
+            cplx a0[NV], a1[NV], a2[NV], a3[NV];
+#pragma unroll
+            for (int t = 0; t < NV; ++t) a0[t] = a1[t] = a2[t] = a3[t] = mk(0.0, 0.0);
             for (int j = lane; j < sc; j += 32) {
                 const double* pr = G + kg_off(sc, j, 4 * kg, 0);
                 const double* pi = G + kg_off(sc, j, 4 * kg, 1);
                 const double2 r01 = *reinterpret_cast<const double2*>(pr), r23 = *reinterpret_cast<const double2*>(pr + 2);
                 const double2 i01 = *reinterpret_cast<const double2*>(pi), i23 = *reinterpret_cast<const double2*>(pi + 2);
-                const cplx wj = xf[ch.p0 + j];
-                cfma(a0, mk(r01.x, i01.x), wj); cfma(a1, mk(r01.y, i01.y), wj);
-                cfma(a2, mk(r23.x, i23.x), wj); cfma(a3, mk(r23.y, i23.y), wj);
+#pragma unroll
+                for (int t = 0; t < NV; ++t) {
+                    const cplx wj = xf[t][ch.p0 + j];
+                    cfma(a0[t], mk(r01.x, i01.x), wj); cfma(a1[t], mk(r01.y, i01.y), wj);
+                    cfma(a2[t], mk(r23.x, i23.x), wj); cfma(a3[t], mk(r23.y, i23.y), wj);
+                }
             }
             for (int i = lane; i < mr; i += 32) {
                 const double* pr = M + kg_off(mr, i, 4 * kg, 0);
                 const double* pi = M + kg_off(mr, i, 4 * kg, 1);
                 const double2 r01 = *reinterpret_cast<const double2*>(pr), r23 = *reinterpret_cast<const double2*>(pr + 2);
                 const double2 i01 = *reinterpret_cast<const double2*>(pi), i23 = *reinterpret_cast<const double2*>(pi + 2);
-                const cplx xi = -xf[ch.p1 + i];
-                cfma(a0, mk(r01.x, i01.x), xi); cfma(a1, mk(r01.y, i01.y), xi);
-                cfma(a2, mk(r23.x, i23.x), xi); cfma(a3, mk(r23.y, i23.y), xi);
+#pragma unroll
+                for (int t = 0; t < NV; ++t) {
+                    const cplx xi = -xf[t][ch.p1 + i];
+                    cfma(a0[t], mk(r01.x, i01.x), xi); cfma(a1[t], mk(r01.y, i01.y), xi);
+                    cfma(a2[t], mk(r23.x, i23.x), xi); cfma(a3[t], mk(r23.y, i23.y), xi);
+                }
             }
 #pragma unroll
-            for (int off = 16; off >= 1; off >>= 1) {
-                a0.x += __shfl_xor_sync(0xffffffffu, a0.x, off); a0.y += __shfl_xor_sync(0xffffffffu, a0.y, off);
-                a1.x += __shfl_xor_sync(0xffffffffu, a1.x, off); a1.y += __shfl_xor_sync(0xffffffffu, a1.y, off);
-                a2.x += __shfl_xor_sync(0xffffffffu, a2.x, off); a2.y += __shfl_xor_sync(0xffffffffu, a2.y, off);
-                a3.x += __shfl_xor_sync(0xffffffffu, a3.x, off); a3.y += __shfl_xor_sync(0xffffffffu, a3.y, off);
+            for (int t = 0; t < NV; ++t) {
+#pragma unroll
+                for (int off = 16; off >= 1; off >>= 1) {
+                    a0[t].x += __shfl_xor_sync(0xffffffffu, a0[t].x, off); a0[t].y += __shfl_xor_sync(0xffffffffu, a0[t].y, off);
+                    a1[t].x += __shfl_xor_sync(0xffffffffu, a1[t].x, off); a1[t].y += __shfl_xor_sync(0xffffffffu, a1[t].y, off);
+                    a2[t].x += __shfl_xor_sync(0xffffffffu, a2[t].x, off); a2[t].y += __shfl_xor_sync(0xffffffffu, a2[t].y, off);
+                    a3[t].x += __shfl_xor_sync(0xffffffffu, a3[t].x, off); a3[t].y += __shfl_xor_sync(0xffffffffu, a3[t].y, off);
+                }
+                if (lane == 0) { tmp[t][4 * kg] = a0[t]; tmp[t][4 * kg + 1] = a1[t]; tmp[t][4 * kg + 2] = a2[t]; tmp[t][4 * kg + 3] = a3[t]; }
             }
-            if (lane == 0) { tmp[4 * kg] = a0; tmp[4 * kg + 1] = a1; tmp[4 * kg + 2] = a2; tmp[4 * kg + 3] = a3; }
         }
         __syncthreads();
-        for (int k = tid; k < sc; k += nthr) xf[ch.p0 + k] = tmp[k];
+        for (int k = tid; k < sc; k += nthr) {
+#pragma unroll
+            for (int t = 0; t < NV; ++t) xf[t][ch.p0 + k] = tmp[t][k];
+        }
         __syncthreads();
     }
     for (int i = tid; i < F.sp; i += nthr) {
-        v[F.cbp + i] = xf[i];
-        if (i < F.s) x[tb.pos2orig[F.cbp + i]] = xf[i];
+#pragma unroll
+        for (int t = 0; t < NV; ++t) {
+            v[t][F.cbp + i] = xf[t][i];
+            if (i < F.s) x[t][tb.pos2orig[F.cbp + i]] = xf[t][i];
+        }
     }
 }
 
+__global__ void __launch_bounds__(kSolveMfThreads)
+mf_bwd_kernel(Tables tb, SolveArgs sa, const int* __restrict__ list) {
+    extern __shared__ __align__(16) unsigned char mf_smem[];
+    const Front F = tb.fronts[list[blockIdx.x]];
+    const int vec = blockIdx.y, sys = vec / sa.nrhs;
+    cplx* const v[1] = {sa.v + (size_t)vec * sa.vStride};
+    cplx* const x[1] = {sa.X + (size_t)vec * sa.ldx};
+    mf_bwd_front<1>(tb, F, sys, v, x, reinterpret_cast<cplx*>(mf_smem));
+}
+
+// Paired backward substitution: one CTA per (front, system) solves vector a and vector b of the system (nrhs = 1 each) with one
+// pass over the front's factor.  list[0, nBoth): both vectors; list[nBoth, n): vector b only (fronts whose pivot part of a
+// already holds the solution — back-substituting it again would start from the solution instead of the eliminated rhs).
+__global__ void __launch_bounds__(kSolveMfThreads)
+mf_bwd_pair_kernel(Tables tb, SolveArgs sa, SolveArgs sb, const int* __restrict__ list, int nBoth) {
+    extern __shared__ __align__(16) unsigned char mf_smem[];
+    const Front F = tb.fronts[list[blockIdx.x]];
+    const int sys = blockIdx.y;
+    cplx* const vb = sb.v + (size_t)sys * sb.vStride;
+    cplx* const xb = sb.X + (size_t)sys * sb.ldx;
+    if ((int)blockIdx.x < nBoth) {
+        cplx* const v[2] = {sa.v + (size_t)sys * sa.vStride, vb};
+        cplx* const x[2] = {sa.X + (size_t)sys * sa.ldx, xb};
+        mf_bwd_front<2>(tb, F, sys, v, x, reinterpret_cast<cplx*>(mf_smem));
+    } else {
+        cplx* const v[1] = {vb};
+        cplx* const x[1] = {xb};
+        mf_bwd_front<1>(tb, F, sys, v, x, reinterpret_cast<cplx*>(mf_smem));
+    }
+}
 
 // Small fronts (single chunk, fp <= kSolveSmallMax): one WARP per (front, right-hand side), eight fronts per CTA, warp-level
 // synchronisation only.  descs[blockIdx.x * 8 + warp] = the front's record: every later load depends on it alone or on one
@@ -850,8 +904,8 @@ mf_fwd_warp_kernel(Tables tb, SolveArgs sa, const SolveDesc* __restrict__ descs,
     const int sp = D.sp, up = D.up, fp = sp + up, fs = D.s, fu = D.u, cbp = D.cbp;
     cplx* w = wsh[warp];
     const cplx* b = sa.B + (size_t)vec * sa.ldb;
-    cplx* v = sa.v + (size_t)vec * sa.Np;
-    cplx* upd = sa.upd + (size_t)vec * sa.updEntries;
+    cplx* v = sa.v + (size_t)vec * sa.vStride;
+    cplx* upd = sa.upd + (size_t)vec * sa.uStride;
     // (a) requests that need the record only: own right-hand-side rows (through pos2orig), the children's row maps and update vectors
     int orow[2];
 #pragma unroll
@@ -897,20 +951,13 @@ mf_fwd_warp_kernel(Tables tb, SolveArgs sa, const SolveDesc* __restrict__ descs,
     for (int i = lane; i < sp; i += 32) v[cbp + i] = w[i];
 }
 
-// Backward substitution, one warp per front.  (Fetching the front's contiguous [G | M] block whole into a shared-memory stage
-// with cp.async was measured: no faster than the direct loads below at any stage size, and slower once the stage costs occupancy.)
-__global__ void __launch_bounds__(kSolveWarpsPerCta * 32)
-mf_bwd_warp_kernel(Tables tb, SolveArgs sa, const SolveDesc* __restrict__ descs, int n) {
-    __shared__ cplx xsh[kSolveWarpsPerCta][kSolveSmallMax];
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int fi = blockIdx.x * kSolveWarpsPerCta + warp;
-    if (fi >= n) return;
-    const SolveDesc& D = descs[fi];                // (fields are read as needed; the row indices ride in the same record)
-    const int vec = blockIdx.y, sys = vec / sa.nrhs;
+// Backward substitution of one front by one warp for NV vectors of the same system (each G / M element loaded once, applied
+// to every vector with the arithmetic of the single-vector sweep); xf[t]: the warp's [kSolveSmallMax] stage of vector t.
+template <int NV>
+__device__ __forceinline__ void mf_bwd_warp_front(const Tables& tb, const SolveDesc& D, int sys, cplx* const (&v)[NV], cplx* const (&x)[NV],
+                                                  cplx* const (&xf)[NV]) {
+    const int lane = threadIdx.x & 31;
     const int sp = D.sp, up = D.up, fs = D.s, fu = D.u, cbp = D.cbp;
-    cplx* xf = xsh[warp];
-    cplx* v = sa.v + (size_t)vec * sa.Np;
-    cplx* x = sa.X + (size_t)vec * sa.ldx;
     const int* rows = tb.rows + D.rowPtr;
     const double* G = tb.fac + (size_t)sys * tb.facStride + D.gOff;
     const double* M = tb.fac + (size_t)sys * tb.facStride + D.mOff;
@@ -921,35 +968,98 @@ mf_bwd_warp_kernel(Tables tb, SolveArgs sa, const SolveDesc* __restrict__ descs,
         const int i = lane + 32 * h;
         urow[h] = i < fu ? (i < kDescRows ? D.rows[i] : rows[i]) : -1;
     }
-    if (lane < sp) xf[lane] = v[cbp + lane];
-    if (lane + 32 < sp) xf[lane + 32] = v[cbp + lane + 32];
+#pragma unroll
+    for (int t = 0; t < NV; ++t) {
+        if (lane < sp) xf[t][lane] = v[t][cbp + lane];
+        if (lane + 32 < sp) xf[t][lane + 32] = v[t][cbp + lane + 32];
+    }
     // x1[k] = sum_j G[j][k] w1[j] - sum_i M[i][k] x2[i] : one lane per k; when the front has fewer than 32 pivots the rows are
     // split over 32 / width sub-groups of lanes and combined with shuffles.  Only the real pivots / update rows are visited: the
     // identity padding is never read back by anybody.
     const int width = fs <= 8 ? 8 : (fs <= 16 ? 16 : 32), nparts = 32 / width, part = lane / width, kl = lane - part * width;
     const int orig0 = (kl < fs && part == 0) ? tb.pos2orig[cbp + kl] : -1;      // (fronts of at most 32 pivots: the common case)
 #pragma unroll
-    for (int h = 0; h < 2; ++h) if (urow[h] >= 0) xf[sp + lane + 32 * h] = v[urow[h]];
+    for (int t = 0; t < NV; ++t)
+#pragma unroll
+        for (int h = 0; h < 2; ++h) if (urow[h] >= 0) xf[t][sp + lane + 32 * h] = v[t][urow[h]];
     __syncwarp();
     for (int k0 = 0; k0 < fs; k0 += width) {
         const int k = k0 + kl;
-        cplx acc = mk(0.0, 0.0);
+        cplx acc[NV];
+#pragma unroll
+        for (int t = 0; t < NV; ++t) acc[t] = mk(0.0, 0.0);
         if (k < fs) {
             const double* gr = G + kg_off(sp, 0, k, 0);
             const double* gi = G + kg_off(sp, 0, k, 1);
-            for (int j = part; j < fs; j += nparts) cfma(acc, mk(gr[4 * j], gi[4 * j]), xf[j]);
+            for (int j = part; j < fs; j += nparts) {
+                const cplx g = mk(gr[4 * j], gi[4 * j]);
+#pragma unroll
+                for (int t = 0; t < NV; ++t) cfma(acc[t], g, xf[t][j]);
+            }
             const double* mr = M + kg_off(up, 0, k, 0);
             const double* mi = M + kg_off(up, 0, k, 1);
-            for (int i = part; i < fu; i += nparts) cfma(acc, mk(-mr[4 * i], -mi[4 * i]), xf[sp + i]);
+            for (int i = part; i < fu; i += nparts) {
+                const cplx m = mk(-mr[4 * i], -mi[4 * i]);
+#pragma unroll
+                for (int t = 0; t < NV; ++t) cfma(acc[t], m, xf[t][sp + i]);
+            }
         }
         for (int off = width; off < 32; off <<= 1) {
-            acc.x += __shfl_xor_sync(0xffffffffu, acc.x, off);
-            acc.y += __shfl_xor_sync(0xffffffffu, acc.y, off);
+#pragma unroll
+            for (int t = 0; t < NV; ++t) {
+                acc[t].x += __shfl_xor_sync(0xffffffffu, acc[t].x, off);
+                acc[t].y += __shfl_xor_sync(0xffffffffu, acc[t].y, off);
+            }
         }
         if (k < fs && part == 0) {
-            v[cbp + k] = acc;
-            x[k0 == 0 ? orig0 : tb.pos2orig[cbp + k]] = acc;
+            const int o = k0 == 0 ? orig0 : tb.pos2orig[cbp + k];
+#pragma unroll
+            for (int t = 0; t < NV; ++t) {
+                v[t][cbp + k] = acc[t];
+                x[t][o] = acc[t];
+            }
         }
+    }
+}
+
+// Backward substitution, one warp per front.  (Fetching the front's contiguous [G | M] block whole into a shared-memory stage
+// with cp.async was measured: no faster than the direct loads below at any stage size, and slower once the stage costs occupancy.)
+__global__ void __launch_bounds__(kSolveWarpsPerCta * 32)
+mf_bwd_warp_kernel(Tables tb, SolveArgs sa, const SolveDesc* __restrict__ descs, int n) {
+    __shared__ cplx xsh[kSolveWarpsPerCta][kSolveSmallMax];
+    const int warp = threadIdx.x >> 5;
+    const int fi = blockIdx.x * kSolveWarpsPerCta + warp;
+    if (fi >= n) return;
+    const SolveDesc& D = descs[fi];                // (fields are read as needed; the row indices ride in the same record)
+    const int vec = blockIdx.y, sys = vec / sa.nrhs;
+    cplx* const v[1] = {sa.v + (size_t)vec * sa.vStride};
+    cplx* const x[1] = {sa.X + (size_t)vec * sa.ldx};
+    cplx* const xf[1] = {xsh[warp]};
+    mf_bwd_warp_front<1>(tb, D, sys, v, x, xf);
+}
+
+// Paired backward substitution, one warp per (front, system) for vectors a and b: descs[0, nBoth) both, descs[nBoth, n) b only
+// (see mf_bwd_pair_kernel).
+__global__ void __launch_bounds__(kSolveWarpsPerCta * 32, 4)
+mf_bwd_pair_warp_kernel(Tables tb, SolveArgs sa, SolveArgs sb, const SolveDesc* __restrict__ descs, int n, int nBoth) {
+    __shared__ cplx xsh[2][kSolveWarpsPerCta][kSolveSmallMax];
+    const int warp = threadIdx.x >> 5;
+    const int fi = blockIdx.x * kSolveWarpsPerCta + warp;
+    if (fi >= n) return;
+    const SolveDesc& D = descs[fi];
+    const int sys = blockIdx.y;
+    cplx* const vb = sb.v + (size_t)sys * sb.vStride;
+    cplx* const xb = sb.X + (size_t)sys * sb.ldx;
+    if (fi < nBoth) {
+        cplx* const v[2] = {sa.v + (size_t)sys * sa.vStride, vb};
+        cplx* const x[2] = {sa.X + (size_t)sys * sa.ldx, xb};
+        cplx* const xf[2] = {xsh[0][warp], xsh[1][warp]};
+        mf_bwd_warp_front<2>(tb, D, sys, v, x, xf);
+    } else {
+        cplx* const v[1] = {vb};
+        cplx* const x[1] = {xb};
+        cplx* const xf[1] = {xsh[1][warp]};
+        mf_bwd_warp_front<1>(tb, D, sys, v, x, xf);
     }
 }
 

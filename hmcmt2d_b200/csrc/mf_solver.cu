@@ -260,6 +260,11 @@ int Solver::build(int nsys_, int maxRhs_, int64_t valCount_) {
     MF_TRY(upload(invMapsHost, &d_invMaps));
     solveSmem = (size_t)(2 * S.maxFp + 16) * sizeof(cplx);
     if (solveSmem > kMaxSmem) return kErrArg;
+    {
+        int mx = 0;
+        for (const Front& F : S.fronts) if (!solve_by_warp(F)) mx = std::max(mx, F.fp() + F.sp);
+        pairSmem = (size_t)2 * mx * sizeof(cplx);      // (checked by backward_pair, the only user)
+    }
 #undef MF_TRY
     return kOk;
 }
@@ -343,13 +348,19 @@ int Solver::add_rhs_pattern(const std::vector<unsigned char>& nz) {
         }
         if (active[k] && F.parent >= 0) active[F.parent] = 1;
     }
-    FwdLists L;
+    PatternLists L;
     int rc;
 #define MF_TRY(x) do { rc = (x); if (rc) return rc; } while (0)
     for (int d = 0; d <= S.maxDepth; ++d) {
-        std::vector<int> sw, sc;
+        std::vector<int> sw, sc, pw, pc;      // active set; all fronts, inactive first (backward_pair)
         for (int k : S.byDepthBig[d]) if (active[k]) sc.push_back(k);
         for (int k : S.byDepthSmall[d]) if (active[k]) (solve_by_warp(S.fronts[k]) ? sw : sc).push_back(k);
+        for (int k : S.byDepthBig[d]) if (!active[k]) pc.push_back(k);
+        for (int k : S.byDepthSmall[d]) if (!active[k]) (solve_by_warp(S.fronts[k]) ? pw : pc).push_back(k);
+        L.nPairWarpBoth.push_back((int)pw.size());
+        L.nPairCtaBoth.push_back((int)pc.size());
+        pw.insert(pw.end(), sw.begin(), sw.end());
+        pc.insert(pc.end(), sc.begin(), sc.end());
         const SolveDesc* pd = nullptr;
         if (!sw.empty()) MF_TRY(upload_solve_descs(sw, &pd));
         L.warpList.push_back(pd);
@@ -359,6 +370,12 @@ int Solver::add_rhs_pattern(const std::vector<unsigned char>& nz) {
         L.ctaList.push_back(sc.empty() ? nullptr : p);
         L.nCta.push_back((int)sc.size());
         L.nFronts += (int)(sw.size() + sc.size());
+        pd = nullptr;
+        if (!pw.empty()) MF_TRY(upload_solve_descs(pw, &pd));
+        L.pairWarpList.push_back(pd);
+        p = nullptr;
+        if (!pc.empty()) MF_TRY(upload(pc, &p));
+        L.pairCtaList.push_back(p);
     }
 #undef MF_TRY
     patterns.push_back(std::move(L));
@@ -369,35 +386,49 @@ int Solver::fwd_fronts(int pattern) const {
     return pattern >= 1 && pattern <= (int)patterns.size() ? patterns[pattern - 1].nFronts : S.K;
 }
 
-int Solver::solve(cudaStream_t st, int nrhs, const cplx* B, int64_t ldb, cplx* X, int64_t ldx, int64_t* nLaunches, int sys0, int n,
-                  int pattern) {
-    if (nrhs < 1 || nrhs > maxRhs || pattern < 0 || pattern > (int)patterns.size()) return kErrArg;
-    if (n < 0) n = this->nsys - sys0;
-    if (sys0 < 0 || n < 1 || sys0 + n > this->nsys) return kErrArg;
-    const int nsys = n;
+Tables Solver::tables(int sys0) const {
     Tables tb{};
     tb.fronts = d_fronts; tb.rows = d_rows; tb.rel = d_rel; tb.children = d_children; tb.orig = d_orig; tb.chunks = d_chunks;
     tb.pos2orig = d_pos2orig; tb.fac = d_fac + (size_t)sys0 * S.factorDoubles;
     tb.arena[0] = d_arena[0] + (size_t)sys0 * S.arenaDoubles[0]; tb.arena[1] = d_arena[1] + (size_t)sys0 * S.arenaDoubles[1];
     tb.facStride = S.factorDoubles; tb.arenaStride[0] = S.arenaDoubles[0]; tb.arenaStride[1] = S.arenaDoubles[1];
     tb.vals = d_vals; tb.valStride = valCount; tb.status = nullptr; tb.prof = nullptr;
-    const size_t vec0 = (size_t)sys0 * nrhs;
-    // the workspaces are laid out for maxRhs vectors per system
-    SolveArgs sa{B + vec0 * ldb, X + vec0 * ldx, ldb, ldx, d_v + (size_t)sys0 * maxRhs * S.Np, d_upd + (size_t)sys0 * maxRhs * S.updEntries,
-                 (int64_t)S.Np, S.updEntries, nrhs};
+    return tb;
+}
+
+// vectors (sys0 + s, r) of a call: right-hand side / solution at B / X + (s*nrhs + r)*ld.  Workspace: from slot `slot` of
+// system sys0 on, consecutive vectors of the call are one slot apart when nrhs > 1 (all calls that pass nrhs > 1 cover their
+// systems' slots 0 .. nrhs-1) and one system apart when nrhs == 1 (slot `slot` of every system).
+SolveArgs Solver::solve_args(const cplx* B, int64_t ldb, cplx* X, int64_t ldx, int sys0, int nrhs, int slot) const {
+    const size_t vec0 = (size_t)sys0 * nrhs, ws0 = (size_t)sys0 * maxRhs + slot;
+    const int64_t per = nrhs == 1 ? maxRhs : 1;
+    return SolveArgs{B ? B + vec0 * ldb : nullptr, X ? X + vec0 * ldx : nullptr, ldb, ldx, d_v + ws0 * S.Np, d_upd + ws0 * S.updEntries,
+                     per * S.Np, per * S.updEntries, nrhs};
+}
+
+int Solver::set_solve_attributes() {
     static PerDeviceOnceMf once;
     if (once.need()) {
         HMCMT_CUDA_TRY(cudaFuncSetAttribute(mf_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxSmem));
         HMCMT_CUDA_TRY(cudaFuncSetAttribute(mf_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxSmem));
+        HMCMT_CUDA_TRY(cudaFuncSetAttribute(mf_bwd_pair_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxSmem));
     }
-    const int nvec = nsys * nrhs;
-    int64_t nl = 0;
-    const FwdLists* P = pattern ? &patterns[pattern - 1] : nullptr;
-    if (P) {
-        // fronts outside the pattern are not visited: their pivot parts and update vectors are zero
-        HMCMT_CUDA_TRY(cudaMemsetAsync(sa.v, 0, (size_t)nvec * S.Np * sizeof(cplx), st));
-        HMCMT_CUDA_TRY(cudaMemsetAsync(sa.upd, 0, (size_t)nvec * S.updEntries * sizeof(cplx), st));
+    return kOk;
+}
+
+// zero the workspace vectors of a call (sa: solve_args): the fronts a pruned forward elimination does not visit hold zero pivot
+// parts and update vectors
+int Solver::clear_ws(cudaStream_t st, const SolveArgs& sa, int nvec) {
+    const struct { cplx* p; int64_t len, stride; } ws[2] = {{sa.v, (int64_t)S.Np, sa.vStride}, {sa.upd, S.updEntries, sa.uStride}};
+    for (const auto& w : ws) {
+        if (w.stride == w.len) HMCMT_CUDA_TRY(cudaMemsetAsync(w.p, 0, (size_t)nvec * w.len * sizeof(cplx), st));
+        else HMCMT_CUDA_TRY(cudaMemset2DAsync(w.p, (size_t)w.stride * sizeof(cplx), 0, (size_t)w.len * sizeof(cplx), nvec, st));
     }
+    return kOk;
+}
+
+int Solver::fwd_sweep(cudaStream_t st, const Tables& tb, const SolveArgs& sa, int nvec, int pattern, int64_t& nl) {
+    const PatternLists* P = pattern ? &patterns[pattern - 1] : nullptr;
     for (int d = S.maxDepth; d >= 0; --d) {
         const DepthSchedule& D = sched[d];
         const int nW = P ? P->nWarp[d] : D.nSolveWarp, nC = P ? P->nCta[d] : D.nSolveCta;
@@ -412,6 +443,23 @@ int Solver::solve(cudaStream_t st, int nrhs, const cplx* B, int64_t ldb, cplx* X
             ++nl;
         }
     }
+    return kOk;
+}
+
+int Solver::solve(cudaStream_t st, int nrhs, const cplx* B, int64_t ldb, cplx* X, int64_t ldx, int64_t* nLaunches, int sys0, int n,
+                  int pattern) {
+    if (nrhs < 1 || nrhs > maxRhs || pattern < 0 || pattern > (int)patterns.size()) return kErrArg;
+    if (n < 0) n = this->nsys - sys0;
+    if (sys0 < 0 || n < 1 || sys0 + n > this->nsys) return kErrArg;
+    int rc = set_solve_attributes();
+    if (rc) return rc;
+    const Tables tb = tables(sys0);
+    const SolveArgs sa = solve_args(B, ldb, X, ldx, sys0, nrhs, 0);
+    const int nvec = n * nrhs;
+    int64_t nl = 0;
+    // fronts outside the pattern are not visited: their pivot parts and update vectors are zero
+    if (pattern && (rc = clear_ws(st, sa, nvec))) return rc;
+    fwd_sweep(st, tb, sa, nvec, pattern, nl);
     for (int d = 0; d <= S.maxDepth; ++d) {
         const DepthSchedule& D = sched[d];
         if (D.nSolveWarp) {
@@ -421,6 +469,74 @@ int Solver::solve(cudaStream_t st, int nrhs, const cplx* B, int64_t ldb, cplx* X
         }
         if (D.nSolveCta) {
             mf_bwd_kernel<<<dim3(D.nSolveCta, nvec), D.solveCtaThreads, solveSmem, st>>>(tb, sa, D.solveCtaList);
+            ++nl;
+        }
+    }
+    HMCMT_CUDA_TRY(cudaGetLastError());
+    if (nLaunches) *nLaunches += nl;
+    return kOk;
+}
+
+int Solver::forward_slot(cudaStream_t st, int slot, const cplx* B, int64_t ldb, int64_t* nLaunches, int sys0, int n, int pattern) {
+    if (slot < 0 || slot >= maxRhs || pattern < 0 || pattern > (int)patterns.size()) return kErrArg;
+    if (n < 0) n = this->nsys - sys0;
+    if (sys0 < 0 || n < 1 || sys0 + n > this->nsys) return kErrArg;
+    int rc = set_solve_attributes();
+    if (rc) return rc;
+    const SolveArgs sa = solve_args(B, ldb, nullptr, 0, sys0, 1, slot);
+    int64_t nl = 0;
+    if (pattern && (rc = clear_ws(st, sa, n))) return rc;
+    fwd_sweep(st, tables(sys0), sa, n, pattern, nl);
+    HMCMT_CUDA_TRY(cudaGetLastError());
+    if (nLaunches) *nLaunches += nl;
+    return kOk;
+}
+
+int Solver::backward_slot(cudaStream_t st, int slot, cplx* X, int64_t ldx, int64_t* nLaunches, int sys0, int n, int pattern) {
+    if (slot < 0 || slot >= maxRhs || pattern < 1 || pattern > (int)patterns.size()) return kErrArg;
+    if (n < 0) n = this->nsys - sys0;
+    if (sys0 < 0 || n < 1 || sys0 + n > this->nsys) return kErrArg;
+    int rc = set_solve_attributes();
+    if (rc) return rc;
+    const Tables tb = tables(sys0);
+    const SolveArgs sa = solve_args(nullptr, 0, X, ldx, sys0, 1, slot);
+    const PatternLists& P = patterns[pattern - 1];
+    int64_t nl = 0;
+    for (int d = 0; d <= S.maxDepth; ++d) {
+        if (const int nW = P.nWarp[d]) {
+            mf_bwd_warp_kernel<<<dim3((nW + kSolveWarpsPerCta - 1) / kSolveWarpsPerCta, n), kSolveWarpsPerCta * 32, 0, st>>>(
+                tb, sa, P.warpList[d], nW);
+            ++nl;
+        }
+        if (const int nC = P.nCta[d]) {
+            mf_bwd_kernel<<<dim3(nC, n), sched[d].solveCtaThreads, solveSmem, st>>>(tb, sa, P.ctaList[d]);
+            ++nl;
+        }
+    }
+    HMCMT_CUDA_TRY(cudaGetLastError());
+    if (nLaunches) *nLaunches += nl;
+    return kOk;
+}
+
+int Solver::backward_pair(cudaStream_t st, cplx* Xa, cplx* Xb, int64_t ldx, int64_t* nLaunches, int sys0, int n, int done) {
+    if (maxRhs < 2 || done < 1 || done > (int)patterns.size() || pairSmem > kMaxSmem) return kErrArg;
+    if (n < 0) n = this->nsys - sys0;
+    if (sys0 < 0 || n < 1 || sys0 + n > this->nsys) return kErrArg;
+    int rc = set_solve_attributes();
+    if (rc) return rc;
+    const Tables tb = tables(sys0);
+    const SolveArgs sa = solve_args(nullptr, 0, Xa, ldx, sys0, 1, 0), sb = solve_args(nullptr, 0, Xb, ldx, sys0, 1, 1);
+    const PatternLists& P = patterns[done - 1];
+    int64_t nl = 0;
+    for (int d = 0; d <= S.maxDepth; ++d) {
+        const DepthSchedule& D = sched[d];
+        if (D.nSolveWarp) {
+            mf_bwd_pair_warp_kernel<<<dim3((D.nSolveWarp + kSolveWarpsPerCta - 1) / kSolveWarpsPerCta, n), kSolveWarpsPerCta * 32, 0, st>>>(
+                tb, sa, sb, P.pairWarpList[d], D.nSolveWarp, P.nPairWarpBoth[d]);
+            ++nl;
+        }
+        if (D.nSolveCta) {
+            mf_bwd_pair_kernel<<<dim3(D.nSolveCta, n), D.solveCtaThreads, pairSmem, st>>>(tb, sa, sb, P.pairCtaList[d], P.nPairCtaBoth[d]);
             ++nl;
         }
     }

@@ -68,6 +68,9 @@ struct DepthSchedule {
     int solveCtaThreads = 256;               // threads per CTA of the CTA-per-front solve kernels at this depth
 };
 
+struct Tables;
+struct SolveArgs;
+
 class Solver {
   public:
     // S is consumed.  nsys systems are factorised together; up to maxRhs right-hand sides per system in one solve call;
@@ -84,15 +87,26 @@ class Solver {
     // numeric factorisation from vals(); status: device array [nsys] (set to -10 on a singular pivot block)
     int factor(cudaStream_t st, int* dStatus, int64_t* nLaunches = nullptr, int sys0 = 0, int n = -1);
     // nrhs right-hand sides per system: vector (sys, r) at B + (sys*nrhs + r)*ldb, original numbering; X may alias B
-    // (B and X are the bases of the whole batch; the range is applied inside)
+    // (B and X are the bases of the whole batch; the range is applied inside).  Uses the workspace slots 0 .. nrhs-1.
     // pattern: 0 = dense right-hand sides, > 0 = an id returned by add_rhs_pattern (the rows outside it MUST be zero)
     int solve(cudaStream_t st, int nrhs, const cplx* B, int64_t ldb, cplx* X, int64_t ldx, int64_t* nLaunches = nullptr, int sys0 = 0,
               int n = -1, int pattern = 0);
+    // The two phases of solve() for one vector per system in workspace slot `slot` (< maxRhs), so that two solves with the same
+    // factors can be interleaved (B, X: vector sys at B + sys*ldb; sys0 / n / pattern as in solve()):
+    //   forward_slot   : forward elimination (leaves the other slots alone);
+    //   backward_slot  : backward substitution of the fronts of pattern's active set only — the fronts whose subtree holds a
+    //                    row of the pattern: the unknowns of those rows and all their ancestors — writing X on their unknowns;
+    //   backward_pair  : backward substitution of slot 0 into Xa and slot 1 into Xb in one pass over the factor, complete except
+    //                    that on the fronts of `done`'s active set only slot 1 is solved: backward_slot(0, done) has already
+    //                    overwritten their slot-0 pivot parts with the solution, which the sweep reads as its ancestors' values.
+    int forward_slot(cudaStream_t st, int slot, const cplx* B, int64_t ldb, int64_t* nLaunches, int sys0, int n, int pattern);
+    int backward_slot(cudaStream_t st, int slot, cplx* X, int64_t ldx, int64_t* nLaunches, int sys0, int n, int pattern);
+    int backward_pair(cudaStream_t st, cplx* Xa, cplx* Xb, int64_t ldx, int64_t* nLaunches, int sys0, int n, int done);
     // Right-hand sides with a known sparsity pattern (nz[i] != 0: row i, original numbering, may be non-zero).  The forward
     // elimination then visits only the fronts whose subtree holds such a row — every other front would hand a zero update
     // vector to its parent — which prunes most of the tree when the sources sit on a few grid lines (MT right-hand sides:
-    // the nodes next to the Dirichlet boundary, the two receiver rows of the adjoint sources).  The backward substitution is
-    // always complete.  Returns the pattern id (> 0), or a negative error code.
+    // the nodes next to the Dirichlet boundary, the two receiver rows of the adjoint sources).  The backward substitution of
+    // solve() is always complete.  Returns the pattern id (> 0), or a negative error code.
     int add_rhs_pattern(const std::vector<unsigned char>& nz);
     // fronts visited by the forward elimination of a pattern (0: all), for diagnostics
     int fwd_fronts(int pattern) const;
@@ -106,19 +120,27 @@ class Solver {
     template <typename Tp>
     int upload(const std::vector<Tp>& h, Tp** d);
     int upload_solve_descs(const std::vector<int>& fronts, const SolveDesc** d);
+    Tables tables(int sys0) const;
+    SolveArgs solve_args(const cplx* B, int64_t ldb, cplx* X, int64_t ldx, int sys0, int nrhs, int slot) const;
+    int set_solve_attributes();
+    int clear_ws(cudaStream_t st, const SolveArgs& sa, int nvec);
+    int fwd_sweep(cudaStream_t st, const Tables& tb, const SolveArgs& sa, int nvec, int pattern, int64_t& nl);
     Symbolic S;
     int nsys = 0, maxRhs = 1;
     int64_t valCount = 0;
     size_t bytes = 0;
     std::vector<void*> owned;
     std::vector<DepthSchedule> sched;
-    struct FwdLists {                            // forward-elimination launch lists of one right-hand-side pattern, per depth
-        std::vector<const SolveDesc*> warpList;
+    struct PatternLists {                        // launch lists of one right-hand-side pattern, per depth
+        std::vector<const SolveDesc*> warpList;  // its active set: forward elimination, backward_slot
         std::vector<const int*> ctaList;
         std::vector<int> nWarp, nCta;
         int nFronts = 0;
+        std::vector<const SolveDesc*> pairWarpList;   // backward_pair(done = this pattern): every front of the depth, those
+        std::vector<const int*> pairCtaList;          // outside the active set first (both slots), then the active set (slot 1)
+        std::vector<int> nPairWarpBoth, nPairCtaBoth;
     };
-    std::vector<FwdLists> patterns;
+    std::vector<PatternLists> patterns;
     // device tables
     Front* d_fronts = nullptr;
     int *d_rows = nullptr, *d_rel = nullptr, *d_children = nullptr, *d_pos2orig = nullptr;
@@ -129,6 +151,7 @@ class Solver {
     cplx *d_vals = nullptr, *d_v = nullptr, *d_upd = nullptr;
     int* d_invMaps = nullptr;                  // inverse row maps (front row -> child row) of the large fronts
     size_t solveSmem = 0;
+    size_t pairSmem = 0;                       // mf_bwd_pair_kernel: two vectors of the largest front and their chunk stages
     unsigned long long* d_prof = nullptr;      // HMCMT_MF_PROF=1: phase cycle counters of mf_small_kernel
 };
 

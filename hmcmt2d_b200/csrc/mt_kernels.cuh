@@ -249,12 +249,13 @@ __global__ void k_rhs(MeshDev M, SysMap sm, const double* __restrict__ sigma, co
     rhs[(size_t)sys * M.N + q] = r;
 }
 
-// full node-ordered field from the interior solution + boundary values (mt2DTE.jl:57-62).
-// grid: (ceil(nNode/256), nSys).  If bc == nullptr the boundary is zero (adjoint field).
+// full node-ordered field from the interior solution + boundary values (mt2DTE.jl:57-62), nodes [n0, n1) of it.
+// grid: (ceil((n1 - n0)/256), nSys).  If bc == nullptr the boundary is zero (adjoint field).
 // (sys0: first system of the group this launch covers; the groups of a step run on different streams, hmcmt_b200.cu)
-__global__ void k_node_field(MeshDev M, const cplx* __restrict__ x, const cplx* __restrict__ bc, cplx* __restrict__ F, int sys0) {
-    int n = blockIdx.x * blockDim.x + threadIdx.x;
-    if (n >= M.nNode) return;
+__global__ void k_node_field(MeshDev M, const cplx* __restrict__ x, const cplx* __restrict__ bc, cplx* __restrict__ F, int sys0, int n0,
+                             int n1) {
+    int n = n0 + blockIdx.x * blockDim.x + threadIdx.x;
+    if (n >= n1) return;
     const int sys = blockIdx.y + sys0, ny = M.ny, nz = M.nz;
     int kn = n / (ny + 1), jn = n - kn * (ny + 1);
     cplx v = mk(0.0, 0.0);

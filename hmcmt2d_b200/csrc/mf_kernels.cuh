@@ -60,6 +60,13 @@ struct Tables {
 // full symmetric ones.
 __device__ __forceinline__ int tl_off(int r, int c) { return ((c >> 2) << 5) | (r << 2) | (c & 3); }
 __device__ __forceinline__ double* mf_tile(double* tiles, int I, int J) { return tiles + (size_t)(I * (I + 1) / 2 + J) * 128; }
+// Mid-size fronts (the 8- and 16-warp instantiations) keep the pivot columns only, tiles (I, J) with J < npb: the pivot triangle
+// as above, then the nub x npb block of F21 row by row.  The update block F22 never enters shared memory (see mf_small_kernel).
+__device__ __forceinline__ int mf_pc_row(int I, int npb) { return I < npb ? I * (I + 1) / 2 : npb * (npb + 1) / 2 + (I - npb) * npb; }
+template <bool PC>
+__device__ __forceinline__ double* mf_tile(double* tiles, int npb, int I, int J) {
+    return PC ? tiles + (size_t)(mf_pc_row(I, npb) + J) * 128 : mf_tile(tiles, I, J);
+}
 
 struct TileFrag {      // A or B operand of one 8x8 complex tile (both k-halves), or its C fragment
     double re[2], im[2];
@@ -107,8 +114,9 @@ __device__ __forceinline__ void frag_add(TileFrag& c, const TileFrag& x) {
 //   C  M' = F21 (-G)      into mbuf (tile (I - npb, kb) at mbuf + ((I - npb) npb + kb) 128)          -> mbuf = -M
 //   D  U  = F22 + M' F21^T  accumulated over all pivots in registers                                  -> update tiles = U
 // The update rows never enter the latency-bound sweep: they see two perfectly parallel products with K = all pivots.
+// PC: the tiles hold the pivot columns only (mf_tile<true>); phase D is then the caller's (it gathers F22 from the children).
 // scratch: 2 npb tiles (column operands of the sweep; may alias mbuf).  All NW warps call; ends with a CTA barrier.
-template <int NW>
+template <int NW, bool PC = false>
 __device__ __forceinline__ void mf_front_factor(double* __restrict__ tiles, double* __restrict__ scratch, double* __restrict__ mbuf,
                                                 double* __restrict__ nainv, int* __restrict__ fail, const int nb, const int npb,
                                                 const int sReal, unsigned long long* __restrict__ prof = nullptr) {
@@ -202,7 +210,7 @@ __device__ __forceinline__ void mf_front_factor(double* __restrict__ tiles, doub
             frag_zero(c); frag_zero(x);
             for (int j = 0; j < npb; ++j) {
                 TileFrag a, b;
-                frag_load(a, mf_tile(tiles, I, j), lane);
+                frag_load(a, mf_tile<PC>(tiles, npb, I, j), lane);
                 if (kb >= j) frag_load(b, mf_tile(tiles, kb, j), lane);       // B[n][k] = (-G)(kb n, j k)
                 else frag_load_t(b, mf_tile(tiles, j, kb), g, t);
                 frag_mma(c, x, a, b);
@@ -213,6 +221,7 @@ __device__ __forceinline__ void mf_front_factor(double* __restrict__ tiles, doub
     }
     __syncthreads();
     MF_SWEEP_MARK(2);      // slot 2: M' = F21 (-G)
+    if (PC) return;
     // ---- D: U(I, J) += sum_kb M'(I, kb) F21(J, kb)^T, lower tiles, two tiles per trip (independent DMMA chains) ----
     {
         const int nU = nub * (nub + 1) / 2;
@@ -276,11 +285,14 @@ __device__ __forceinline__ void mf_store_tile(const double* __restrict__ T, doub
 // ------------------------------------------------------------------------------------------------------------------------
 // small fronts: one CTA per (front, system).  list[blockIdx.x] = front id.
 // (register budget: the two- and four-warp instantiations serve the thousands of tiny fronts at the bottom of the tree, where the
-// number of fronts resident per SM hides the latency of the 8x8 inversions: 64 registers per thread -> 16 / 8 CTAs per SM)
+// number of fronts resident per SM hides the latency of the 8x8 inversions: 64 registers per thread -> 16 / 8 CTAs per SM.
+// The 8- and 16-warp instantiations (kMid) keep only the pivot columns in shared memory, so that 4 / 2 of them fit on an SM
+// beside each other: 64 registers per thread as well.)
 template <int NW>
-__global__ void __launch_bounds__(NW * 32, NW <= 4 ? (NW == 1 ? 16 : 32 / NW) : (NW == 8 ? 2 : 1))
+__global__ void __launch_bounds__(NW * 32, NW <= 4 ? (NW == 1 ? 16 : 32 / NW) : (NW == 8 ? 4 : 2))
 mf_small_kernel(Tables tb, const SmallDesc* __restrict__ descs) {
     constexpr int NT = NW * 32;
+    constexpr bool kMid = NW >= 8;
     extern __shared__ __align__(16) unsigned char mf_smem[];
     SmallDesc& F = *reinterpret_cast<SmallDesc*>(mf_smem);      // the first kFrontDescBytes of the dynamic block
     const int sys = blockIdx.y, tid = threadIdx.x, lane = tid & 31;
@@ -293,7 +305,7 @@ mf_small_kernel(Tables tb, const SmallDesc* __restrict__ descs) {
         reinterpret_cast<int*>(&F)[i] = reinterpret_cast<const int*>(descs + blockIdx.x)[i];
     __syncthreads();
     const int fp = F.sp + F.up, nb = fp >> 3, npb = F.sp >> 3, nub = nb - npb;
-    const int nT = nb * (nb + 1) / 2;
+    const int nT = kMid ? mf_pc_row(nb, npb) : nb * (nb + 1) / 2;      // tiles kept in shared memory
     double* tiles = reinterpret_cast<double*>(mf_smem + kFrontDescBytes);
     double* mbuf = tiles + (size_t)nT * 128;                                   // sweep scratch, then M'
     double* nainv = mbuf + (size_t)(2 * npb > nub * npb ? 2 * npb : nub * npb) * 128;
@@ -301,7 +313,9 @@ mf_small_kernel(Tables tb, const SmallDesc* __restrict__ descs) {
     // row maps of all children, back to back, already split into the two address parts of the tile layout: an entry (a, b),
     // a >= b, of the front sits at tiles + rowPart(a) + colPart(b)
     int2* relS = reinterpret_cast<int2*>(fail + 4);
-    auto rel_parts = [](int r) { return make_int2(((r >> 3) * ((r >> 3) + 1) / 2) * 128 + (r & 7) * 4, (r >> 3) * 128 + ((r & 4) << 3) + (r & 3)); };
+    auto rel_parts = [npb](int r) {
+        return make_int2((kMid ? mf_pc_row(r >> 3, npb) : (r >> 3) * ((r >> 3) + 1) / 2) * 128 + (r & 7) * 4, (r >> 3) * 128 + ((r & 4) << 3) + (r & 3));
+    };
     // everything that depends on the record alone is requested now: the children's row maps, the first batches of the children's
     // update matrices, the first original entry of every thread (and its value); the latency hides behind the zeroing
     const int nChild = F.nChild;
@@ -314,6 +328,8 @@ mf_small_kernel(Tables tb, const SmallDesc* __restrict__ descs) {
             base += cu;
         }
     }
+    // kMid: inverse row maps of the update rows, child c at invS + c * up: update row a of the front -> row of child c (-1: none)
+    int* invS = reinterpret_cast<int*>(relS + ((F.cU[0] + F.cU[1] + F.cU[2] + F.cU[3] + 1) & ~1));
     // Extend-add of the children's update matrices.  Work items = (column group of four, block of 32 rows) of a child's lower
     // triangle (16-byte loads, 64 bytes per lane and item), dealt round-robin to the warps in batches of kBatch.  Every warp
     // walks ITS batches of all children in order with two batches in flight: the loads of batch k+2 are issued before batch k
@@ -321,7 +337,7 @@ mf_small_kernel(Tables tb, const SmallDesc* __restrict__ descs) {
     // or two per child.  Children are scattered one after the other (a CTA barrier per child boundary: entries of one child
     // never collide, plain adds, fixed order -> deterministic).
     const double* carena = tb.arena[F.par ^ 1] + (size_t)sys * tb.arenaStride[F.par ^ 1];
-    constexpr int kBatch = NW <= 4 ? 1 : 2;      // (the small instantiations live on 64 registers)
+    constexpr int kBatch = 1;      // (every instantiation lives on 64 registers)
     struct Batch {
         double2 r01[kBatch], r23[kBatch], i01[kBatch], i23[kBatch];
         int ii[kBatch], jg[kBatch];
@@ -331,7 +347,7 @@ mf_small_kernel(Tables tb, const SmallDesc* __restrict__ descs) {
     auto load_batch = [&](Batch& bt) {
         while (curC < nChild) {
             const int cu = F.cU[curC];
-            if (curQ < ((cu + 3) >> 2) * ((cu + 31) >> 5)) break;
+            if (curQ < (((kMid ? F.cPiv[curC] : cu) + 3) >> 2) * ((cu + 31) >> 5)) break;
             ++curC;
             curQ = warp * kBatch;
         }
@@ -339,7 +355,7 @@ mf_small_kernel(Tables tb, const SmallDesc* __restrict__ descs) {
         if (bt.c < 0) return;
         const int cu = F.cU[curC], ld = F.cLd[curC], off = F.cFirst[curC];
         const double* U = carena + F.cOff[curC];
-        const int ng = (cu + 3) >> 2, nrb = (cu + 31) >> 5;
+        const int ng = ((kMid ? F.cPiv[curC] : cu) + 3) >> 2, nrb = (cu + 31) >> 5;
 #pragma unroll
         for (int bq = 0; bq < kBatch; ++bq) {
             const int q = curQ + bq;
@@ -366,15 +382,27 @@ mf_small_kernel(Tables tb, const SmallDesc* __restrict__ descs) {
         ov0 = oe0.src < 0 ? mk(1.0, 0.0) : vals[oe0.src];
     }
     for (int i = tid; i < nT * 64; i += NT) reinterpret_cast<double2*>(tiles)[i] = make_double2(0.0, 0.0);
+    if (kMid)
+        for (int i = tid; i < nChild * F.up; i += NT) invS[i] = -1;
     if (tid == 0) *fail = 0;
     __syncthreads();
     MF_PROF_MARK(0);
+    if (kMid) {      // (read by phase D only: many barriers away)
+        int base = 0;
+        for (int c = 0; c < nChild; ++c) {
+            const int cu = F.cU[c];
+            const int* rel = tb.rel + F.cRel[c];
+            for (int i = F.cPiv[c] + tid; i < cu; i += NT) invS[base + rel[i] - F.sp] = i;
+            base += F.up;
+        }
+    }
     auto addr = [&](int a, int b) {       // a >= b
-        return tiles + (size_t)((a >> 3) * ((a >> 3) + 1) / 2 + (b >> 3)) * 128 + tl_off(a & 7, b & 7);
+        return tiles + (size_t)((kMid ? mf_pc_row(a >> 3, npb) : (a >> 3) * ((a >> 3) + 1) / 2) + (b >> 3)) * 128 + tl_off(a & 7, b & 7);
     };
     {
         auto scatter = [&](const Batch& bt) {
             const int2* relC = relS + ((bt.c > 0 ? F.cU[0] : 0) + (bt.c > 1 ? F.cU[1] : 0) + (bt.c > 2 ? F.cU[2] : 0));
+            const int jEnd = kMid ? F.cPiv[bt.c] : 0;      // kMid: the columns that land in the pivot columns only
 #pragma unroll
             for (int bq = 0; bq < kBatch; ++bq) {
                 const int i = bt.ii[bq];
@@ -385,7 +413,7 @@ mf_small_kernel(Tables tb, const SmallDesc* __restrict__ descs) {
                 double* rowp = tiles + relC[i].x;
 #pragma unroll
                 for (int jj = 0; jj < 4; ++jj) {
-                    if (4 * jg + jj > i) break;
+                    if (4 * jg + jj > i || (kMid && 4 * jg + jj >= jEnd)) break;
                     double* d = rowp + relC[4 * jg + jj].y;
                     d[0] += re[jj];
                     d[64] += im[jj];
@@ -421,7 +449,66 @@ mf_small_kernel(Tables tb, const SmallDesc* __restrict__ descs) {
     }
     __syncthreads();
     MF_PROF_MARK(1);
-    mf_front_factor<NW>(tiles, mbuf, mbuf, nainv, fail, nb, npb, F.s, tb.prof ? tb.prof + 32 + _pc * 4 : nullptr);
+    mf_front_factor<NW, kMid>(tiles, mbuf, mbuf, nainv, fail, nb, npb, F.s, tb.prof ? tb.prof + 32 + _pc * 4 : nullptr);
+    if (kMid && nub > 0) {
+        // ---- D: U = F22 + M' F21^T, lower tiles, two per trip, written from the registers to the update arena.  F22 is gathered
+        // from the children's update matrices through the inverse row maps straight into the accumulators: every element starts
+        // at +0.0 and takes the children's entries in child order, the very sums the extend-add into a zeroed F22 formed.
+        const long long tD = tb.prof ? clock64() : 0;
+        const int g = lane >> 2, t = lane & 3, up = F.up;
+        double* U = tb.arena[F.par] + (size_t)sys * tb.arenaStride[F.par] + F.uOff;
+        auto gather = [&](TileFrag& c, int I, int J) {      // elements (a, b), (a, b + 1) of the update block
+            const int a = 8 * I + g, b = 8 * J + 2 * t;
+            frag_zero(c);
+#pragma unroll
+            for (int ch = 0; ch < kSmallChildren; ++ch) {
+                const int* inv = invS + ch * up;
+                const int ia = ch < nChild ? inv[a] : -1;
+                if (ia < 0) continue;
+                const int ib0 = inv[b], ib1 = inv[b + 1];
+                const double* Uc = carena + F.cOff[ch];
+                const int ld = F.cLd[ch], off = F.cFirst[ch];
+                if (ib0 >= 0 && ib0 <= ia) { c.re[0] += Uc[kg_off(ld, off + ia, off + ib0, 0)]; c.im[0] += Uc[kg_off(ld, off + ia, off + ib0, 1)]; }
+                if (ib1 >= 0 && ib1 <= ia) { c.re[1] += Uc[kg_off(ld, off + ia, off + ib1, 0)]; c.im[1] += Uc[kg_off(ld, off + ia, off + ib1, 1)]; }
+            }
+        };
+        auto store = [&](const TileFrag& c, int I, int J) {
+            double* o = U + kg_off(up, 8 * I + g, 8 * J + 2 * t, 0);
+            *reinterpret_cast<double2*>(o) = make_double2(c.re[0], c.re[1]);
+            *reinterpret_cast<double2*>(o + 4 * up) = make_double2(c.im[0], c.im[1]);
+        };
+        const int nU = nub * (nub + 1) / 2;
+        int I = 0, J = warp;
+        while (J > I) { J -= I + 1; ++I; }
+        for (int L = warp; L < nU; L += 2 * NW) {
+            const int I0 = I, J0 = J;
+            J += NW;
+            while (J > I) { J -= I + 1; ++I; }
+            const bool two = L + NW < nU;
+            const int I1 = I, J1 = J;
+            J += NW;
+            while (J > I) { J -= I + 1; ++I; }
+            TileFrag c0, x0, c1, x1;
+            gather(c0, I0, J0);
+            frag_zero(x0);
+            if (two) { gather(c1, I1, J1); frag_zero(x1); }
+            for (int kb = 0; kb < npb; ++kb) {
+                TileFrag a, b;
+                frag_load(a, mbuf + (size_t)(I0 * npb + kb) * 128, lane);
+                frag_load(b, mf_tile<true>(tiles, npb, npb + J0, kb), lane);
+                frag_mma(c0, x0, a, b);
+                if (two) {
+                    frag_load(a, mbuf + (size_t)(I1 * npb + kb) * 128, lane);
+                    frag_load(b, mf_tile<true>(tiles, npb, npb + J1, kb), lane);
+                    frag_mma(c1, x1, a, b);
+                }
+            }
+            frag_add(c0, x0);
+            store(c0, I0, J0);
+            if (two) { frag_add(c1, x1); store(c1, I1, J1); }
+        }
+        if (tb.prof && tid == 0) atomicAdd(tb.prof + 32 + _pc * 4 + 3, (unsigned long long)(clock64() - tD));
+    }
     MF_PROF_MARK(4);
     if (tid == 0 && *fail) tb.status[sys] = kErrSingular;
     // outputs, tile by tile: G = -(pivot x pivot), M = -M' (factor arena), U = update x update (update arena, lower tiles)
@@ -439,6 +526,8 @@ mf_small_kernel(Tables tb, const SmallDesc* __restrict__ descs) {
         double* M = fac + F.mOff;
         for (int I = warp; I < nub; I += NW)
             for (int J = 0; J < npb; ++J) mf_store_tile<false>(mbuf + (size_t)(I * npb + J) * 128, M, up, I * 8, J * 8, -1.0, lane);
+    }
+    if (!kMid && up > 0) {
         double* U = tb.arena[F.par] + (size_t)sys * tb.arenaStride[F.par] + F.uOff;
         int I = 0, J = warp;
         while (J > I) { J -= I + 1; ++I; }

@@ -137,12 +137,17 @@ int Solver::build(int nsys_, int maxRhs_, int64_t valCount_) {
         D.nSmall = (int)sm.size();
         if (D.nSmall) {
             int mx = 0;
+            for (int k : sm) mx = std::max(mx, S.fronts[k].fp());
+            auto knob = [](const char* name, int dflt) { const char* e = std::getenv(name); return e ? std::atoi(e) : dflt; };
+            // warps per front by the largest front of the launch (measured optimum at cfg2; one warp per front needs no CTA barrier)
+            const int f1 = knob("HMCMT_MF_FP1", 40), f2 = knob("HMCMT_MF_FP2", 40), f4 = knob("HMCMT_MF_FP4", 64), f8 = knob("HMCMT_MF_FP8", 96);
+            D.smallWarps = mx <= f1 ? 1 : (mx <= f2 ? 2 : (mx <= f4 ? 4 : (mx <= f8 ? 8 : 16)));
             D.smallSmem = 0;
             std::vector<SmallDesc> descs;
             for (int k : sm) {
                 const Front& F = S.fronts[k];
-                mx = std::max(mx, F.fp());
-                D.smallSmem = std::max(D.smallSmem, mf_front_smem_bytes(F.fp() / 8, F.sp / 8, mf_rel_total(S, k)));
+                D.smallSmem = std::max(D.smallSmem, D.smallWarps >= 8 ? mf_mid_front_smem_bytes(F.fp() / 8, F.sp / 8, mf_rel_total(S, k), F.nChild)
+                                                                      : mf_front_smem_bytes(F.fp() / 8, F.sp / 8, mf_rel_total(S, k)));
                 SmallDesc sd{};
                 sd.sp = F.sp; sd.up = F.up; sd.s = F.s; sd.nChild = F.nChild; sd.nOrig = F.nOrig; sd.origPtr = F.origPtr;
                 sd.par = F.depth & 1; sd.front = k;
@@ -150,16 +155,16 @@ int Solver::build(int nsys_, int maxRhs_, int64_t valCount_) {
                 for (int c = 0; c < std::min(F.nChild, kDescChildren); ++c) {
                     const Front& C = S.fronts[S.children[F.childPtr + c]];
                     sd.cOff[c] = C.frontOff; sd.cLd[c] = C.ldU(); sd.cFirst[c] = C.offU(); sd.cU[c] = C.u; sd.cRel[c] = C.rowPtr;
+                    int piv = 0;
+                    while (piv < C.u && S.rel[C.rowPtr + piv] < F.sp) ++piv;
+                    if (piv > 255) return kErrArg;
+                    sd.cPiv[c] = (unsigned char)piv;
                 }
                 descs.push_back(sd);
             }
             SmallDesc* pd = nullptr;
             MF_TRY(upload(descs, &pd));
             D.smallDescs = pd;
-            auto knob = [](const char* name, int dflt) { const char* e = std::getenv(name); return e ? std::atoi(e) : dflt; };
-            // warps per front by the largest front of the launch (measured optimum at cfg2; one warp per front needs no CTA barrier)
-            const int f1 = knob("HMCMT_MF_FP1", 40), f2 = knob("HMCMT_MF_FP2", 40), f4 = knob("HMCMT_MF_FP4", 64), f8 = knob("HMCMT_MF_FP8", 96);
-            D.smallWarps = mx <= f1 ? 1 : (mx <= f2 ? 2 : (mx <= f4 ? 4 : (mx <= f8 ? 8 : 16)));
         }
         D.nBig = (int)bg.size();
         D.bigBytes = (size_t)S.bigDoublesAtDepth[d] * sizeof(double);

@@ -27,6 +27,7 @@ struct SmallDesc {
     int64_t gOff, mOff, uOff;
     int64_t cOff[kDescChildren];          // child update matrices (arena of the other parity)
     int cLd[kDescChildren], cFirst[kDescChildren], cU[kDescChildren], cRel[kDescChildren];   // ld, first row / column, real rows, rel offset
+    unsigned char cPiv[kDescChildren];    // the child's rows that land in the pivot columns (a prefix: the rows are sorted)
 };
 
 // The same for the warp-per-front solve kernels (fronts of at most 64 rows, a single pivot chunk): offsets / counts of the front

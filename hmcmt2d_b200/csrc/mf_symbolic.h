@@ -37,6 +37,15 @@ inline size_t mf_front_smem_bytes(int nb, int npb, int relTotal = 0) {
     const size_t nT = (size_t)nb * (nb + 1) / 2, nS = 2 * (size_t)npb, nM = (size_t)(nb - npb) * npb;
     return kFrontDescBytes + (nT + (nS > nM ? nS : nM) + 1) * 128 * sizeof(double) + 16 + (((size_t)relTotal + 1) & ~(size_t)1) * 2 * sizeof(int);
 }
+// The 8- and 16-warp instantiations (launches whose largest front has more than 64 rows) keep only the pivot columns: the
+// pivot triangle and the F21 block, no F22 (gathered from the children straight into the registers of the Schur product),
+// plus one inverse row map of the update rows per child (nChild x (nb - npb) * 8 ints).  The small / global-memory
+// classification (Symbolic::fronts[].isBig) stays on mf_front_smem_bytes, so this layout moves no front between the paths.
+inline size_t mf_mid_front_smem_bytes(int nb, int npb, int relTotal, int nChild) {
+    const size_t nub = (size_t)(nb - npb), nT = (size_t)npb * (npb + 1) / 2 + nub * npb, nS = 2 * (size_t)npb, nM = nub * npb;
+    return kFrontDescBytes + (nT + (nS > nM ? nS : nM) + 1) * 128 * sizeof(double) + 16 + (((size_t)relTotal + 1) & ~(size_t)1) * 2 * sizeof(int) +
+           (size_t)nChild * nub * 8 * sizeof(int);
+}
 constexpr size_t kFrontSmemMax = 227 * 1024;
 
 // lower-triangular entry of the original matrix (row >= col, original numbering) and where its value comes from

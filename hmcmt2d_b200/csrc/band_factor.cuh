@@ -262,10 +262,16 @@ __device__ __forceinline__ void gj_invert8(cplx& a0, cplx& a1, bool& bad, const 
 #pragma unroll 1
         for (int k = 0; k < nsteps; ++k) pivot_step(k);
     }
-    const double den = fma(q.x, q.x, q.y * q.y);
-    if (!(den > 0.0) || isinf(den)) bad = true;
-    const double iden = __drcp_rn(den);
-    const cplx qi = mk(q.x * iden, -q.y * iden);
+    // 1/q = s conj(qs) / |qs|^2 with qs = s q, s = 2^-(exponent of q) exact: |qs|^2 lies in [1, 8) whatever the scale of the
+    // matrix, so neither overflows nor turns subnormal where |q|^2 would (|q| beyond ~2^511 or below ~2^-511); for every other q
+    // the result is bit-identical to conj(q) / |q|^2
+    const int eq = (__double2hiint(fmax(fabs(q.x), fabs(q.y))) >> 20) & 0x7ff;
+    const double sq = __hiloint2double((2046 - eq) << 20, 0);
+    const cplx qs = mk(q.x * sq, q.y * sq);
+    const double den = fma(qs.x, qs.x, qs.y * qs.y);
+    const double iden = __drcp_rn(den) * sq;
+    if (!(den > 0.0) || isinf(den) || isinf(iden)) bad = true;
+    const cplx qi = mk(qs.x * iden, -qs.y * iden);
     a0 = a0 * qi;
     a1 = a1 * qi;
 }

@@ -807,7 +807,7 @@ struct SolveArgs {
     int64_t vStride, uStride;
     int nrhs;
 };
-constexpr int kSolveMfThreads = 256;      // upper bound; launched with 128 threads where no front of the depth exceeds 144 rows
+// block size: kSolveMfThreads (mf_symbolic.h) at most; launched with 128 threads where no front of the depth exceeds 144 rows
 
 __global__ void __launch_bounds__(kSolveMfThreads)
 mf_fwd_kernel(Tables tb, SolveArgs sa, const int* __restrict__ list) {

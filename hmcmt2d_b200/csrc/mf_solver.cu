@@ -22,9 +22,6 @@ struct PerDeviceOnceMf {
     }
 };
 constexpr size_t kMaxSmem = 227 * 1024;
-constexpr int kSolveWarpMaxFp = 64;  // solves: warp-per-front kernels up to this front size
-// solves: one warp per front (record-driven kernels) for small fronts with few children, one CTA per front otherwise
-inline bool solve_by_warp(const Front& F) { return !F.isBig && F.fp() <= kSolveWarpMaxFp && F.nChild <= kDescChildren; }
 
 template <int NW>
 int launch_small(cudaStream_t st, const Tables& tb, const SmallDesc* list, int n, int nsys, size_t smem) {
@@ -128,6 +125,7 @@ int Solver::build(int nsys_, int maxRhs_, int64_t valCount_) {
 
     // launch schedule
     std::vector<int> invMapsHost;
+    const SchedKnobs knobs = SchedKnobs::from_env();
     sched.assign(S.maxDepth + 1, DepthSchedule());
     for (int d = 0; d <= S.maxDepth; ++d) {
         DepthSchedule& D = sched[d];
@@ -138,10 +136,7 @@ int Solver::build(int nsys_, int maxRhs_, int64_t valCount_) {
         if (D.nSmall) {
             int mx = 0;
             for (int k : sm) mx = std::max(mx, S.fronts[k].fp());
-            auto knob = [](const char* name, int dflt) { const char* e = std::getenv(name); return e ? std::atoi(e) : dflt; };
-            // warps per front by the largest front of the launch (measured optimum at cfg2; one warp per front needs no CTA barrier)
-            const int f1 = knob("HMCMT_MF_FP1", 40), f2 = knob("HMCMT_MF_FP2", 40), f4 = knob("HMCMT_MF_FP4", 64), f8 = knob("HMCMT_MF_FP8", 96);
-            D.smallWarps = mx <= f1 ? 1 : (mx <= f2 ? 2 : (mx <= f4 ? 4 : (mx <= f8 ? 8 : 16)));
+            D.smallWarps = mf_small_warps(mx, knobs);
             D.smallSmem = 0;
             std::vector<SmallDesc> descs;
             for (int k : sm) {
@@ -170,7 +165,7 @@ int Solver::build(int nsys_, int maxRhs_, int64_t valCount_) {
         D.bigBytes = (size_t)S.bigDoublesAtDepth[d] * sizeof(double);
         // solves: one warp per front up to kSolveWarpMaxFp rows, one CTA per front above
         std::vector<int> sw, sc(bg);
-        for (int k : sm) (solve_by_warp(S.fronts[k]) ? sw : sc).push_back(k);
+        for (int k : sm) (mf_solve_by_warp(S.fronts[k]) ? sw : sc).push_back(k);
         D.nSolveWarp = (int)sw.size();
         D.nSolveCta = (int)sc.size();
         if (D.nSolveWarp) MF_TRY(upload_solve_descs(sw, &D.solveWarpList));
@@ -178,9 +173,7 @@ int Solver::build(int nsys_, int maxRhs_, int64_t valCount_) {
         {
             int mxc = 0;
             for (int k : sc) mxc = std::max(mxc, S.fronts[k].fp());
-            const char* e = std::getenv("HMCMT_MF_SOLVE_THREADS");      // 0: by front size
-            const int forced = e ? std::atoi(e) : 0;
-            D.solveCtaThreads = forced ? forced : (mxc <= 144 ? 128 : kSolveMfThreads);
+            D.solveCtaThreads = mf_solve_cta_threads(mxc, knobs);
         }
         if (!D.nBig) continue;
         MF_TRY(upload(bg, &p));
@@ -267,7 +260,7 @@ int Solver::build(int nsys_, int maxRhs_, int64_t valCount_) {
     if (solveSmem > kMaxSmem) return kErrArg;
     {
         int mx = 0;
-        for (const Front& F : S.fronts) if (!solve_by_warp(F)) mx = std::max(mx, F.fp() + F.sp);
+        for (const Front& F : S.fronts) if (!mf_solve_by_warp(F)) mx = std::max(mx, F.fp() + F.sp);
         pairSmem = (size_t)2 * mx * sizeof(cplx);      // (checked by backward_pair, the only user)
     }
 #undef MF_TRY
@@ -359,9 +352,9 @@ int Solver::add_rhs_pattern(const std::vector<unsigned char>& nz) {
     for (int d = 0; d <= S.maxDepth; ++d) {
         std::vector<int> sw, sc, pw, pc;      // active set; all fronts, inactive first (backward_pair)
         for (int k : S.byDepthBig[d]) if (active[k]) sc.push_back(k);
-        for (int k : S.byDepthSmall[d]) if (active[k]) (solve_by_warp(S.fronts[k]) ? sw : sc).push_back(k);
+        for (int k : S.byDepthSmall[d]) if (active[k]) (mf_solve_by_warp(S.fronts[k]) ? sw : sc).push_back(k);
         for (int k : S.byDepthBig[d]) if (!active[k]) pc.push_back(k);
-        for (int k : S.byDepthSmall[d]) if (!active[k]) (solve_by_warp(S.fronts[k]) ? pw : pc).push_back(k);
+        for (int k : S.byDepthSmall[d]) if (!active[k]) (mf_solve_by_warp(S.fronts[k]) ? pw : pc).push_back(k);
         L.nPairWarpBoth.push_back((int)pw.size());
         L.nPairCtaBoth.push_back((int)pc.size());
         pw.insert(pw.end(), sw.begin(), sw.end());

@@ -15,6 +15,7 @@
 #pragma once
 #include <algorithm>
 #include <cstdint>
+#include <cstdlib>
 #include <functional>
 #include <numeric>
 #include <queue>
@@ -477,6 +478,60 @@ inline int mf_rel_total(const Symbolic& S, int k) {
     int n = 0;
     for (int c = 0; c < F.nChild; ++c) n += S.fronts[S.children[F.childPtr + c]].u;
     return n;
+}
+
+// ------------------------------------------------------------------------------------------------------------------------
+// launch-schedule rules of the numeric phase (mf_solver.cu), kept here so that host tools can classify fronts without CUDA
+constexpr int kSolveWarpMaxFp = 64;       // solves: warp-per-front kernels up to this front size
+constexpr int kSolveMfThreads = 256;      // CTA-per-front solve kernels: upper bound, 128 where no front of the depth exceeds 144 rows
+
+// tuning knobs read from the environment when a solver builds its schedule (and hashed into the Level-1 shim's cache key)
+struct SchedKnobs {
+    int fp1 = 40, fp2 = 40, fp4 = 64, fp8 = 96;      // HMCMT_MF_FP1/2/4/8: largest front of a launch per warp count
+    int solveThreads = 0;                            // HMCMT_MF_SOLVE_THREADS: CTA-solve threads, 0 = by front size
+    static SchedKnobs from_env() {
+        auto knob = [](const char* name, int dflt) { const char* e = std::getenv(name); return e ? std::atoi(e) : dflt; };
+        SchedKnobs k;
+        k.fp1 = knob("HMCMT_MF_FP1", k.fp1); k.fp2 = knob("HMCMT_MF_FP2", k.fp2);
+        k.fp4 = knob("HMCMT_MF_FP4", k.fp4); k.fp8 = knob("HMCMT_MF_FP8", k.fp8);
+        k.solveThreads = knob("HMCMT_MF_SOLVE_THREADS", 0);
+        return k;
+    }
+};
+
+// warps per front of a single-CTA launch, by the largest front of the launch (measured optimum at cfg2; one warp per front needs
+// no CTA barrier)
+inline int mf_small_warps(int maxFp, const SchedKnobs& k) {
+    return maxFp <= k.fp1 ? 1 : (maxFp <= k.fp2 ? 2 : (maxFp <= k.fp4 ? 4 : (maxFp <= k.fp8 ? 8 : 16)));
+}
+// solves: one warp per front (record-driven kernels) for small fronts with few children, one CTA per front otherwise
+inline bool mf_solve_by_warp(const Front& F) { return !F.isBig && F.fp() <= kSolveWarpMaxFp && F.nChild <= kSmallChildren; }
+// threads of the CTA-per-front solve kernels at a depth whose largest CTA-solved front has maxFp rows
+inline int mf_solve_cta_threads(int maxFp, const SchedKnobs& k) {
+    return k.solveThreads ? k.solveThreads : (maxFp <= 144 ? 128 : kSolveMfThreads);
+}
+
+// Level-1 analysis of a 1-based CSC pattern (n columns, colptr[n] - 1 entries, both triangles or one): the lower triangle
+// (row >= col) is what the factorisation reads, entry k takes its value from nzval[k]; ordered by level-set bisection.
+inline bool mf_analyse_csc(int64_t n, const int64_t* rowval, const int64_t* colptr, int leaf, int fSmall, Symbolic& S) {
+    std::vector<Entry> ent;
+    ent.reserve((size_t)(colptr[n] - 1) / 2 + n);
+    std::vector<int> ptr(n + 1, 0);
+    for (int64_t j = 0; j < n; ++j)
+        for (int64_t k = colptr[j] - 1; k < colptr[j + 1] - 1; ++k) {
+            const int64_t i = rowval[k] - 1;
+            if (i < 0 || i >= n) return false;
+            if (i < j) continue;
+            ent.push_back(Entry{(int)i, (int)j, (int)k});
+            if (i != j) { ++ptr[i + 1]; ++ptr[j + 1]; }
+        }
+    for (int64_t i = 0; i < n; ++i) ptr[i + 1] += ptr[i];
+    std::vector<int> adj(ptr[n]), at(ptr.begin(), ptr.end() - 1);
+    for (const Entry& e : ent)
+        if (e.row != e.col) { adj[at[e.row]++] = e.col; adj[at[e.col]++] = e.row; }
+    std::vector<std::vector<int>> sn;
+    mf_order_graph((int)n, ptr, adj, leaf, sn);
+    return mf_symbolic((int)n, sn, ent, fSmall, S);
 }
 
 // pattern of the MT stencil systems in the internal ordering (mt_kernels.cuh): value array = [diag N | e1 N | e2 N]

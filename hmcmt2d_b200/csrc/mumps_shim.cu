@@ -67,7 +67,8 @@ void free_factor(Factor* f) {
 }
 
 // ---- multifrontal path ----------------------------------------------------------------------------------------------
-// symbolic analysis cached per sparsity pattern (key: n, nnz and an FNV hash of colptr / rowval)
+// symbolic analysis cached per sparsity pattern (key: n, nnz and an FNV hash of colptr / rowval and of every knob the analysis or
+// the solver's launch schedule reads: a pooled solver of the same key is reused as it was built)
 struct PatternKey {
     int64_t n, nnz;
     uint64_t h;
@@ -85,32 +86,16 @@ uint64_t fnv(const int64_t* p, int64_t n, uint64_t h) {
 
 const mf::Symbolic* symbolic_for(int64_t n, const int64_t* rowval, const int64_t* colptr) {
     const int64_t nnz = colptr[n] - 1;
-    const int64_t knobs[2] = {mf_leaf_size(), mf_small_front()};
-    PatternKey key{n, nnz, fnv(knobs, 2, fnv(rowval, nnz, fnv(colptr, n + 1, 0xcbf29ce484222325ull)))};
+    const mf::SchedKnobs sk = mf::SchedKnobs::from_env();
+    const int64_t knobs[7] = {mf_leaf_size(), mf_small_front(), sk.fp1, sk.fp2, sk.fp4, sk.fp8, sk.solveThreads};
+    PatternKey key{n, nnz, fnv(knobs, 7, fnv(rowval, nnz, fnv(colptr, n + 1, 0xcbf29ce484222325ull)))};
     {
         std::lock_guard<std::mutex> lk(g_mu);
         auto it = g_symbolic.find(key);
         if (it != g_symbolic.end()) return it->second;
     }
-    std::vector<mf::Entry> ent;
-    ent.reserve((size_t)nnz / 2 + n);
-    std::vector<int> ptr(n + 1, 0);
-    for (int64_t j = 0; j < n; ++j)
-        for (int64_t k = colptr[j] - 1; k < colptr[j + 1] - 1; ++k) {
-            const int64_t i = rowval[k] - 1;
-            if (i < 0 || i >= n) return nullptr;
-            if (i < j) continue;                          // the lower triangle is what LDL^T reads
-            ent.push_back(mf::Entry{(int)i, (int)j, (int)k});
-            if (i != j) { ++ptr[i + 1]; ++ptr[j + 1]; }
-        }
-    for (int64_t i = 0; i < n; ++i) ptr[i + 1] += ptr[i];
-    std::vector<int> adj(ptr[n]), at(ptr.begin(), ptr.end() - 1);
-    for (const mf::Entry& e : ent)
-        if (e.row != e.col) { adj[at[e.row]++] = e.col; adj[at[e.col]++] = e.row; }
-    std::vector<std::vector<int>> sn;
-    mf::mf_order_graph((int)n, ptr, adj, mf_leaf_size(), sn);
     mf::Symbolic* S = new mf::Symbolic();
-    if (!mf::mf_symbolic((int)n, sn, ent, mf_small_front(), *S)) { delete S; return nullptr; }
+    if (!mf::mf_analyse_csc(n, rowval, colptr, mf_leaf_size(), mf_small_front(), *S)) { delete S; return nullptr; }
     std::lock_guard<std::mutex> lk(g_mu);
     if (g_symbolic.size() >= 8) {                         // a handful of patterns at most (TE / TM, real / complex tests)
         for (auto& kv : g_pool)

@@ -229,8 +229,8 @@ int mf_push_size() {
 }
 int mf_small_front() {
     const char* e = std::getenv("HMCMT_MF_FSMALL");
-    int v = e ? std::atoi(e) : 144;
-    return v < 0 ? 0 : (v > 144 ? 144 : v);
+    int v = e ? std::atoi(e) : 256;
+    return v < 0 ? 0 : (v > 256 ? 256 : v);
 }
 }  // namespace hmcmt
 

@@ -115,11 +115,14 @@ __device__ __forceinline__ void frag_add(TileFrag& c, const TileFrag& x) {
 //   D  U  = F22 + M' F21^T  accumulated over all pivots in registers                                  -> update tiles = U
 // The update rows never enter the latency-bound sweep: they see two perfectly parallel products with K = all pivots.
 // PC: the tiles hold the pivot columns only (mf_tile<true>); phase D is then the caller's (it gathers F22 from the children).
+// STREAM (PC only): phase C writes -M' = M straight from the registers to the factor arena (mglob, k-grouped, ldm rows) instead
+// of mbuf.
 // scratch: 2 npb tiles (column operands of the sweep; may alias mbuf).  All NW warps call; ends with a CTA barrier.
-template <int NW, bool PC = false>
+template <int NW, bool PC = false, bool STREAM = false>
 __device__ __forceinline__ void mf_front_factor(double* __restrict__ tiles, double* __restrict__ scratch, double* __restrict__ mbuf,
                                                 double* __restrict__ nainv, int* __restrict__ fail, const int nb, const int npb,
-                                                const int sReal, unsigned long long* __restrict__ prof = nullptr) {
+                                                const int sReal, unsigned long long* __restrict__ prof = nullptr,
+                                                double* mglob = nullptr, const int ldm = 0) {
     const int tid = threadIdx.x, lane = tid & 31;
     long long _s0 = prof ? clock64() : 0;
 #define MF_SWEEP_MARK(slot) do { if (prof && tid == 0) { const long long _t = clock64(); atomicAdd(prof + (slot), (unsigned long long)(_t - _s0)); _s0 = _t; } } while (0)
@@ -216,7 +219,13 @@ __device__ __forceinline__ void mf_front_factor(double* __restrict__ tiles, doub
                 frag_mma(c, x, a, b);
             }
             frag_add(c, x);
-            cfrag_store(c, mbuf + (size_t)(Iu * npb + kb) * 128, g, t);
+            if (STREAM) {
+                double* o = mglob + kg_off(ldm, 8 * Iu + g, 8 * kb + 2 * t, 0);
+                *reinterpret_cast<double2*>(o) = make_double2(-c.re[0], -c.re[1]);
+                *reinterpret_cast<double2*>(o + 4 * ldm) = make_double2(-c.im[0], -c.im[1]);
+            } else {
+                cfrag_store(c, mbuf + (size_t)(Iu * npb + kb) * 128, g, t);
+            }
         }
     }
     __syncthreads();
@@ -287,17 +296,17 @@ __device__ __forceinline__ void mf_store_tile(const double* __restrict__ T, doub
 // (register budget: the two- and four-warp instantiations serve the thousands of tiny fronts at the bottom of the tree, where the
 // number of fronts resident per SM hides the latency of the 8x8 inversions: 64 registers per thread -> 16 / 8 CTAs per SM.
 // The 8- and 16-warp instantiations (kMid) keep only the pivot columns in shared memory, so that 4 / 2 of them fit on an SM
-// beside each other: 64 registers per thread as well.)
-template <int NW>
-__global__ void __launch_bounds__(NW * 32, NW <= 4 ? (NW == 1 ? 16 : 32 / NW) : (NW == 8 ? 4 : 2))
-mf_small_kernel(Tables tb, const SmallDesc* __restrict__ descs) {
+// beside each other: 64 registers per thread as well.  STREAM: mf_small_stream_kernel, see there.)
+template <int NW, bool STREAM>
+__device__ __forceinline__ void mf_small_front(const Tables& tb, const SmallDesc* __restrict__ descs) {
     constexpr int NT = NW * 32;
     constexpr bool kMid = NW >= 8;
+    static_assert(!STREAM || kMid, "streamed M' exists in the pivot-column layout only");
     extern __shared__ __align__(16) unsigned char mf_smem[];
     SmallDesc& F = *reinterpret_cast<SmallDesc*>(mf_smem);      // the first kFrontDescBytes of the dynamic block
     const int sys = blockIdx.y, tid = threadIdx.x, lane = tid & 31;
     const int warp = __shfl_sync(0xffffffffu, tid >> 5, 0);
-    constexpr int _pc = NW <= 2 ? 0 : (NW == 4 ? 1 : (NW == 8 ? 2 : 3));      // profiler class
+    constexpr int _pc = NW <= 2 ? 0 : (NW == 4 ? 1 : (NW == 8 ? 2 : 3));      // profiler class (streamed: with the 16 warps)
     long long _t0 = clock64();
     // the front's record: one coalesced read
     static_assert(sizeof(SmallDesc) % 4 == 0 && sizeof(SmallDesc) <= kFrontDescBytes, "SmallDesc is copied word by word into the head of the dynamic shared memory");
@@ -307,8 +316,8 @@ mf_small_kernel(Tables tb, const SmallDesc* __restrict__ descs) {
     const int fp = F.sp + F.up, nb = fp >> 3, npb = F.sp >> 3, nub = nb - npb;
     const int nT = kMid ? mf_pc_row(nb, npb) : nb * (nb + 1) / 2;      // tiles kept in shared memory
     double* tiles = reinterpret_cast<double*>(mf_smem + kFrontDescBytes);
-    double* mbuf = tiles + (size_t)nT * 128;                                   // sweep scratch, then M'
-    double* nainv = mbuf + (size_t)(2 * npb > nub * npb ? 2 * npb : nub * npb) * 128;
+    double* mbuf = tiles + (size_t)nT * 128;                                   // sweep scratch, then M' (unless streamed)
+    double* nainv = mbuf + (size_t)(STREAM || 2 * npb > nub * npb ? 2 * npb : nub * npb) * 128;
     int* fail = reinterpret_cast<int*>(nainv + 128);
     // row maps of all children, back to back, already split into the two address parts of the tile layout: an entry (a, b),
     // a >= b, of the front sits at tiles + rowPart(a) + colPart(b)
@@ -449,7 +458,9 @@ mf_small_kernel(Tables tb, const SmallDesc* __restrict__ descs) {
     }
     __syncthreads();
     MF_PROF_MARK(1);
-    mf_front_factor<NW, kMid>(tiles, mbuf, mbuf, nainv, fail, nb, npb, F.s, tb.prof ? tb.prof + 32 + _pc * 4 : nullptr);
+    double* fac = tb.fac + (size_t)sys * tb.facStride;
+    mf_front_factor<NW, kMid, STREAM>(tiles, mbuf, mbuf, nainv, fail, nb, npb, F.s, tb.prof ? tb.prof + 32 + _pc * 4 : nullptr,
+                                      fac + F.mOff, F.up);
     if (kMid && nub > 0) {
         // ---- D: U = F22 + M' F21^T, lower tiles, two per trip, written from the registers to the update arena.  F22 is gathered
         // from the children's update matrices through the inverse row maps straight into the accumulators: every element starts
@@ -477,42 +488,87 @@ mf_small_kernel(Tables tb, const SmallDesc* __restrict__ descs) {
             *reinterpret_cast<double2*>(o) = make_double2(c.re[0], c.re[1]);
             *reinterpret_cast<double2*>(o + 4 * up) = make_double2(c.im[0], c.im[1]);
         };
-        const int nU = nub * (nub + 1) / 2;
-        int I = 0, J = warp;
-        while (J > I) { J -= I + 1; ++I; }
-        for (int L = warp; L < nU; L += 2 * NW) {
-            const int I0 = I, J0 = J;
-            J += NW;
+        if (!STREAM) {
+            const int nU = nub * (nub + 1) / 2;
+            int I = 0, J = warp;
             while (J > I) { J -= I + 1; ++I; }
-            const bool two = L + NW < nU;
-            const int I1 = I, J1 = J;
-            J += NW;
-            while (J > I) { J -= I + 1; ++I; }
-            TileFrag c0, x0, c1, x1;
-            gather(c0, I0, J0);
-            frag_zero(x0);
-            if (two) { gather(c1, I1, J1); frag_zero(x1); }
-            for (int kb = 0; kb < npb; ++kb) {
-                TileFrag a, b;
-                frag_load(a, mbuf + (size_t)(I0 * npb + kb) * 128, lane);
-                frag_load(b, mf_tile<true>(tiles, npb, npb + J0, kb), lane);
-                frag_mma(c0, x0, a, b);
-                if (two) {
-                    frag_load(a, mbuf + (size_t)(I1 * npb + kb) * 128, lane);
-                    frag_load(b, mf_tile<true>(tiles, npb, npb + J1, kb), lane);
-                    frag_mma(c1, x1, a, b);
+            for (int L = warp; L < nU; L += 2 * NW) {
+                const int I0 = I, J0 = J;
+                J += NW;
+                while (J > I) { J -= I + 1; ++I; }
+                const bool two = L + NW < nU;
+                const int I1 = I, J1 = J;
+                J += NW;
+                while (J > I) { J -= I + 1; ++I; }
+                TileFrag c0, x0, c1, x1;
+                gather(c0, I0, J0);
+                frag_zero(x0);
+                if (two) { gather(c1, I1, J1); frag_zero(x1); }
+                for (int kb = 0; kb < npb; ++kb) {
+                    TileFrag a, b;
+                    frag_load(a, mbuf + (size_t)(I0 * npb + kb) * 128, lane);
+                    frag_load(b, mf_tile<true>(tiles, npb, npb + J0, kb), lane);
+                    frag_mma(c0, x0, a, b);
+                    if (two) {
+                        frag_load(a, mbuf + (size_t)(I1 * npb + kb) * 128, lane);
+                        frag_load(b, mf_tile<true>(tiles, npb, npb + J1, kb), lane);
+                        frag_mma(c1, x1, a, b);
+                    }
                 }
+                frag_add(c0, x0);
+                store(c0, I0, J0);
+                if (two) { frag_add(c1, x1); store(c1, I1, J1); }
             }
-            frag_add(c0, x0);
-            store(c0, I0, J0);
-            if (two) { frag_add(c1, x1); store(c1, I1, J1); }
+        } else {
+            // Streamed M': the A operand is -M from the factor arena, written by this CTA's phase C one barrier ago (plain
+            // coherent loads, never the non-coherent path).  A work item is up to kRow tiles (I, J0 .. J0 + kRow - 1) of one tile
+            // row, so every A fragment read from L2 serves kRow products; the next fragment is requested before the products of
+            // the current one.  Per tile the same operations in the same order as above: U is bit-identical to resident M'.
+            constexpr int kRow = 4;
+            const double* Mg = fac + F.mOff;
+            auto load_a = [&](TileFrag& a, int I, int kb) {
+#pragma unroll
+                for (int kk = 0; kk < 2; ++kk) {
+                    const double* p = Mg + kg_off(up, 8 * I + g, 8 * kb + 4 * kk + t, 0);
+                    a.re[kk] = -p[0];
+                    a.im[kk] = -p[4 * up];
+                }
+            };
+            int I = 0, q = warp;      // item q of row I: tiles J0 = kRow q ...; row I has I / kRow + 1 items
+            while (q > I / kRow) { q -= I / kRow + 1; ++I; }
+            while (I < nub) {
+                const int J0 = kRow * q, nJ = min(kRow, I + 1 - J0);
+                TileFrag c[kRow], x[kRow];
+#pragma unroll
+                for (int r = 0; r < kRow; ++r)
+                    if (r < nJ) { gather(c[r], I, J0 + r); frag_zero(x[r]); }
+                TileFrag a;
+                load_a(a, I, 0);
+                for (int kb = 0; kb < npb; ++kb) {
+                    TileFrag an;
+                    if (kb + 1 < npb) load_a(an, I, kb + 1);
+#pragma unroll
+                    for (int r = 0; r < kRow; ++r)
+                        if (r < nJ) {
+                            TileFrag b;
+                            frag_load(b, mf_tile<true>(tiles, npb, npb + J0 + r, kb), lane);
+                            frag_mma(c[r], x[r], a, b);
+                        }
+                    a = an;
+                }
+#pragma unroll
+                for (int r = 0; r < kRow; ++r)
+                    if (r < nJ) { frag_add(c[r], x[r]); store(c[r], I, J0 + r); }
+                q += NW;
+                while (I < nub && q > I / kRow) { q -= I / kRow + 1; ++I; }
+            }
         }
         if (tb.prof && tid == 0) atomicAdd(tb.prof + 32 + _pc * 4 + 3, (unsigned long long)(clock64() - tD));
     }
     MF_PROF_MARK(4);
     if (tid == 0 && *fail) tb.status[sys] = kErrSingular;
-    // outputs, tile by tile: G = -(pivot x pivot), M = -M' (factor arena), U = update x update (update arena, lower tiles)
-    double* fac = tb.fac + (size_t)sys * tb.facStride;
+    // outputs, tile by tile: G = -(pivot x pivot), M = -M' (factor arena; streamed: already there), U = update x update (update
+    // arena, lower tiles)
     const int sp = F.sp, up = F.up;
     {
         double* G = fac + F.gOff;
@@ -522,7 +578,7 @@ mf_small_kernel(Tables tb, const SmallDesc* __restrict__ descs) {
                 else mf_store_tile<true>(mf_tile(tiles, J, I), G, sp, I * 8, J * 8, -1.0, lane);
             }
     }
-    if (up > 0) {
+    if (!STREAM && up > 0) {
         double* M = fac + F.mOff;
         for (int I = warp; I < nub; I += NW)
             for (int J = 0; J < npb; ++J) mf_store_tile<false>(mbuf + (size_t)(I * npb + J) * 128, M, up, I * 8, J * 8, -1.0, lane);
@@ -539,6 +595,17 @@ mf_small_kernel(Tables tb, const SmallDesc* __restrict__ descs) {
     }
     MF_PROF_MARK(5);
     if (tb.prof && tid == 0) { atomicAdd(tb.prof + _pc * 8 + 6, 1ull); atomicAdd(tb.prof + _pc * 8 + 7, (unsigned long long)npb); }
+}
+
+template <int NW>
+__global__ void __launch_bounds__(NW * 32, NW <= 4 ? (NW == 1 ? 16 : 32 / NW) : (NW == 8 ? 4 : 2))
+mf_small_kernel(Tables tb, const SmallDesc* __restrict__ descs) {
+    mf_small_front<NW, false>(tb, descs);
+}
+// Fronts whose pivot columns fit in shared memory but not together with M' (more than 144 rows): M' goes through the factor
+// arena (L2).  Such a front takes most of an SM's shared memory, so one CTA per SM: 16 warps with up to 128 registers.
+__global__ void __launch_bounds__(16 * 32, 1) mf_small_stream_kernel(Tables tb, const SmallDesc* __restrict__ descs) {
+    mf_small_front<16, true>(tb, descs);
 }
 
 // ------------------------------------------------------------------------------------------------------------------------

@@ -30,6 +30,12 @@ int launch_small(cudaStream_t st, const Tables& tb, const SmallDesc* list, int n
     mf_small_kernel<NW><<<dim3(n, nsys), NW * 32, smem, st>>>(tb, list);
     return kOk;
 }
+int launch_stream(cudaStream_t st, const Tables& tb, const SmallDesc* list, int n, int nsys, size_t smem) {
+    static PerDeviceOnceMf once;
+    if (once.need()) HMCMT_CUDA_TRY(cudaFuncSetAttribute(mf_small_stream_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxSmem));
+    mf_small_stream_kernel<<<dim3(n, nsys), 16 * 32, smem, st>>>(tb, list);
+    return kOk;
+}
 }  // namespace
 
 template <typename Tp>
@@ -136,13 +142,16 @@ int Solver::build(int nsys_, int maxRhs_, int64_t valCount_) {
         if (D.nSmall) {
             int mx = 0;
             for (int k : sm) mx = std::max(mx, S.fronts[k].fp());
-            D.smallWarps = mf_small_warps(mx, knobs);
+            D.smallStream = mf_small_stream(S, sm);
+            D.smallWarps = D.smallStream ? 16 : mf_small_warps(mx, knobs);
             D.smallSmem = 0;
             std::vector<SmallDesc> descs;
             for (int k : sm) {
                 const Front& F = S.fronts[k];
-                D.smallSmem = std::max(D.smallSmem, D.smallWarps >= 8 ? mf_mid_front_smem_bytes(F.fp() / 8, F.sp / 8, mf_rel_total(S, k), F.nChild)
-                                                                      : mf_front_smem_bytes(F.fp() / 8, F.sp / 8, mf_rel_total(S, k)));
+                const int nb = F.fp() / 8, npb = F.sp / 8, rt = mf_rel_total(S, k);
+                D.smallSmem = std::max(D.smallSmem, D.smallStream ? mf_stream_front_smem_bytes(nb, npb, rt, F.nChild)
+                                                    : D.smallWarps >= 8 ? mf_mid_front_smem_bytes(nb, npb, rt, F.nChild)
+                                                                        : mf_front_smem_bytes(nb, npb, rt));
                 SmallDesc sd{};
                 sd.sp = F.sp; sd.up = F.up; sd.s = F.s; sd.nChild = F.nChild; sd.nOrig = F.nOrig; sd.origPtr = F.origPtr;
                 sd.par = F.depth & 1; sd.front = k;
@@ -158,6 +167,7 @@ int Solver::build(int nsys_, int maxRhs_, int64_t valCount_) {
                 descs.push_back(sd);
             }
             SmallDesc* pd = nullptr;
+            if (D.smallSmem > kMaxSmem) return kErrArg;
             MF_TRY(upload(descs, &pd));
             D.smallDescs = pd;
         }
@@ -296,7 +306,8 @@ int Solver::factor(cudaStream_t st, int* dStatus, int64_t* nLaunches, int sys0, 
         const DepthSchedule& D = sched[d];
         if (D.nSmall) {
             int rc = kOk;
-            if (D.smallWarps == 1) rc = launch_small<1>(st, tb, D.smallDescs, D.nSmall, nsys, D.smallSmem);
+            if (D.smallStream) rc = launch_stream(st, tb, D.smallDescs, D.nSmall, nsys, D.smallSmem);
+            else if (D.smallWarps == 1) rc = launch_small<1>(st, tb, D.smallDescs, D.nSmall, nsys, D.smallSmem);
             else if (D.smallWarps == 2) rc = launch_small<2>(st, tb, D.smallDescs, D.nSmall, nsys, D.smallSmem);
             else if (D.smallWarps == 4) rc = launch_small<4>(st, tb, D.smallDescs, D.nSmall, nsys, D.smallSmem);
             else if (D.smallWarps == 8) rc = launch_small<8>(st, tb, D.smallDescs, D.nSmall, nsys, D.smallSmem);

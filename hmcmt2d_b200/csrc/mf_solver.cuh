@@ -43,6 +43,7 @@ struct SolveDesc {
 
 struct DepthSchedule {
     int nSmall = 0, smallWarps = 4;
+    bool smallStream = false;                // M' streamed through the factor arena (mf_small_stream_kernel, 16 warps)
     size_t smallSmem = 0;
     const SmallDesc* smallDescs = nullptr;
     int nBig = 0;

@@ -40,14 +40,32 @@ inline size_t mf_front_smem_bytes(int nb, int npb, int relTotal = 0) {
 }
 // The 8- and 16-warp instantiations (launches whose largest front has more than 64 rows) keep only the pivot columns: the
 // pivot triangle and the F21 block, no F22 (gathered from the children straight into the registers of the Schur product),
-// plus one inverse row map of the update rows per child (nChild x (nb - npb) * 8 ints).  The small / global-memory
-// classification (Symbolic::fronts[].isBig) stays on mf_front_smem_bytes, so this layout moves no front between the paths.
+// plus one inverse row map of the update rows per child (nChild x (nb - npb) * 8 ints).  M' = F21 (-G) stays in shared
+// memory beside them (resident M').
 inline size_t mf_mid_front_smem_bytes(int nb, int npb, int relTotal, int nChild) {
     const size_t nub = (size_t)(nb - npb), nT = (size_t)npb * (npb + 1) / 2 + nub * npb, nS = 2 * (size_t)npb, nM = nub * npb;
     return kFrontDescBytes + (nT + (nS > nM ? nS : nM) + 1) * 128 * sizeof(double) + 16 + (((size_t)relTotal + 1) & ~(size_t)1) * 2 * sizeof(int) +
            (size_t)nChild * nub * 8 * sizeof(int);
 }
+// The same layout without M' (streamed M', mf_small_stream_kernel): the products write M' to the factor arena as M and the
+// Schur product reads it back from there (L2), so shared memory holds the pivot columns, the sweep scratch and the row maps.
+inline size_t mf_stream_front_smem_bytes(int nb, int npb, int relTotal, int nChild) {
+    const size_t nub = (size_t)(nb - npb), nT = (size_t)npb * (npb + 1) / 2 + nub * npb, nS = 2 * (size_t)npb;
+    return kFrontDescBytes + (nT + nS + 1) * 128 * sizeof(double) + 16 + (((size_t)relTotal + 1) & ~(size_t)1) * 2 * sizeof(int) +
+           (size_t)nChild * nub * 8 * sizeof(int);
+}
 constexpr size_t kFrontSmemMax = 227 * 1024;
+// Fronts of up to kFullFrontMaxFp rows are classified on the whole-front layout (mf_front_smem_bytes), whatever instantiation
+// later runs them.  Larger ones (up to fSmall) run in the pivot-column layout of the 8 / 16-warp instantiations: with M' in
+// shared memory when that fits, else with M' streamed through the factor arena.
+constexpr int kFullFrontMaxFp = 144;
+inline bool mf_front_needs_stream(int nb, int npb, int relTotal, int nChild) {
+    return mf_mid_front_smem_bytes(nb, npb, relTotal, nChild) > kFrontSmemMax;
+}
+inline size_t mf_large_front_smem_bytes(int nb, int npb, int relTotal, int nChild) {
+    return mf_front_needs_stream(nb, npb, relTotal, nChild) ? mf_stream_front_smem_bytes(nb, npb, relTotal, nChild)
+                                                            : mf_mid_front_smem_bytes(nb, npb, relTotal, nChild);
+}
 
 // lower-triangular entry of the original matrix (row >= col, original numbering) and where its value comes from
 struct Entry {
@@ -430,7 +448,9 @@ inline bool mf_symbolic(int N, const std::vector<std::vector<int>>& snodes, cons
         int relTotal = 0;
         for (int c = 0; c < F.nChild; ++c) relTotal += S.fronts[S.children[F.childPtr + c]].u;
         // (the single-CTA kernel's front record describes up to kSmallChildren children)
-        F.isBig = (fp > fSmall || F.nChild > kSmallChildren || mf_front_smem_bytes(fp / 8, F.sp / 8, relTotal) > kFrontSmemMax) ? 1 : 0;
+        const size_t smem = fp <= kFullFrontMaxFp ? mf_front_smem_bytes(fp / 8, F.sp / 8, relTotal)
+                                                  : mf_large_front_smem_bytes(fp / 8, F.sp / 8, relTotal, F.nChild);
+        F.isBig = (fp > fSmall || F.nChild > kSmallChildren || smem > kFrontSmemMax) ? 1 : 0;
         S.maxFp = std::max(S.maxFp, fp);
         (F.isBig ? S.maxFpBig : S.maxFpSmall) = std::max(F.isBig ? S.maxFpBig : S.maxFpSmall, fp);
         (F.isBig ? S.byDepthBig : S.byDepthSmall)[F.depth].push_back(k);
@@ -500,9 +520,18 @@ struct SchedKnobs {
 };
 
 // warps per front of a single-CTA launch, by the largest front of the launch (measured optimum at cfg2; one warp per front needs
-// no CTA barrier)
+// no CTA barrier).  Fronts above kFullFrontMaxFp rows exist only in the pivot-column layout: at least 8 warps.
 inline int mf_small_warps(int maxFp, const SchedKnobs& k) {
-    return maxFp <= k.fp1 ? 1 : (maxFp <= k.fp2 ? 2 : (maxFp <= k.fp4 ? 4 : (maxFp <= k.fp8 ? 8 : 16)));
+    const int w = maxFp <= k.fp1 ? 1 : (maxFp <= k.fp2 ? 2 : (maxFp <= k.fp4 ? 4 : (maxFp <= k.fp8 ? 8 : 16)));
+    return maxFp > kFullFrontMaxFp && w < 8 ? 8 : w;
+}
+// a single-CTA launch streams M' (16 warps, mf_small_stream_kernel) when one of its fronts needs it
+inline bool mf_small_stream(const Symbolic& S, const std::vector<int>& launch) {
+    for (int k : launch) {
+        const Front& F = S.fronts[k];
+        if (F.fp() > kFullFrontMaxFp && mf_front_needs_stream(F.fp() / 8, F.sp / 8, mf_rel_total(S, k), F.nChild)) return true;
+    }
+    return false;
 }
 // solves: one warp per front (record-driven kernels) for small fronts with few children, one CTA per front otherwise
 inline bool mf_solve_by_warp(const Front& F) { return !F.isBig && F.fp() <= kSolveWarpMaxFp && F.nChild <= kSmallChildren; }

@@ -254,6 +254,22 @@ class Plan:
         _lib.check(self.L.hmcmt_jacobian(self.h, J.ctypes.data_as(C.POINTER(C.c_double))), "hmcmt_jacobian")
         return J
 
+    def jvec(self, dsig):
+        """J dsig for the last forward evaluation, J being what `jacobian` returns: dsig [nChains, nAC] conductivity perturbation
+        of the active cells -> [nChains, nData] (complex, or real rows for Rho_Pha), without forming J."""
+        d = np.ascontiguousarray(dsig, dtype=np.float64).reshape(self.nChains, self.nAC)
+        jv = np.zeros((self.nChains, self.nData), dtype=self.dtype)
+        _lib.check(self.L.hmcmt_jvec(self.h, _lib.f64(d), jv.ctypes.data_as(C.POINTER(C.c_double))), "hmcmt_jvec")
+        return jv
+
+    def gn_hessvec(self, v, total=False):
+        """Gauss-Newton Hessian of the data misfit in ln(sigma) times v: D Re(J^H Wd^2 J) D v, D = diag(sigma_active), for the
+        last forward evaluation; total=True adds the model-norm part beta Wm v."""
+        vv = self._m(v)
+        hv = np.zeros((self.nChains, self.nAC))
+        _lib.check(self.L.hmcmt_gn_hessvec(self.h, _lib.f64(vv), 1 if total else 0, _lib.f64(hv)), "hmcmt_gn_hessvec")
+        return hv
+
     def forward_gradient(self, m, total=False):
         """compDataGradient (HMCSampler.jl:277-330): predicted data, data misfit, gradient w.r.t. ln(sigma).  total=True adds the
         model-norm part beta Wm (m - m_ref) on the device (m_ref from set_state), as proposeLeapfrog does right afterwards."""
@@ -597,6 +613,26 @@ def compJacTMatVec(exTE, hxTM, datVec, mt2dMesh, mtData, activeCell=None, AinvTE
         full[pl._keep["act"]] = g
         return np.asarray(activeCell.T @ full).reshape(-1)
     return g
+
+
+def compJacMatVec(exTE, hxTM, dsig, mt2dMesh, mtData, activeCell=None, AinvTE=None, AinvTM=None):
+    """J dsig, the forward-mode twin of `compJacTMatVec`: the predicted impedances' derivative along the conductivity
+    perturbation dsig of the active cells (the columns of activeCell, or the plan's own active set), for the fields / factors of
+    the MT2DFwdData the handles belong to.  Equals compJacMat(...) @ dsig without forming the matrix."""
+    h = AinvTE if isinstance(AinvTE, FactorHandle) else AinvTM
+    if not isinstance(h, FactorHandle):
+        raise ValueError("compJacMatVec needs the factor handle returned by MT2DFwdSolver (AinvTE/AinvTM)")
+    pl = h.plan
+    if h.generation != pl.generation:
+        raise RuntimeError("compJacMatVec: the factors of this MT2DFwdData were overwritten by a later evaluation on the same "
+                           "mesh / survey; call MT2DFwdSolver again (one set of factors is kept resident per plan)")
+    if "Rho_Pha" in mtData.dataType:
+        raise NotImplementedError("explicit Jacobian products: Impedance data only, as compJacMat (Plan.jvec serves Rho_Pha)")
+    d = np.asarray(dsig, dtype=np.float64).reshape(-1)
+    if activeCell is not None:
+        # map by cell index, whatever the caller's selector looks like (the plan's active set is 'all non-air cells')
+        d = np.asarray(activeCell @ d).reshape(-1)[pl._keep["act"]]
+    return pl.jvec(d)[0]
 
 
 def compJacMat(exTE, hxTM, mt2dMesh, mtData, activeCell=None, AinvTE=None, AinvTM=None, linSolver: str = "b200"):

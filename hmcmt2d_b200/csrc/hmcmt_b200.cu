@@ -82,6 +82,11 @@ struct hmcmt_plan {
     DevBuf<double> xbuf, Gpart, phiPart, phi, gsig, gdata, gtotal, energies, panels, curM, curP, chainScal, zmom;
     DevBuf<int> fid, iL, iR, tjL, tjR, cell2act, act2cell, wmPtr, wmIdx, status, driftFlag, packed2full, full2packed, Lsteps;
     DevBuf<cplx> obs, bc, bcs, rhs, x, F, lam, Lam, srows, qrow, scratch, predFull, ainvz, zadj, vin, predPacked, wexp, conCols, respFull;
+    // tangent mode (hmcmt_jvec / hmcmt_gn_hessvec), allocated on first use: dbc [nSys][nb], the full-layout tangent jvFull
+    // [nChains][nFull], the conductivity direction dsigA [nChains][nAC] and the Gauss-Newton product's [v | 0 | gsig | gdata |
+    // gtotal] (gnBuf, 5 [nChains][nAC]: k_reduce_grad writes there, so the plan's own gradient stays)
+    DevBuf<cplx> dbc, jvFull;
+    DevBuf<double> dsigA, gnBuf;
     DevBuf<BandSys> sysDesc;
     DevBuf<SolveJob> jobs, fwdJobs;                 // fwdJobs: back-substitution sweeps of the fused forward systems (split systems)
     // wide meshes (half-bandwidth > 104): nested-dissection multifrontal solver (mf_solver.cuh) instead of the band kernels
@@ -704,6 +709,9 @@ int compute_step_graph(hmcmt_plan* pl) {
             return compute_step_eager(pl);
         }
         cudaGraphDestroy(graph);
+        // evJoin was last recorded inside the capture and cannot be waited on outside it; the replays join the side stream
+        // inside the graph, so an eager wait after them (hmcmt_jtvec, hmcmt_jvec, hmcmt_gn_hessvec) has nothing left to wait for
+        HMCMT_CUDA_TRY(cudaEventRecord(pl->evJoin, pl->side));
         pl->graphState = 2;
     }
     HMCMT_CUDA_TRY(cudaGraphLaunch(pl->graphExec, pl->stream));
@@ -1195,7 +1203,7 @@ void hmcmt_destroy(hmcmt_plan* pl) {
     pl->driftFlag.release(); pl->packed2full.release(); pl->full2packed.release(); pl->Lsteps.release(); pl->obs.release(); pl->bc.release(); pl->bcs.release();
     pl->rhs.release(); pl->x.release(); pl->F.release(); pl->lam.release(); pl->Lam.release(); pl->srows.release(); pl->qrow.release();
     pl->scratch.release(); pl->predFull.release(); pl->ainvz.release(); pl->zadj.release(); pl->vin.release();
-    pl->predPacked.release(); pl->conCols.release(); pl->xbuf.release(); pl->wexp.release(); pl->respFull.release(); pl->gradK.release(); pl->Lband.release(); pl->massBuf.release(); pl->massStatus.release(); delete pl->massSolver; pl->massSolver = nullptr; pl->mfSys.release(); delete pl->mfs; pl->mfs = nullptr; pl->fwdJobs.release(); pl->sysDesc.release(); pl->jobs.release();
+    pl->predPacked.release(); pl->conCols.release(); pl->dbc.release(); pl->jvFull.release(); pl->dsigA.release(); pl->gnBuf.release(); pl->xbuf.release(); pl->wexp.release(); pl->respFull.release(); pl->gradK.release(); pl->Lband.release(); pl->massBuf.release(); pl->massStatus.release(); delete pl->massSolver; pl->massSolver = nullptr; pl->mfSys.release(); delete pl->mfs; pl->mfs = nullptr; pl->fwdJobs.release(); pl->sysDesc.release(); pl->jobs.release();
     if (pl->pin) cudaFreeHost(pl->pin);
     delete pl;
 }
@@ -1504,6 +1512,106 @@ int hmcmt_jacobian(hmcmt_plan* pl, double* J) {
     // the adjoint passes overwrote the responses / misfit of the data residual: restore them for later calls
     rc = rx_phase(pl, false, nullptr);
     if (rc) return rc;
+    return check_status(pl);
+}
+
+// the tangent buffers, allocated on first use so that plans that never ask for J v carry none of them
+static int ensure_tangent(hmcmt_plan* pl) {
+    if (pl->jvFull.p) return kOk;
+    const MeshDev& M = pl->M;
+    int rc;
+    if ((rc = pl->dbc.alloc((size_t)pl->nSys * M.nb)) || (rc = pl->dsigA.alloc((size_t)pl->nChains * pl->nAC))) return rc;
+    const size_t smem = (size_t)(6 * (M.ny + 1) + 2 * M.ny) * sizeof(cplx);
+    auto k = pl->dataKind ? k_rx_tangent<true, false> : pl->tipper ? k_rx_tangent<false, true> : k_rx_tangent<false, false>;
+    if (smem > 48 * 1024) HMCMT_CUDA_TRY(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    return pl->jvFull.alloc((size_t)pl->nChains * pl->nFull);
+}
+
+// jvFull <- J dsigA for the resident state: dbc = dBC dsig, the tangent right-hand side, one solve per system with the resident
+// factors (the multifrontal path back-substitutes only the receiver path: only rows zid, zid + 1 are read), the tangent field
+// on those rows and the tangent receiver functional.  Overwrites lam and the receiver rows of Lam.
+static int jvec_device(hmcmt_plan* pl) {
+    const MeshDev& M = pl->M;
+    cudaStream_t st = pl->stream;
+    const int nSys = pl->nSys;
+    int rc = kOk;
+    if (!pl->haveSens && (rc = launch_sens_side(pl))) return rc;
+    HMCMT_CUDA_TRY(cudaStreamWaitEvent(st, pl->evJoin, 0));
+    k_bc_tangent<<<dim3((M.ny + 1 + 127) / 128, nSys), 128, 0, st>>>(M, pl->sm, pl->freqs.p, pl->cell2act.p, pl->dsigA.p, pl->nAC,
+                                                                     pl->scratch.p, pl->dbc.p);
+    LAUNCH_CHECK(pl);
+    k_tangent_rhs<<<dim3((M.N + 255) / 256, nSys), 256, 0, st>>>(M, pl->sm, pl->freqs.p, pl->sigma.p, pl->cell2act.p, pl->dsigA.p, pl->nAC,
+                                                                 pl->F.p, pl->bcs.p, pl->dbc.p, pl->lam.p);
+    LAUNCH_CHECK(pl);
+    if (pl->useMf) {
+        if ((rc = pl->mfs->forward_slot(st, 0, pl->lam.p, M.N, &pl->launches, 0, nSys, 0)) ||
+            (rc = pl->mfs->backward_slot(st, 0, pl->lam.p, M.N, &pl->launches, 0, nSys, pl->patRx)))
+            return rc;
+    } else {
+        if ((rc = launch_solve(st, pl->T, pl->jobs.p, nSys, pl->dom))) return rc;
+        pl->launches += pl->dom.split ? 3 : 1;
+    }
+    const int rx0 = M.zid * (M.ny + 1), rx1 = (M.zid + 2) * (M.ny + 1);
+    k_node_field<<<dim3((rx1 - rx0 + 255) / 256, nSys), 256, 0, st>>>(M, pl->lam.p, pl->dbc.p, pl->Lam.p, 0, rx0, rx1);
+    LAUNCH_CHECK(pl);
+    const size_t smem = (size_t)(6 * (M.ny + 1) + 2 * M.ny) * sizeof(cplx);
+    auto k = pl->dataKind ? k_rx_tangent<true, false> : pl->tipper ? k_rx_tangent<false, true> : k_rx_tangent<false, false>;
+    k<<<nSys, kRxThreads, smem, st>>>(M, pl->rx, pl->sm, pl->cm, pl->freqs.p, pl->sigma.p, pl->cell2act.p, pl->dsigA.p, pl->nAC, pl->F.p,
+                                      pl->Lam.p, pl->jvFull.p);
+    LAUNCH_CHECK(pl);
+    return kOk;
+}
+
+int hmcmt_jvec(hmcmt_plan* pl, const double* dsig, double* jv) {
+    if (!pl || !dsig || !jv || !pl->haveForward) return kErrArg;
+    HMCMT_CUDA_TRY(cudaSetDevice(pl->device));
+    int rc = ensure_tangent(pl);
+    if (rc) return rc;
+    cudaStream_t st = pl->stream;
+    HMCMT_CUDA_TRY(cudaMemcpyAsync(pl->dsigA.p, dsig, sizeof(double) * (size_t)pl->nChains * pl->nAC, cudaMemcpyHostToDevice, st));
+    if ((rc = jvec_device(pl))) return rc;
+    // packed order through the prediction packers, staged in vin (adjoint scratch: the predictions stay as they are)
+    const dim3 grid((pl->nData + 255) / 256, pl->nChains);
+    if (pl->dataKind)
+        k_pack_pred_real<<<grid, 256, 0, st>>>(pl->nData, pl->nFull, pl->packed2full.p, reinterpret_cast<const double*>(pl->jvFull.p),
+                                               reinterpret_cast<double*>(pl->vin.p));
+    else
+        k_pack_pred<<<grid, 256, 0, st>>>(pl->nData, pl->nFull, pl->packed2full.p, pl->jvFull.p, pl->vin.p);
+    LAUNCH_CHECK(pl);
+    HMCMT_CUDA_TRY(cudaMemcpyAsync(jv, pl->vin.p, datum_bytes(pl) * (size_t)pl->nChains * pl->nData, cudaMemcpyDeviceToHost, st));
+    HMCMT_CUDA_TRY(cudaStreamSynchronize(st));
+    return check_status(pl);
+}
+
+int hmcmt_gn_hessvec(hmcmt_plan* pl, const double* v, int32_t with_prior, double* hv) {
+    if (!pl || !v || !hv || !pl->haveForward) return kErrArg;
+    HMCMT_CUDA_TRY(cudaSetDevice(pl->device));
+    int rc = ensure_tangent(pl);
+    if (rc) return rc;
+    const MeshDev& M = pl->M;
+    cudaStream_t st = pl->stream;
+    const size_t nA = (size_t)pl->nChains * pl->nAC;
+    if (!pl->gnBuf.p) {
+        if ((rc = pl->gnBuf.alloc(5 * nA))) return rc;
+        HMCMT_CUDA_TRY(cudaMemsetAsync(pl->gnBuf.p + nA, 0, sizeof(double) * nA, st));      // m_ref = 0 of the prior term
+    }
+    double *vD = pl->gnBuf.p, *zero = vD + nA, *gs = zero + nA, *gd = gs + nA, *gt = gd + nA;
+    HMCMT_CUDA_TRY(cudaMemcpyAsync(vD, v, sizeof(double) * nA, cudaMemcpyHostToDevice, st));
+    const dim3 gA((pl->nAC + 255) / 256, pl->nChains);
+    k_sigma_scale<<<gA, 256, 0, st>>>(pl->nAC, M.nCell, pl->act2cell.p, pl->sigma.p, vD, pl->dsigA.p);
+    LAUNCH_CHECK(pl);
+    if ((rc = jvec_device(pl))) return rc;
+    k_gn_weight<<<dim3((pl->nFull + 255) / 256, pl->nChains), 256, 0, st>>>(pl->nFull, pl->dataKind, pl->wd.p, pl->wdPha.p, pl->jvFull.p,
+                                                                            pl->vin.p);
+    LAUNCH_CHECK(pl);
+    // J^T of the weighted tangent through the adjoint machinery (the receiver functional recomputes the same predictions and
+    // misfit from the unchanged fields), then the chain rule and prior term of the gradient's reduction with (m, m_ref) = (v, 0)
+    if ((rc = rx_phase(pl, true, pl->vin.p)) || (rc = adjoint_phase(pl, false))) return rc;
+    k_reduce_grad<<<gA, 256, 0, st>>>(pl->nAC, M.nCell, pl->nSysPerChain, pl->act2cell.p, pl->Gpart.p, vD, zero, pl->wmPtr.p, pl->wmIdx.p,
+                                      pl->wmVal.p, pl->beta, pl->sigma.p, gs, gd, gt);
+    LAUNCH_CHECK(pl);
+    HMCMT_CUDA_TRY(cudaMemcpyAsync(hv, with_prior ? gt : gd, sizeof(double) * nA, cudaMemcpyDeviceToHost, st));
+    HMCMT_CUDA_TRY(cudaStreamSynchronize(st));
     return check_status(pl);
 }
 

@@ -933,6 +933,282 @@ k_contract_cells(MeshDev M, SysMap sm, const double* __restrict__ freqs, const d
 }
 
 // ---------------------------------------------------------------------------------------------
+// K12: tangent (forward) mode J dsig, the transpose of K9 / K10 / the adjoint of K6+K7 term by term (hmcmt_jvec, DESIGN 4.7).
+// dsig [nChains][nAC] is the conductivity perturbation of the active cells; an inactive cell has none.
+__device__ __forceinline__ double dsig_cell(const int* __restrict__ cell2act, const double* __restrict__ dsig, int c) {
+    const int a = cell2act[c];
+    return a >= 0 ? dsig[a] : 0.0;
+}
+// sum_kp ds(kp) dF[row][kp] of the columns sens_column computes, rows 1..nz into out[0..nz-1] (or null: the last row only,
+// returned).  The columns share one recursion over the layers; only their starting values (through Z_top) and the two layer
+// matrices a column's own layer enters differ, so the sum runs that recursion once with the weighted sums of those terms.
+// The overflow guard of sens_column: rows past jb+1 are zero and row jb+1 keeps the columns kp <= jb only — a second state
+// `lo` carries the part of the sum from those columns (the deeper ones enter rows <= jb only through Z_top).
+template <typename DS>
+__device__ cplx sens_tangent(const MeshDev& M, const ProfScalars& P, int mode, double omu, DS ds, cplx* __restrict__ out) {
+    const int nz = M.nz, jb = *P.jbreak;
+    const cplx z1 = *P.z1, k1 = P.ka[0], zero = mk(0.0, 0.0), one = mk(1.0, 0.0);
+    cplx dz = zero, dzLo = zero;
+    for (int kp = 0; kp < nz; ++kp) {
+        const cplx t = ds(kp) * P.dz1[kp];
+        dz += t;
+        if (kp <= jb) dzLo += t;
+    }
+    const cplx dk0 = ds(0) * P.dka[0];
+    auto start = [&](cplx d, cplx& eu, cplx& ed) {
+        if (mode == 0) {
+            eu = 0.5 * omu / (z1 * k1) * (one / z1 * d + one / k1 * dk0);
+            ed = -eu;
+        } else {
+            const cplx a = (omu / (k1 * k1)) * dk0;
+            eu = 0.5 * (d + a);
+            ed = 0.5 * (d - a);
+        }
+    };
+    cplx Eu, Ed, Lu, Ld;
+    start(dz, Eu, Ed);
+    start(dzLo, Lu, Ld);
+    cplx last = zero;
+    for (int j = 0; j < nz; ++j) {
+        cplx dF = zero;
+        if (j <= jb) {
+            const cplx eu = P.eu[j], ed = P.ed[j];
+            const double sj = ds(j), sn = (j + 1 < nz && j < jb) ? ds(j + 1) : 0.0;   // columns kp = j, j+1 (kp = jb+1 is cut)
+            const cplx* S = P.dS + 4 * j;
+            const cplx* N = P.dN + 4 * j;
+            const cplx iu = sj * (S[0] * eu + S[1] * ed) + sn * (N[0] * eu + N[1] * ed);
+            const cplx id = sj * (S[2] * eu + S[3] * ed) + sn * (N[2] * eu + N[3] * ed);
+            const cplx bu = (j == jb) ? Lu : Eu, bd = (j == jb) ? Ld : Ed;
+            const cplx nEu = 0.5 * (P.m11[j] * bu + P.m12[j] * bd + iu);
+            const cplx nEd = 0.5 * (P.m21[j] * bu + P.m22[j] * bd + id);
+            if (j < jb) {
+                const cplx lu = 0.5 * (P.m11[j] * Lu + P.m12[j] * Ld + iu);
+                Ld = 0.5 * (P.m21[j] * Lu + P.m22[j] * Ld + id);
+                Lu = lu;
+            }
+            Eu = nEu; Ed = nEd;
+            if (mode == 0) dF = nEu + nEd;
+            else {
+                const cplx kao = P.kao[j], dk1 = sn * P.dka[j + 1];
+                dF = (kao * nEd - kao * nEu) + (P.ed[j + 1] / omu) * dk1 - (P.eu[j + 1] / omu) * dk1;
+            }
+        }
+        if (out) out[j] = dF;
+        last = dF;
+    }
+    return last;
+}
+// dbc = dBC dsig: one thread per profile p of a system (p = 0 left, 1 right column, p >= 2 bottom node jn = p - 1), each
+// O(nz); the top row has no derivative.  grid (ceil((ny+1)/128), nSys), block 128
+__global__ void __launch_bounds__(128)
+k_bc_tangent(MeshDev M, SysMap sm, const double* __restrict__ freqs, const int* __restrict__ cell2act, const double* __restrict__ dsig,
+             int nAC, const cplx* __restrict__ scratch, cplx* __restrict__ dbc) {
+    const int p = blockIdx.x * blockDim.x + threadIdx.x, sys = blockIdx.y, ny = M.ny, nz = M.nz;
+    if (p > ny) return;
+    int ch, mi, mode, f;
+    sys_decode(sm, sys, ch, mi, mode, f);
+    const double omu = 2.0 * kPi * freqs[f] * kMu0;
+    const double* ds = dsig + (size_t)ch * nAC;
+    cplx* b = dbc + (size_t)sys * M.nb;
+    b[p] = mk(0.0, 0.0);                                                  // top row (ny + 1 entries, one per thread)
+    const int pr = p < 2 ? p : 2;
+    const ProfScalars P = prof_ptrs(const_cast<cplx*>(scratch) + ((size_t)sys * 3 + pr) * prof_stride(nz), nz);
+    if (pr < 2) {
+        const int jc = pr == 0 ? 0 : ny - 1;
+        sens_tangent(M, P, mode, omu, [&](int k) { return dsig_cell(cell2act, ds, k * ny + jc); }, b + ny + 1 + pr * nz);
+    } else {
+        const int jn = p - 1;
+        const double yl = M.yLen[jn - 1], yr = M.yLen[jn], wl = yl / (yl + yr), wr = yr / (yl + yr);     // the colw weights
+        b[ny + 1 + 2 * nz + (jn - 1)] = sens_tangent(
+            M, P, mode, omu, [&](int k) { return wl * dsig_cell(cell2act, ds, k * ny + jn - 1) + wr * dsig_cell(cell2act, ds, k * ny + jn); },
+            nullptr);
+    }
+}
+
+// tangent right-hand side on the interior unknowns (internal ordering): the coefficient of Lambda_n in k_contract_cells applied
+// to dsig, plus W dbc of the t = W lambda + s step of k_contract_cols.  grid (ceil(N/256), nSys)
+__global__ void __launch_bounds__(256)
+k_tangent_rhs(MeshDev M, SysMap sm, const double* __restrict__ freqs, const double* __restrict__ sigma, const int* __restrict__ cell2act,
+              const double* __restrict__ dsig, int nAC, const cplx* __restrict__ F, const cplx* __restrict__ bcs,
+              const cplx* __restrict__ dbc, cplx* __restrict__ rhs) {
+    const int q = blockIdx.x * blockDim.x + threadIdx.x;
+    if (q >= M.N) return;
+    const int sys = blockIdx.y, ny = M.ny, nz = M.nz;
+    int ch, mi, mode, f;
+    sys_decode(sm, sys, ch, mi, mode, f);
+    int jn, kn;
+    jk_of(M, q, jn, kn);
+    const double omega = 2.0 * kPi * freqs[f];
+    const double* sig = sigma + (size_t)ch * M.nCell;
+    const double* ds = dsig + (size_t)ch * nAC;
+    const cplx* Fs = F + (size_t)sys * M.nNode;
+    const cplx* bs = bcs + (size_t)sys * M.nb;
+    auto node = [&](int j, int k) { return (size_t)k * (ny + 1) + j; };
+    auto Hf = [&](int j, int k) -> cplx {
+        if (j >= 1 && j <= ny - 1 && k >= 1 && k <= nz - 1) return Fs[node(j, k)];
+        if (k == 0) return bs[j];
+        if (j == 0) return bs[ny + 1 + (k - 1)];
+        if (j == ny) return bs[ny + 1 + nz + (k - 1)];
+        return bs[ny + 1 + 2 * nz + (j - 1)];
+    };
+    cplx r = mk(0.0, 0.0);
+#pragma unroll
+    for (int dk = 0; dk < 2; ++dk)
+#pragma unroll
+        for (int dj = 0; dj < 2; ++dj) {
+            const int jc = jn - 1 + dj, kc = kn - 1 + dk, c = kc * ny + jc;
+            const double d = dsig_cell(cell2act, ds, c);
+            if (d == 0.0) continue;
+            const double dy = M.yLen[jc], dz = M.zLen[kc], area = dy * dz;
+            if (mode == 0) {
+                r += (d * area) * (mk(0.0, -omega) * (0.25 * Fs[node(jn, kn)]));
+            } else {
+                const double s = sig[c], pre = area * (-1.0 / (s * s)) * 0.5;
+                const cplx ghy = (Hf(jc + 1, kn) - Hf(jc, kn)) / dy;          // the cell's y-edge on node row kn
+                const cplx ghz = (Hf(jn, kc + 1) - Hf(jn, kc)) / dz;          // its z-edge on node column jn
+                const double sy = (jn == jc + 1) ? 1.0 : -1.0, sz = (kn == kc + 1) ? 1.0 : -1.0;
+                r += (d * pre) * (ghy * (-sy / dy) + ghz * (-sz / dz));
+            }
+        }
+    if (jn == 1 || jn == ny - 1 || kn == nz - 1) {
+        const StencilW w = stencil_at(M, sig, mode, jn, kn);
+        const cplx* b = dbc + (size_t)sys * M.nb;
+        if (jn == 1) r += w.wyL * b[ny + 1 + (kn - 1)];
+        if (jn == ny - 1) r += w.wyR * b[ny + 1 + nz + (kn - 1)];
+        if (kn == nz - 1) r += w.wzD * b[ny + 1 + 2 * nz + (jn - 1)];
+    }
+    rhs[(size_t)sys * M.N + q] = r;
+}
+
+// Tangent receiver functional: the forward mode of k_rx_adjoint's reverse recipe (its normalised sensitivity weights), from the
+// field tangent dF on node rows zid, zid+1 (interior: the tangent solve, boundary: dbc) and dsig on cell row zid, into the full
+// data layout jv (rho / phase plans: the real pair (d rho_a, d phase)).  One CTA per system; the receivers are independent.
+template <bool kRhoPhase, bool kTipper>
+__global__ void __launch_bounds__(kRxThreads)
+k_rx_tangent(MeshDev M, RxDev rx, SysMap sm, CompMap cm, const double* __restrict__ freqs, const double* __restrict__ sigma,
+             const int* __restrict__ cell2act, const double* __restrict__ dsig, int nAC, const cplx* __restrict__ F,
+             const cplx* __restrict__ dF, cplx* __restrict__ jv) {
+    extern __shared__ __align__(16) unsigned char smraw[];
+    const int ny = M.ny;
+    cplx* F0 = reinterpret_cast<cplx*>(smraw);        // ny+1
+    cplx* F1 = F0 + (ny + 1);
+    cplx* G0 = F1 + (ny + 1);
+    cplx* dF0 = G0 + (ny + 1);
+    cplx* dF1 = dF0 + (ny + 1);
+    cplx* dG0 = dF1 + (ny + 1);
+    cplx* Qc = dG0 + (ny + 1);                         // ny
+    cplx* dQc = Qc + ny;                               // ny
+    const int sys = blockIdx.x;
+    int ch, mi, mode, f;
+    sys_decode(sm, sys, ch, mi, mode, f);
+    const int tid = threadIdx.x;
+    const double omega = 2.0 * kPi * freqs[f];
+    const double h = M.zLen[M.zid];
+    const double* sig1 = sigma + (size_t)ch * M.nCell + (size_t)M.zid * ny;
+    const double* ds = dsig + (size_t)ch * nAC;
+    const int* c2a = cell2act + (size_t)M.zid * ny;
+    const cplx* Fs = F + (size_t)sys * M.nNode;
+    const cplx* dFs = dF + (size_t)sys * M.nNode;
+    const cplx iw = mk(0.0, omega), iwmu = mk(0.0, omega * kMu0);
+    for (int j = tid; j <= ny; j += kRxThreads) {
+        F0[j] = Fs[(size_t)M.zid * (ny + 1) + j];
+        F1[j] = Fs[(size_t)(M.zid + 1) * (ny + 1) + j];
+        dF0[j] = dFs[(size_t)M.zid * (ny + 1) + j];
+        dF1[j] = dFs[(size_t)(M.zid + 1) * (ny + 1) + j];
+    }
+    __syncthreads();
+    for (int j = tid; j < ny; j += kRxThreads) {
+        if (mode == 0) {
+            Qc[j] = (0.75 * ((F0[j + 1] - F0[j]) / M.yLen[j] / iw) + 0.25 * ((F1[j + 1] - F1[j]) / M.yLen[j] / iw)) / kMu0;
+            dQc[j] = (0.75 * ((dF0[j + 1] - dF0[j]) / M.yLen[j] / iw) + 0.25 * ((dF1[j + 1] - dF1[j]) / M.yLen[j] / iw)) / kMu0;
+        } else {
+            const cplx jzq = 0.75 * (-((F0[j + 1] - F0[j]) / M.yLen[j])) + 0.25 * (-((F1[j + 1] - F1[j]) / M.yLen[j]));
+            const cplx djzq = 0.75 * (-((dF0[j + 1] - dF0[j]) / M.yLen[j])) + 0.25 * (-((dF1[j + 1] - dF1[j]) / M.yLen[j]));
+            Qc[j] = jzq / sig1[j];
+            dQc[j] = djzq / sig1[j] - jzq * (dsig_cell(c2a, ds, j) / (sig1[j] * sig1[j]));
+        }
+    }
+    __syncthreads();
+    for (int i = tid + 1; i < ny; i += kRxThreads) {
+        const double yb = 0.5 * M.yLen[i - 1] + 0.5 * M.yLen[i];
+        const double d0 = dsig_cell(c2a, ds, i - 1), d1 = dsig_cell(c2a, ds, i);
+        const cplx Q = 0.75 * F0[i] + 0.25 * F1[i], dQ = 0.75 * dF0[i] + 0.25 * dF1[i];
+        const cplx dEz = (Qc[i] - Qc[i - 1]) / yb, ddEz = (dQc[i] - dQc[i - 1]) / yb;
+        if (mode == 0) {
+            const double sv = (0.5 * (sig1[i - 1] * M.yLen[i - 1]) + 0.5 * (sig1[i] * M.yLen[i])) / yb;
+            const double dsv = (0.5 * (d0 * M.yLen[i - 1]) + 0.5 * (d1 * M.yLen[i])) / yb;
+            G0[i] = -((F1[i] - F0[i]) / h / iwmu) - (dEz - sv * Q) * (0.5 * h);
+            dG0[i] = -((dF1[i] - dF0[i]) / h / iwmu) - (ddEz - sv * dQ - dsv * Q) * (0.5 * h);
+        } else {
+            const double rv = (0.5 * ((1.0 / sig1[i - 1]) * M.yLen[i - 1]) + 0.5 * ((1.0 / sig1[i]) * M.yLen[i])) / yb;
+            const double drv = (0.5 * ((-d0 / (sig1[i - 1] * sig1[i - 1])) * M.yLen[i - 1]) + 0.5 * ((-d1 / (sig1[i] * sig1[i])) * M.yLen[i])) / yb;
+            const cplx JyH = (F1[i] - F0[i]) / h, dJyH = (dF1[i] - dF0[i]) / h;
+            G0[i] = JyH * rv - (dEz + iwmu * Q) * (0.5 * h);
+            dG0[i] = dJyH * rv + JyH * drv - (ddEz + iwmu * dQ) * (0.5 * h);
+        }
+    }
+    __syncthreads();
+    if (tid == 0) { G0[0] = G0[1]; G0[ny] = G0[ny - 1]; dG0[0] = dG0[1]; dG0[ny] = dG0[ny - 1]; }
+    __syncthreads();
+    const int nC = kTipper ? cm.nComp : sm.nModes;
+    const int zc = kTipper ? (mi == 0 ? cm.zc[0] : cm.zc[1]) : mi;
+    const size_t row0 = ((size_t)ch * sm.nFreq + f) * rx.nRx;
+    for (int r = tid; r < rx.nRx; r += kRxThreads) {
+        const int iL = rx.iL[r], iR = rx.iR[r];
+        const double wl = rx.wL[r], wr = rx.wR[r];
+        if (!(kTipper && zc < 0)) {
+            cplx numS, denS, dnum, dden;
+            if (mode == 0) {
+                numS = wl * F0[iL] + wr * F0[iR]; denS = wl * G0[iL] + wr * G0[iR];
+                dnum = wl * dF0[iL] + wr * dF0[iR]; dden = wl * dG0[iL] + wr * dG0[iR];
+            } else {
+                numS = wl * G0[iL] + wr * G0[iR]; denS = wl * F0[iL] + wr * F0[iR];
+                dnum = wl * dG0[iL] + wr * dG0[iR]; dden = wl * dF0[iL] + wr * dF0[iR];
+            }
+            const cplx dZ = dnum / denS - numS * dden / (denS * denS);
+            const size_t di = (row0 + r) * nC + zc;
+            if constexpr (kRhoPhase) {
+                const int id = rx.fid[r];           // the forward (un-normalised) Z, as the adjoint weight V uses it
+                const double d1 = rx.fdy1[r], d2 = rx.fdy2[r];
+                const cplx Z = (mode == 0) ? (F0[id - 1] * d2 + F0[id] * d1) / (G0[id - 1] * d2 + G0[id] * d1)
+                                           : (G0[id - 1] * d2 + G0[id] * d1) / (F0[id - 1] * d2 + F0[id] * d1);
+                const cplx zd = cconj(Z) * dZ;
+                jv[di] = mk(2.0 / (omega * kMu0) * zd.x, 180.0 / kPi * zd.y / cabs2(Z));
+            } else {
+                jv[di] = dZ;
+            }
+        }
+        if constexpr (kTipper) {
+            if (mi == cm.tmi) {
+                const int jL = rx.tjL[r], jR = rx.tjR[r];
+                const double vl = rx.twL[r], vr = rx.twR[r];
+                const cplx hzr = vl * ((F0[jL + 1] - F0[jL]) / M.yLen[jL] / iwmu) + vr * ((F0[jR + 1] - F0[jR]) / M.yLen[jR] / iwmu);
+                const cplx dhzr = vl * ((dF0[jL + 1] - dF0[jL]) / M.yLen[jL] / iwmu) + vr * ((dF0[jR + 1] - dF0[jR]) / M.yLen[jR] / iwmu);
+                const cplx hyr = wl * G0[iL] + wr * G0[iR], dhyr = wl * dG0[iL] + wr * dG0[iR];
+                jv[(row0 + r) * nC + cm.tc] = (dhzr - (hzr / hyr) * dhyr) / hyr;
+            }
+        }
+    }
+}
+
+// Gauss-Newton data weights on a tangent in the full layout: vin = Wd^2 jv (rho / phase plans: (w_rho^2 d rho, w_phi^2 d phi)).
+// grid (ceil(nFull/256), nChains)
+__global__ void k_gn_weight(int nFull, int rhoPhase, const double* __restrict__ wd, const double* __restrict__ wdPha,
+                            const cplx* __restrict__ jv, cplx* __restrict__ vin) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x, ch = blockIdx.y;
+    if (i >= nFull) return;
+    const cplx t = jv[(size_t)ch * nFull + i];
+    const double w = wd[i], wp = rhoPhase ? wdPha[i] : w;
+    vin[(size_t)ch * nFull + i] = mk(w * w * t.x, (rhoPhase ? wp * wp : w * w) * t.y);
+}
+// dsig = sigma_active * v: the ln(sigma) direction v as a conductivity perturbation.  grid (ceil(nAC/256), nChains)
+__global__ void k_sigma_scale(int nAC, int nCell, const int* __restrict__ act2cell, const double* __restrict__ sigma,
+                              const double* __restrict__ v, double* __restrict__ dsig) {
+    const int a = blockIdx.x * blockDim.x + threadIdx.x, ch = blockIdx.y;
+    if (a < nAC) dsig[(size_t)ch * nAC + a] = sigma[(size_t)ch * nCell + act2cell[a]] * v[(size_t)ch * nAC + a];
+}
+
+// ---------------------------------------------------------------------------------------------
 // Reduction over systems + chain rule + prior gradient (HMCSampler.jl:306, :223-224, :255-256):
 //   grad[a] = sigma_a * sum_sys Gpart[sys][cell(a)] + beta * (Wm (m - mref))[a]     (fixed summation order)
 // grid: (ceil(nAC/256), nChains)

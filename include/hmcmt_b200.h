@@ -160,6 +160,20 @@ int hmcmt_jtvec(hmcmt_plan* plan, const double* v, double* gsig);
  * part fills that receiver's row in every (frequency, mode) system at once: 2 nRx passes instead of nData. */
 int hmcmt_jacobian(hmcmt_plan* plan, double* J);
 
+/* J·dsig for the state of the last forward evaluation (forward-mode directional derivative, no explicit Jacobian).
+ *   dsig [nChains][nAC]: conductivity perturbation of the active cells.
+ *   jv   [nChains][nData] in the packed order: complex, or real (d rho_a, d phase rows) for Rho_Pha plans.
+ * The result is hmcmt_jacobian's J times dsig: the exact transpose of the adjoint hmcmt_jtvec runs, with the same boundary-
+ * condition approximations.  One tangent boundary recursion, one solve per system with the resident factors and the tangent
+ * receiver functional; runs on the plan's stream and leaves the fields, factors, predictions, misfit and chain state as they
+ * were.  -3 without a prior forward evaluation or on NULL arguments. */
+int hmcmt_jvec(hmcmt_plan* plan, const double* dsig, double* jv);
+/* Gauss-Newton Hessian of the data misfit in the sampler's coordinates m = ln sigma:
+ *   hv = D Re(J^H Wd^2 J) D v,  D = diag(sigma_active);  Wd = 1/|err| per row (wd / wdPha for rho / phase rows).
+ * with_prior != 0 adds beta Wm v.  v, hv: [nChains][nAC].  One hmcmt_jvec and one hmcmt_jtvec pass; the plan's gradient of the
+ * last evaluation is kept.  -3 without a prior forward evaluation or on NULL arguments. */
+int hmcmt_gn_hessvec(hmcmt_plan* plan, const double* v, int32_t with_prior, double* hv);
+
 /* compDataGradient(mtMesh,mtData,invParam,hmcprior)  HMCSampler.jl:277-330:
  * m -> pred [nChains][nData] complex, phi_d [nChains], grad [nChains][nAC] (w.r.t. log conductivity,
  * data part only, as the reference returns it). Host buffers; H2D/D2H inside. */

@@ -270,6 +270,24 @@ class Plan:
         _lib.check(self.L.hmcmt_gn_hessvec(self.h, _lib.f64(vv), 1 if total else 0, _lib.f64(hv)), "hmcmt_gn_hessvec")
         return hv
 
+    def gauss_newton(self, m0=None, mref=None, max_iter=10, max_cg=10, cg_tol=1e-2, max_ls=8, max_step=3.0, tol_rel=1e-4):
+        """Posterior mode of every chain by projected Gauss-Newton-CG (hmcmt_gauss_newton): minimises phi_d(m) + 1/2 beta
+        (m - m_ref)^T Wm (m - m_ref) within the plan's bounds, every CG product from the resident factors.  m0: start model
+        (default: the plan's current model); mref: sets the reference model first (set_state).  Returns (m [nChains, nAC],
+        history [nChains, max_iter + 1, 6] = (phi_d, phi_m, |P g|, CG iterations, alpha, line-search trials) per accepted step,
+        info [nChains, 2] = (accepted steps, stop reason: 0 max_iter, 1 tolerance, 2 line search failed)).  The plan is left
+        evaluated at m: forward_gradient(m, total=True) would reproduce its state, and jvec / gn_hessvec / jacobian work there."""
+        if mref is not None:
+            self.set_state(mref=mref)
+        self.generation = getattr(self, "generation", 0) + 1
+        m = np.zeros((self.nChains, self.nAC))
+        hist = np.zeros((self.nChains, max(int(max_iter), 0) + 1, 6))
+        info = np.zeros((self.nChains, 2), dtype=np.int32)
+        mm = None if m0 is None else self._m(m0)
+        _lib.check(self.L.hmcmt_gauss_newton(self.h, None if mm is None else _lib.f64(mm), int(max_iter), int(max_cg), float(cg_tol), int(max_ls), float(max_step),
+                                             float(tol_rel), _lib.f64(m), _lib.f64(hist), _lib.i32(info)), "hmcmt_gauss_newton")
+        return m, hist, info
+
     def forward_gradient(self, m, total=False):
         """compDataGradient (HMCSampler.jl:277-330): predicted data, data misfit, gradient w.r.t. ln(sigma).  total=True adds the
         model-norm part beta Wm (m - m_ref) on the device (m_ref from set_state), as proposeLeapfrog does right afterwards."""

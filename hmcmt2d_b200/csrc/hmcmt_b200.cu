@@ -87,6 +87,11 @@ struct hmcmt_plan {
     // gtotal] (gnBuf, 5 [nChains][nAC]: k_reduce_grad writes there, so the plan's own gradient stays)
     DevBuf<cplx> dbc, jvFull;
     DevBuf<double> dsigA, gnBuf;
+    // projected Gauss-Newton-CG (hmcmt_gauss_newton), allocated on first use: gnVec 6 [nChains][nAC] = [m_k | g_k | delta | r | p |
+    // q], the active set gnAct [nChains][nAC], the p^T q block partials gnPart, the per-chain scalars / flags gnS / gnI (GnScalar /
+    // GnFlag of mt_kernels.cuh) and gnE, k_energies' output for the trial points
+    DevBuf<double> gnVec, gnPart, gnS, gnE;
+    DevBuf<int> gnAct, gnI;
     DevBuf<BandSys> sysDesc;
     DevBuf<SolveJob> jobs, fwdJobs;                 // fwdJobs: back-substitution sweeps of the fused forward systems (split systems)
     // wide meshes (half-bandwidth > 104): nested-dissection multifrontal solver (mf_solver.cuh) instead of the band kernels
@@ -1203,7 +1208,7 @@ void hmcmt_destroy(hmcmt_plan* pl) {
     pl->driftFlag.release(); pl->packed2full.release(); pl->full2packed.release(); pl->Lsteps.release(); pl->obs.release(); pl->bc.release(); pl->bcs.release();
     pl->rhs.release(); pl->x.release(); pl->F.release(); pl->lam.release(); pl->Lam.release(); pl->srows.release(); pl->qrow.release();
     pl->scratch.release(); pl->predFull.release(); pl->ainvz.release(); pl->zadj.release(); pl->vin.release();
-    pl->predPacked.release(); pl->conCols.release(); pl->dbc.release(); pl->jvFull.release(); pl->dsigA.release(); pl->gnBuf.release(); pl->xbuf.release(); pl->wexp.release(); pl->respFull.release(); pl->gradK.release(); pl->Lband.release(); pl->massBuf.release(); pl->massStatus.release(); delete pl->massSolver; pl->massSolver = nullptr; pl->mfSys.release(); delete pl->mfs; pl->mfs = nullptr; pl->fwdJobs.release(); pl->sysDesc.release(); pl->jobs.release();
+    pl->predPacked.release(); pl->conCols.release(); pl->dbc.release(); pl->jvFull.release(); pl->dsigA.release(); pl->gnBuf.release(); pl->gnVec.release(); pl->gnPart.release(); pl->gnS.release(); pl->gnE.release(); pl->gnAct.release(); pl->gnI.release(); pl->xbuf.release(); pl->wexp.release(); pl->respFull.release(); pl->gradK.release(); pl->Lband.release(); pl->massBuf.release(); pl->massStatus.release(); delete pl->massSolver; pl->massSolver = nullptr; pl->mfSys.release(); delete pl->mfs; pl->mfs = nullptr; pl->fwdJobs.release(); pl->sysDesc.release(); pl->jobs.release();
     if (pl->pin) cudaFreeHost(pl->pin);
     delete pl;
 }
@@ -1583,6 +1588,25 @@ int hmcmt_jvec(hmcmt_plan* pl, const double* dsig, double* jv) {
     return check_status(pl);
 }
 
+// The Gauss-Newton product D Re(J^H Wd^2 J) D v for the resident state, v [nChains][nAC] in device memory, up to the per-system
+// partials in Gpart: the caller reduces them over the systems (k_reduce_grad for hmcmt_gn_hessvec, k_reduce_gn for the CG of
+// hmcmt_gauss_newton).  Needs ensure_tangent.
+static int gn_partials(hmcmt_plan* pl, const double* v) {
+    const MeshDev& M = pl->M;
+    cudaStream_t st = pl->stream;
+    k_sigma_scale<<<dim3((pl->nAC + 255) / 256, pl->nChains), 256, 0, st>>>(pl->nAC, M.nCell, pl->act2cell.p, pl->sigma.p, v, pl->dsigA.p);
+    LAUNCH_CHECK(pl);
+    int rc;
+    if ((rc = jvec_device(pl))) return rc;
+    k_gn_weight<<<dim3((pl->nFull + 255) / 256, pl->nChains), 256, 0, st>>>(pl->nFull, pl->dataKind, pl->wd.p, pl->wdPha.p, pl->jvFull.p,
+                                                                            pl->vin.p);
+    LAUNCH_CHECK(pl);
+    // J^T of the weighted tangent through the adjoint machinery (the receiver functional recomputes the same predictions and
+    // misfit from the unchanged fields)
+    if ((rc = rx_phase(pl, true, pl->vin.p))) return rc;
+    return adjoint_phase(pl, false);
+}
+
 int hmcmt_gn_hessvec(hmcmt_plan* pl, const double* v, int32_t with_prior, double* hv) {
     if (!pl || !v || !hv || !pl->haveForward) return kErrArg;
     HMCMT_CUDA_TRY(cudaSetDevice(pl->device));
@@ -1597,18 +1621,11 @@ int hmcmt_gn_hessvec(hmcmt_plan* pl, const double* v, int32_t with_prior, double
     }
     double *vD = pl->gnBuf.p, *zero = vD + nA, *gs = zero + nA, *gd = gs + nA, *gt = gd + nA;
     HMCMT_CUDA_TRY(cudaMemcpyAsync(vD, v, sizeof(double) * nA, cudaMemcpyHostToDevice, st));
-    const dim3 gA((pl->nAC + 255) / 256, pl->nChains);
-    k_sigma_scale<<<gA, 256, 0, st>>>(pl->nAC, M.nCell, pl->act2cell.p, pl->sigma.p, vD, pl->dsigA.p);
-    LAUNCH_CHECK(pl);
-    if ((rc = jvec_device(pl))) return rc;
-    k_gn_weight<<<dim3((pl->nFull + 255) / 256, pl->nChains), 256, 0, st>>>(pl->nFull, pl->dataKind, pl->wd.p, pl->wdPha.p, pl->jvFull.p,
-                                                                            pl->vin.p);
-    LAUNCH_CHECK(pl);
-    // J^T of the weighted tangent through the adjoint machinery (the receiver functional recomputes the same predictions and
-    // misfit from the unchanged fields), then the chain rule and prior term of the gradient's reduction with (m, m_ref) = (v, 0)
-    if ((rc = rx_phase(pl, true, pl->vin.p)) || (rc = adjoint_phase(pl, false))) return rc;
-    k_reduce_grad<<<gA, 256, 0, st>>>(pl->nAC, M.nCell, pl->nSysPerChain, pl->act2cell.p, pl->Gpart.p, vD, zero, pl->wmPtr.p, pl->wmIdx.p,
-                                      pl->wmVal.p, pl->beta, pl->sigma.p, gs, gd, gt);
+    if ((rc = gn_partials(pl, vD))) return rc;
+    // the chain rule and prior term of the gradient's reduction with (m, m_ref) = (v, 0)
+    k_reduce_grad<<<dim3((pl->nAC + 255) / 256, pl->nChains), 256, 0, st>>>(pl->nAC, M.nCell, pl->nSysPerChain, pl->act2cell.p, pl->Gpart.p,
+                                                                            vD, zero, pl->wmPtr.p, pl->wmIdx.p, pl->wmVal.p, pl->beta,
+                                                                            pl->sigma.p, gs, gd, gt);
     LAUNCH_CHECK(pl);
     HMCMT_CUDA_TRY(cudaMemcpyAsync(hv, with_prior ? gt : gd, sizeof(double) * nA, cudaMemcpyDeviceToHost, st));
     HMCMT_CUDA_TRY(cudaStreamSynchronize(st));
@@ -1682,6 +1699,133 @@ int hmcmt_get_state(hmcmt_plan* pl, double* m, double* p) {
     if (p) HMCMT_CUDA_TRY(cudaMemcpyAsync(p, pl->p.p, bytes, cudaMemcpyDeviceToHost, pl->stream));
     HMCMT_CUDA_TRY(cudaStreamSynchronize(pl->stream));
     return kOk;
+}
+
+// the Gauss-Newton buffers, allocated on first use (and the tangent ones the CG's products need)
+static int ensure_gn(hmcmt_plan* pl) {
+    int rc = ensure_tangent(pl);
+    if (rc || pl->gnI.p) return rc;
+    const size_t nA = (size_t)pl->nChains * pl->nAC, nPart = (size_t)pl->nChains * ((pl->nAC + kGnReduceThreads - 1) / kGnReduceThreads);
+    if ((rc = pl->gnVec.alloc(6 * nA)) || (rc = pl->gnAct.alloc(nA)) || (rc = pl->gnPart.alloc(nPart)) ||
+        (rc = pl->gnS.alloc((size_t)pl->nChains * kGnS)) || (rc = pl->gnE.alloc(2 * (size_t)pl->nChains)))
+        return rc;
+    return pl->gnI.alloc((size_t)pl->nChains * kGnI);
+}
+
+// the per-chain flags into the pinned staging buffer, the device error flags, one synchronisation
+static int gn_read_flags(hmcmt_plan* pl) {
+    HMCMT_CUDA_TRY(cudaMemcpyAsync(pl->pin, pl->gnI.p, sizeof(int) * pl->gnI.n, cudaMemcpyDeviceToHost, pl->stream));
+    return check_status(pl);
+}
+
+// Projected Gauss-Newton-CG, every chain on its own (include/hmcmt_b200.h, DESIGN.md 4.8).  The host drives the outer iteration
+// and the line search; every per-chain decision is taken on the device, from values that do not depend on the other chains.
+int hmcmt_gauss_newton(hmcmt_plan* pl, const double* m0, int32_t maxIter, int32_t maxCG, double cgTol, int32_t maxLS, double maxStep,
+                       double tolRel, double* m_out, double* history, int32_t* info) {
+    if (!pl || !m_out || !history || !info || maxIter < 0 || maxCG < 1 || maxLS < 1 || !(maxStep > 0.0) || !(cgTol >= 0.0) ||
+        !std::isfinite(cgTol) || !(tolRel >= 0.0) || !std::isfinite(tolRel))
+        return kErrArg;
+    HMCMT_CUDA_TRY(cudaSetDevice(pl->device));
+    int rc = ensure_gn(pl);
+    if (rc) return rc;
+    cudaStream_t st = pl->stream;
+    const int nCh = pl->nChains, nAC = pl->nAC;
+    const size_t nA = (size_t)nCh * nAC, nHist = (size_t)nCh * (maxIter + 1) * kGnHist;
+    const size_t bytes = std::max(sizeof(double) * (nA + nHist) + sizeof(int) * pl->gnI.n, (size_t)1 << 20);
+    if ((rc = ensure_pin(pl, bytes))) return rc;
+    DevBuf<double> hist;
+    if ((rc = hist.alloc(nHist))) return rc;
+    double *mk = pl->gnVec.p, *gk = mk + nA, *delta = gk + nA, *r = delta + nA, *p = r + nA, *q = p + nA;
+    const int nPart = (nAC + kGnReduceThreads - 1) / kGnReduceThreads;
+    const int* flags = reinterpret_cast<const int*>(pl->pin);
+    auto any = [&](int slot, int value) {
+        for (int ch = 0; ch < nCh; ++ch)
+            if (flags[(size_t)ch * kGnI + slot] == value) return true;
+        return false;
+    };
+    // evaluation of the current model, then phi_m of it (k_energies' prior reduction; its kinetic half is not used)
+    auto evaluate = [&]() -> int {
+        int e = compute_step(pl, true, nullptr);
+        if (e) return e;
+        k_energies<<<nCh, kHmcThreads, 0, st>>>(nAC, pl->m.p, pl->mref.p, pl->p.p, pl->wmPtr.p, pl->wmIdx.p, pl->wmVal.p, pl->beta,
+                                                pl->gnE.p, nullptr);
+        LAUNCH_CHECK(pl);
+        return kOk;
+    };
+    auto linearise = [&](int first) -> int {
+        k_gn_linearise<<<nCh, kHmcThreads, 0, st>>>(nAC, first, maxIter, tolRel, pl->lo, pl->hi, pl->m.p, pl->gtotal.p, pl->phi.p,
+                                                    pl->gnE.p, mk, gk, pl->gnAct.p, r, p, delta, pl->gnS.p, pl->gnI.p, hist.p);
+        LAUNCH_CHECK(pl);
+        return kOk;
+    };
+    auto run = [&]() -> int {
+        int e;
+        pl->sigmaDirect = false;
+        if (m0) {
+            std::memcpy(pl->pin, m0, sizeof(double) * nA);
+            HMCMT_CUDA_TRY(cudaMemcpyAsync(pl->m.p, pl->pin, sizeof(double) * nA, cudaMemcpyHostToDevice, st));
+        }
+        HMCMT_CUDA_TRY(cudaMemsetAsync(hist.p, 0, sizeof(double) * nHist, st));
+        HMCMT_CUDA_TRY(cudaMemsetAsync(pl->gnI.p, 0, sizeof(int) * pl->gnI.n, st));
+        k_gn_project<<<dim3((nAC + 255) / 256, nCh), 256, 0, st>>>(nAC, pl->lo, pl->hi, pl->m.p);
+        LAUNCH_CHECK(pl);
+        if ((e = evaluate()) || (e = linearise(1)) || (e = gn_read_flags(pl))) return e;
+        for (int it = 0; it < maxIter && any(kGnActive, 1); ++it) {
+            // CG on P H P delta = -P g: maxCG products of all chains, no host round trip (a chain whose CG stopped is masked)
+            for (int j = 0; j < maxCG; ++j) {
+                if ((e = gn_partials(pl, p))) return e;
+                k_reduce_gn<<<dim3(nPart, nCh), kGnReduceThreads, 0, st>>>(nAC, pl->M.nCell, pl->nSysPerChain, pl->act2cell.p, pl->Gpart.p,
+                                                                           p, pl->wmPtr.p, pl->wmIdx.p, pl->wmVal.p, pl->beta, pl->sigma.p,
+                                                                           pl->gnAct.p, q, pl->gnPart.p);
+                LAUNCH_CHECK(pl);
+                k_gn_cg_update<<<nCh, kHmcThreads, 0, st>>>(nAC, nPart, cgTol, pl->gnPart.p, q, r, p, delta, pl->gnS.p, pl->gnI.p);
+                LAUNCH_CHECK(pl);
+            }
+            k_gn_direction<<<nCh, kHmcThreads, 0, st>>>(nAC, maxStep, delta, pl->gnI.p);
+            LAUNCH_CHECK(pl);
+            // Armijo backtracking on the projected path: one evaluation of all chains per trial; a chain that accepted keeps its
+            // model, so its evaluation (deterministic) stays that of its accepted trial
+            for (int t = 0; t < maxLS; ++t) {
+                k_gn_trial<<<nCh, kHmcThreads, 0, st>>>(nAC, t, pl->lo, pl->hi, mk, gk, delta, pl->m.p, pl->gnS.p, pl->gnI.p);
+                LAUNCH_CHECK(pl);
+                if ((e = evaluate())) return e;
+                k_gn_armijo<<<(nCh + 127) / 128, 128, 0, st>>>(nCh, t, maxLS, pl->phi.p, pl->gnE.p, pl->gnS.p, pl->gnI.p);
+                LAUNCH_CHECK(pl);
+                if ((e = gn_read_flags(pl))) return e;
+                if (!any(kGnLs, kLsSearch)) break;
+            }
+            if (any(kGnLs, kLsFailed)) {
+                // the chains whose search failed keep m_k; one more evaluation makes the resident state that of the models kept
+                k_gn_revert<<<nCh, kHmcThreads, 0, st>>>(nAC, mk, pl->m.p, pl->gnI.p);
+                LAUNCH_CHECK(pl);
+                if ((e = compute_step(pl, true, nullptr))) return e;
+            }
+            if ((e = linearise(0)) || (e = gn_read_flags(pl))) return e;
+        }
+        return kOk;
+    };
+    rc = run();
+    if (rc == kOk) {
+        unsigned char* pin = reinterpret_cast<unsigned char*>(pl->pin);
+        const size_t oH = sizeof(double) * nA, oI = oH + sizeof(double) * nHist;
+        if (cudaMemcpyAsync(pin, pl->m.p, oH, cudaMemcpyDeviceToHost, st) != cudaSuccess ||
+            cudaMemcpyAsync(pin + oH, hist.p, sizeof(double) * nHist, cudaMemcpyDeviceToHost, st) != cudaSuccess ||
+            cudaMemcpyAsync(pin + oI, pl->gnI.p, sizeof(int) * pl->gnI.n, cudaMemcpyDeviceToHost, st) != cudaSuccess ||
+            cudaStreamSynchronize(st) != cudaSuccess)
+            rc = kErrCuda;
+        if (rc == kOk) {
+            std::memcpy(m_out, pin, oH);
+            std::memcpy(history, pin + oH, sizeof(double) * nHist);
+            const int* f = reinterpret_cast<const int*>(pin + oI);
+            for (int ch = 0; ch < nCh; ++ch) {
+                info[2 * ch] = f[(size_t)ch * kGnI + kGnAcc];
+                info[2 * ch + 1] = f[(size_t)ch * kGnI + kGnReason];
+            }
+        }
+    }
+    cudaStreamSynchronize(st);
+    hist.release();
+    return rc;
 }
 
 static int trajectory_device(hmcmt_plan* pl, double dt, int Lmax, const int* dL) {

@@ -1339,4 +1339,222 @@ k_energies(int nAC, const double* __restrict__ m, const double* __restrict__ mre
     if (threadIdx.x == 0) { out[ch * 2] = 0.5 * k; out[ch * 2 + 1] = 0.5 * pm * beta; }
 }
 
+// ---------------------------------------------------------------------------------------------
+// Projected Gauss-Newton-CG (hmcmt_gauss_newton).  Every chain runs its own iteration; the per-chain scalars and flags live on
+// the device (S [nChains][kGnS], I [nChains][kGnI]) so that the CG loop needs no host round trip.  Every reduction is either one
+// CTA per chain (block_reduce over a fixed blockDim) or fixed-size block partials folded by one CTA in block order: the results
+// do not depend on timing, on the other chains or on how the launches were issued.
+enum GnScalar { kGnU, kGnPhid, kGnPhim, kGnRR, kGnRR0, kGnGtd, kGnAlpha, kGnS };
+enum GnFlag { kGnActive, kGnReason, kGnAcc, kGnCgRun, kGnCgIt, kGnLs, kGnTrials, kGnI };
+enum GnLs { kLsSearch, kLsAccepted, kLsFailed, kLsIdle };
+constexpr int kGnHist = 6;            // history row: phi_d, phi_m, |P g|, CG iterations, alpha, line-search trials
+constexpr int kGnReduceThreads = 256;
+
+// m <- clip(m, lo, hi).  grid (ceil(nAC/256), nChains)
+__global__ void k_gn_project(int nAC, double lo, double hi, double* __restrict__ m) {
+    const int a = blockIdx.x * blockDim.x + threadIdx.x, ch = blockIdx.y;
+    if (a < nAC) m[(size_t)ch * nAC + a] = fmin(fmax(m[(size_t)ch * nAC + a], lo), hi);
+}
+
+// New linearisation point of every chain that accepted a step (first: of every chain, iteration 0): U = phi_d + phi_m, the
+// active set A = {m <= lo, g > 0} u {m >= hi, g < 0}, r = p = -P g, delta = 0, the history row and the stopping tests
+// (decrease below tolRel U_k, or P g = 0).  en: k_energies output ([ch][1] = phi_m).  grid nChains, block kHmcThreads
+__global__ void __launch_bounds__(kHmcThreads)
+k_gn_linearise(int nAC, int first, int maxIter, double tolRel, double lo, double hi, const double* __restrict__ m,
+               const double* __restrict__ g, const double* __restrict__ phi, const double* __restrict__ en, double* __restrict__ mk,
+               double* __restrict__ gk, int* __restrict__ act, double* __restrict__ r, double* __restrict__ p, double* __restrict__ delta,
+               double* __restrict__ S, int* __restrict__ I, double* __restrict__ hist) {
+    __shared__ double sh[32];
+    const int ch = blockIdx.x;
+    double* s = S + (size_t)ch * kGnS;
+    int* f = I + (size_t)ch * kGnI;
+    if (!first && !(f[kGnActive] && f[kGnLs] == kLsAccepted)) return;
+    const size_t o = (size_t)ch * nAC;
+    double rr = 0.0;
+    for (int a = threadIdx.x; a < nAC; a += blockDim.x) {
+        const double mi = m[o + a], gi = g[o + a];
+        const int A = (mi <= lo && gi > 0.0) || (mi >= hi && gi < 0.0);
+        const double ri = A ? 0.0 : -gi;
+        mk[o + a] = mi;
+        gk[o + a] = gi;
+        act[o + a] = A;
+        r[o + a] = ri;
+        p[o + a] = ri;
+        delta[o + a] = 0.0;
+        rr += ri * ri;
+    }
+    rr = block_reduce(rr, false, sh);
+    if (threadIdx.x == 0) {
+        const double phid = phi[ch], phim = en[2 * ch + 1], U = phid + phim;
+        const int acc = first ? 0 : f[kGnAcc] + 1;
+        bool stop = rr == 0.0;
+        if (!first && s[kGnU] - U <= tolRel * s[kGnU]) stop = true;
+        double* h = hist + ((size_t)ch * (maxIter + 1) + acc) * kGnHist;
+        h[0] = phid;
+        h[1] = phim;
+        h[2] = sqrt(rr);
+        h[3] = first ? 0.0 : (double)f[kGnCgIt];
+        h[4] = first ? 0.0 : s[kGnAlpha];
+        h[5] = first ? 0.0 : (double)f[kGnTrials];
+        s[kGnU] = U;
+        s[kGnPhid] = phid;
+        s[kGnPhim] = phim;
+        s[kGnRR] = rr;
+        s[kGnRR0] = rr;
+        f[kGnAcc] = acc;
+        f[kGnActive] = stop ? 0 : 1;
+        f[kGnReason] = stop ? 1 : 0;
+        f[kGnCgRun] = stop ? 0 : 1;
+        f[kGnCgIt] = 0;
+    }
+}
+
+// The reduction over systems of the Gauss-Newton product (k_reduce_grad with (m, m_ref) = (p, 0)), masked: q = P (H p), and the
+// per-block partials of p^T q.  grid (ceil(nAC/kGnReduceThreads), nChains), block kGnReduceThreads
+__global__ void __launch_bounds__(kGnReduceThreads)
+k_reduce_gn(int nAC, int nCell, int nSysPerChain, const int* __restrict__ act2cell, const double* __restrict__ Gpart,
+            const double* __restrict__ p, const int* __restrict__ wmPtr, const int* __restrict__ wmIdx, const double* __restrict__ wmVal,
+            double beta, const double* __restrict__ sigma, const int* __restrict__ act, double* __restrict__ q, double* __restrict__ part) {
+    __shared__ double sh[32];
+    const int a = blockIdx.x * blockDim.x + threadIdx.x, ch = blockIdx.y;
+    double pq = 0.0;
+    if (a < nAC) {
+        const int c = act2cell[a];
+        const double* G = Gpart + (size_t)ch * nSysPerChain * nCell;
+        double acc = 0.0;
+        for (int s = 0; s < nSysPerChain; ++s) acc += G[(size_t)s * nCell + c];
+        const double* pp = p + (size_t)ch * nAC;
+        double pr = 0.0;
+        for (int k = wmPtr[a]; k < wmPtr[a + 1]; ++k) pr += wmVal[k] * pp[wmIdx[k]];
+        const double gd = sigma[(size_t)ch * nCell + c] * acc;
+        const double qa = act[(size_t)ch * nAC + a] ? 0.0 : gd + beta * pr;
+        q[(size_t)ch * nAC + a] = qa;
+        pq = pp[a] * qa;
+    }
+    pq = block_reduce(pq, false, sh);
+    if (threadIdx.x == 0) part[(size_t)ch * gridDim.x + blockIdx.x] = pq;
+}
+
+// One CG update of every chain whose CG still runs: p^T q from the partials (in block order), alpha = r^T r / p^T q,
+// delta += alpha p, r -= alpha q, stop at |r| <= cgTol |r_0|, else p = r + (r_new^T r_new / r^T r) p.  p^T q <= 0 stops the
+// chain's CG (delta = r_0 if that happens at its first iteration).  grid nChains, block kHmcThreads
+__global__ void __launch_bounds__(kHmcThreads)
+k_gn_cg_update(int nAC, int nPart, double cgTol, const double* __restrict__ part, const double* __restrict__ q, double* __restrict__ r,
+               double* __restrict__ p, double* __restrict__ delta, double* __restrict__ S, int* __restrict__ I) {
+    __shared__ double sh[32];
+    const int ch = blockIdx.x;
+    double* s = S + (size_t)ch * kGnS;
+    int* f = I + (size_t)ch * kGnI;
+    if (!f[kGnCgRun]) return;
+    const size_t o = (size_t)ch * nAC;
+    const double rr = s[kGnRR], rr0 = s[kGnRR0];
+    const int it = f[kGnCgIt];
+    double pq = 0.0;
+    for (int b = threadIdx.x; b < nPart; b += blockDim.x) pq += part[(size_t)ch * nPart + b];
+    pq = block_reduce(pq, false, sh);
+    if (!(pq > 0.0)) {
+        if (it == 0)
+            for (int a = threadIdx.x; a < nAC; a += blockDim.x) delta[o + a] = r[o + a];
+        if (threadIdx.x == 0) f[kGnCgRun] = 0;
+        return;
+    }
+    const double alpha = rr / pq;
+    double rn = 0.0;
+    for (int a = threadIdx.x; a < nAC; a += blockDim.x) {
+        delta[o + a] += alpha * p[o + a];
+        const double ri = r[o + a] - alpha * q[o + a];
+        r[o + a] = ri;
+        rn += ri * ri;
+    }
+    rn = block_reduce(rn, false, sh);
+    const bool done = sqrt(rn) <= cgTol * sqrt(rr0);
+    if (!done) {
+        const double b = rn / rr;
+        for (int a = threadIdx.x; a < nAC; a += blockDim.x) p[o + a] = r[o + a] + b * p[o + a];
+    }
+    if (threadIdx.x == 0) {
+        s[kGnRR] = rn;
+        f[kGnCgIt] = it + 1;
+        if (done) f[kGnCgRun] = 0;
+    }
+}
+
+// Step length of every running chain: delta scaled so that max|delta_i| <= maxStep, the line search armed; stopped chains sit it
+// out.  grid nChains, block kHmcThreads
+__global__ void __launch_bounds__(kHmcThreads)
+k_gn_direction(int nAC, double maxStep, double* __restrict__ delta, int* __restrict__ I) {
+    __shared__ double sh[32];
+    const int ch = blockIdx.x;
+    int* f = I + (size_t)ch * kGnI;
+    if (!f[kGnActive]) {
+        if (threadIdx.x == 0) f[kGnLs] = kLsIdle;
+        return;
+    }
+    double* d = delta + (size_t)ch * nAC;
+    double mx = 0.0;
+    for (int a = threadIdx.x; a < nAC; a += blockDim.x) mx = fmax(mx, fabs(d[a]));
+    mx = block_reduce(mx, true, sh);
+    if (mx > maxStep)
+        for (int a = threadIdx.x; a < nAC; a += blockDim.x) d[a] = d[a] / mx * maxStep;
+    if (threadIdx.x == 0) {
+        f[kGnLs] = kLsSearch;
+        f[kGnTrials] = 0;
+    }
+}
+
+// Trial t of the line search of every chain still searching: m = clip(m_k + 2^-t delta, lo, hi) and g_k^T (m - m_k).
+// grid nChains, block kHmcThreads
+__global__ void __launch_bounds__(kHmcThreads)
+k_gn_trial(int nAC, int t, double lo, double hi, const double* __restrict__ mk, const double* __restrict__ gk,
+           const double* __restrict__ delta, double* __restrict__ m, double* __restrict__ S, const int* __restrict__ I) {
+    __shared__ double sh[32];
+    const int ch = blockIdx.x;
+    if (I[(size_t)ch * kGnI + kGnLs] != kLsSearch) return;
+    const size_t o = (size_t)ch * nAC;
+    const double al = ldexp(1.0, -t);
+    double gtd = 0.0;
+    for (int a = threadIdx.x; a < nAC; a += blockDim.x) {
+        const double v = fmin(fmax(mk[o + a] + al * delta[o + a], lo), hi);
+        m[o + a] = v;
+        gtd += gk[o + a] * (v - mk[o + a]);
+    }
+    gtd = block_reduce(gtd, false, sh);
+    if (threadIdx.x == 0) {
+        S[(size_t)ch * kGnS + kGnGtd] = gtd;
+        S[(size_t)ch * kGnS + kGnAlpha] = al;
+    }
+}
+
+// Armijo test of trial t: accept when U(m) <= U_k + 1e-4 g_k^T (m - m_k); the last trial (maxLS) fails the search.
+// grid ceil(nChains/128), block 128
+__global__ void k_gn_armijo(int nChains, int t, int maxLS, const double* __restrict__ phi, const double* __restrict__ en,
+                            const double* __restrict__ S, int* __restrict__ I) {
+    const int ch = blockIdx.x * blockDim.x + threadIdx.x;
+    if (ch >= nChains) return;
+    int* f = I + (size_t)ch * kGnI;
+    if (f[kGnLs] != kLsSearch) return;
+    const double* s = S + (size_t)ch * kGnS;
+    const double U = phi[ch] + en[2 * ch + 1];
+    if (U <= s[kGnU] + 1e-4 * s[kGnGtd]) {
+        f[kGnLs] = kLsAccepted;
+        f[kGnTrials] = t + 1;
+    } else if (t + 1 >= maxLS) {
+        f[kGnLs] = kLsFailed;
+        f[kGnTrials] = t + 1;
+    }
+}
+
+// A chain whose line search failed goes back to m_k and stops.  grid nChains, block kHmcThreads
+__global__ void __launch_bounds__(kHmcThreads)
+k_gn_revert(int nAC, const double* __restrict__ mk, double* __restrict__ m, int* __restrict__ I) {
+    const int ch = blockIdx.x;
+    int* f = I + (size_t)ch * kGnI;
+    if (f[kGnLs] != kLsFailed) return;
+    for (int a = threadIdx.x; a < nAC; a += blockDim.x) m[(size_t)ch * nAC + a] = mk[(size_t)ch * nAC + a];
+    if (threadIdx.x == 0) {
+        f[kGnActive] = 0;
+        f[kGnReason] = 2;
+    }
+}
+
 }  // namespace hmcmt

@@ -65,6 +65,8 @@ def load() -> C.CDLL:
     lib.hmcmt_jacobian.argtypes = [vp, _f64p]
     lib.hmcmt_jvec.argtypes = [vp, _f64p, _f64p]
     lib.hmcmt_gn_hessvec.argtypes = [vp, _f64p, C.c_int32, _f64p]
+    lib.hmcmt_gauss_newton.argtypes = [vp, _f64p, C.c_int32, C.c_int32, C.c_double, C.c_int32, C.c_double, C.c_double, _f64p,
+                                       _f64p, _i32p]
     lib.hmcmt_status.argtypes = [vp]
     lib.hmcmt_set_mass_matrix.argtypes = [vp, C.c_int32]
     lib.hmcmt_set_response_kind.argtypes = [vp, C.c_int32]
@@ -113,7 +115,7 @@ EXPORTED_SYMBOLS = [
     "factor_mumps_cmplx_", "factor_mumps_", "solve_mumps_cmplx_", "solve_mumps_", "solve_mumps_sparse_rhs_",
     "solve_mumps_cmplx_sparse_rhs_", "destroy_mumps_", "destroy_mumps_cmplx_",
     "hmcmt_plan_create", "hmcmt_plan_create_rho_phase", "hmcmt_destroy", "hmcmt_plan_info", "hmcmt_forward", "hmcmt_forward_sigma", "hmcmt_jtvec",
-    "hmcmt_forward_gradient", "hmcmt_forward_gradient_total", "hmcmt_jacobian", "hmcmt_jvec", "hmcmt_gn_hessvec", "hmcmt_status", "hmcmt_set_mass_matrix", "hmcmt_set_response_kind", "hmcmt_get_responses",
+    "hmcmt_forward_gradient", "hmcmt_forward_gradient_total", "hmcmt_jacobian", "hmcmt_jvec", "hmcmt_gn_hessvec", "hmcmt_gauss_newton", "hmcmt_status", "hmcmt_set_mass_matrix", "hmcmt_set_response_kind", "hmcmt_get_responses",
     "hmcmt_set_state", "hmcmt_get_state", "hmcmt_leapfrog_trajectory", "hmcmt_leapfrog_steps_device", "hmcmt_sync",
     "hmcmt_step_partial", "hmcmt_exchange_buffer", "hmcmt_step_finish", "hmcmt_nccl_unique_id", "hmcmt_nccl_init",
     "hmcmt_leapfrog_steps_sharded",

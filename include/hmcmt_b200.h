@@ -173,6 +173,28 @@ int hmcmt_jvec(hmcmt_plan* plan, const double* dsig, double* jv);
  * with_prior != 0 adds beta Wm v.  v, hv: [nChains][nAC].  One hmcmt_jvec and one hmcmt_jtvec pass; the plan's gradient of the
  * last evaluation is kept.  -3 without a prior forward evaluation or on NULL arguments. */
 int hmcmt_gn_hessvec(hmcmt_plan* plan, const double* v, int32_t with_prior, double* hv);
+/* Projected Gauss-Newton-CG for the posterior mode, every chain on its own: minimises
+ *   U(m) = phi_d(m) + 1/2 beta (m - m_ref)^T Wm (m - m_ref)   over  ln sigma_min <= m_i <= ln sigma_max
+ * (the sampler's potential energy, with the plan's m_ref of hmcmt_set_state and the plan's bounds).  Iteration k:
+ *   - evaluate U(m_k) and g_k (the plan's gradient evaluation, prior included);
+ *   - active set A = {m_i <= lo and g_i > 0} u {m_i >= hi and g_i < 0}, P the mask that zeroes A;
+ *   - CG from delta = 0 on P H P delta = -P g, H = D Re(J^H Wd^2 J) D + beta Wm (hmcmt_gn_hessvec with the prior): at most maxCG
+ *     iterations, stop at |r| <= cgTol |r_0|; p^T H p <= 0 stops the CG (delta = r_0 if that happens at its first iteration);
+ *   - delta scaled so that max |delta_i| <= maxStep;
+ *   - Armijo backtracking on m(alpha) = clip(m_k + alpha delta, lo, hi), alpha = 1, 1/2, ..., at most maxLS trials: accept when
+ *     U(m(alpha)) <= U(m_k) + 1e-4 g_k^T (m(alpha) - m_k);
+ *   - the chain stops when U_k - U_{k+1} <= tolRel U_k or P g = 0 (stop reason 1), or when its line search fails: it then keeps
+ *     m_k (stop reason 2).  maxIter outer iterations at most (stop reason 0).
+ * m0: [nChains][nAC] start model, or NULL for the plan's current model; it is projected onto the bounds first.
+ * m_out: [nChains][nAC].  history: [nChains][maxIter + 1][6], one row per accepted step, row 0 the start: (phi_d, phi_m, |P g|_2,
+ * CG iterations, alpha, line-search trials); rows after a chain stopped are zero.  info: [nChains][2] = (accepted steps, stop
+ * reason).  A chain's results do not depend on the other chains of the plan or on how the launches were issued.
+ * Afterwards the plan's model, fields, factors, predictions, misfit and gradient are those of m_out, as after
+ * hmcmt_forward_gradient_total(m_out); the momentum, m_ref and the mass matrix are untouched.
+ * -3 on NULL m_out / history / info, maxIter < 0, maxCG < 1, maxLS < 1, maxStep <= 0, or a negative or non-finite cgTol / tolRel;
+ * the device error flags (as hmcmt_status reports them) are checked once per outer iteration. */
+int hmcmt_gauss_newton(hmcmt_plan* plan, const double* m0, int32_t maxIter, int32_t maxCG, double cgTol, int32_t maxLS,
+                       double maxStep, double tolRel, double* m_out, double* history, int32_t* info);
 
 /* compDataGradient(mtMesh,mtData,invParam,hmcprior)  HMCSampler.jl:277-330:
  * m -> pred [nChains][nData] complex, phi_d [nChains], grad [nChains][nAC] (w.r.t. log conductivity,

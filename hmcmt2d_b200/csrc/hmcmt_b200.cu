@@ -1985,8 +1985,11 @@ int hmcmt_run_chain(hmcmt_plan* pl, double dt, int32_t nsamples, double rhoref, 
     cudaStream_t st = pl->stream;
     pl->sigmaDirect = false;
     // momentum draws travel in chunks through a two-slot device ring filled by a copy stream, so the sampling loop never
-    // synchronises the compute stream with the host; everything else is uploaded once
-    const int chunk = (int)std::max<size_t>(1, std::min<size_t>((size_t)nsamples, ((size_t)64 << 20) / (nState * sizeof(double))));
+    // synchronises the compute stream with the host; everything else is uploaded once.  A slot holds at most
+    // HMCMT_RUN_CHAIN_STAGE_BYTES (64 MiB) of draws, and at least one sample
+    size_t stageBytes = (size_t)64 << 20;
+    if (const char* e = std::getenv("HMCMT_RUN_CHAIN_STAGE_BYTES"); e && std::atoll(e) > 0) stageBytes = (size_t)std::atoll(e);
+    const int chunk = (int)std::max<size_t>(1, std::min<size_t>((size_t)nsamples, stageBytes / (nState * sizeof(double))));
     DevBuf<double> dModel, dStats, dUacc, dZ;
     DevBuf<int> dAcc, dL;
     DevBuf<unsigned char> dData;                     // [nChains][nsamples+1][nData] packed data (complex, or real for rho / phase plans)

@@ -288,6 +288,43 @@ class Plan:
                                              float(tol_rel), _lib.f64(m), _lib.f64(hist), _lib.i32(info)), "hmcmt_gauss_newton")
         return m, hist, info
 
+    def gn_eig(self, k, r=None, omega=None, seed=0):
+        """Low-rank Gauss-Newton Hessian at the last forward evaluation (after gauss_newton: the mode), hmcmt_gn_eig: the k dominant
+        pairs of H v = lambda beta Wm v, H = D Re(J^H Wd^2 J) D, by a randomized eigensolver with r test vectors (default min(nAC,
+        96, k + 10)).  omega [nChains, r, nAC] standard normal, drawn with numpy from seed when not given.  The plan keeps the
+        decomposition for set_mass_matrix(2) and laplace_sample.  Returns (lam [nChains, k] descending, V [nChains, k, nAC] with
+        V^T beta Wm V = I, info [nChains, 2] = (columns kept after B-orthonormalisation, pairs kept)); entries beyond the pairs
+        kept are zero."""
+        k = int(k)
+        if r is None:
+            r = min(self.nAC, 96, k + 10)
+        r = int(r)
+        if omega is None:
+            omega = np.random.default_rng(seed).standard_normal((self.nChains, r, self.nAC))
+        om = np.ascontiguousarray(omega, dtype=np.float64).reshape(self.nChains, r, self.nAC)
+        lam = np.zeros((self.nChains, k))
+        V = np.zeros((self.nChains, k, self.nAC))
+        info = np.zeros((self.nChains, 2), dtype=np.int32)
+        _lib.check(self.L.hmcmt_gn_eig(self.h, k, r, _lib.f64(om), _lib.f64(lam), _lib.f64(V), _lib.i32(info)), "hmcmt_gn_eig")
+        return lam, V, info
+
+    def set_mass_matrix(self, kind):
+        """Mass matrix of the sampler: 0 identity, 1 Wm, 2 beta Wm + H_k (the low-rank Gauss-Newton Hessian of gn_eig)."""
+        _lib.check(self.L.hmcmt_set_mass_matrix(self.h, int(kind)), "hmcmt_set_mass_matrix")
+
+    def laplace_sample(self, z=None, ns=1, seed=0):
+        """Draws of the Laplace approximation N(m_lin, M^-1), M = beta Wm + H_k of gn_eig at its linearisation point m_lin
+        (hmcmt_laplace_sample): m_lin + M^-1 S z, S S^T = M.  z [nChains, ns, nAC] standard normal, drawn with numpy from seed
+        when not given.  The bounds are not applied.  Returns [nChains, ns, nAC]."""
+        if z is None:
+            z = np.random.default_rng(seed).standard_normal((self.nChains, int(ns), self.nAC))
+        zz = np.ascontiguousarray(z, dtype=np.float64)
+        ns = zz.size // (self.nChains * self.nAC)
+        zz = zz.reshape(self.nChains, ns, self.nAC)
+        out = np.zeros_like(zz)
+        _lib.check(self.L.hmcmt_laplace_sample(self.h, ns, _lib.f64(zz), _lib.f64(out)), "hmcmt_laplace_sample")
+        return out
+
     def forward_gradient(self, m, total=False):
         """compDataGradient (HMCSampler.jl:277-330): predicted data, data misfit, gradient w.r.t. ln(sigma).  total=True adds the
         model-norm part beta Wm (m - m_ref) on the device (m_ref from set_state), as proposeLeapfrog does right afterwards."""

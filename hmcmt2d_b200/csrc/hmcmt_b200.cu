@@ -100,13 +100,19 @@ struct hmcmt_plan {
     int patRhs = 0, patAdj = 0;                     // sparsity patterns of the forward / adjoint right-hand sides (Solver::add_rhs_pattern)
     int patRx = 0;                                  // the receiver rows zid, zid + 1: its active set is the receiver path (gradient_range)
     // non-diagonal mass matrix M = Wm (setMassMatrix(invParam) HMCSampler.jl:478-489): invM p through a multifrontal
-    // factorisation of Wm, sqrtM z through the banded Cholesky factor of Wm (natural ordering, as the reference's dense one)
-    bool massOn = false;
+    // factorisation of Wm, sqrtM z through the banded Cholesky factor of Wm (natural ordering, as the reference's dense one).
+    // massKind: 0 identity, 1 Wm, 2 beta Wm + H_k (the low-rank Gauss-Newton Hessian of hmcmt_gn_eig)
+    int massKind = 0;
     mf::Solver* massSolver = nullptr;
     DevBuf<double> gradK, Lband;
     DevBuf<cplx> massBuf;
     DevBuf<int> massStatus;
     int massBw = 0;
+    // the decomposition of hmcmt_gn_eig (eigK columns per chain, zero beyond k'): eigV, eigW = sqrt(beta) L^T V [nChains][eigK][nAC],
+    // eigLam, eigD = lambda / (1 + lambda), eigA = sqrt(1 + lambda) - 1 [nChains][eigK], the linearisation point eigMlin
+    // [nChains][nAC]; eigS [nChains][eigK] and eigPart (block partials of V^T p, W^T z) are the scratch of mass kind 2
+    int eigK = 0;
+    DevBuf<double> eigV, eigW, eigLam, eigD, eigA, eigMlin, eigS, eigPart;
     // frequency-sharded steps: NCCL communicator over the ranks that share this chain (hmcmt_nccl_init)
     ncclComm_t comm = nullptr;
     int commWorld = 1;
@@ -780,23 +786,90 @@ __global__ void k_bandL_matvec(int n, int bw, const double* __restrict__ Lband, 
     p[(size_t)ch * n + i] = acc;
 }
 
-// gradK = invM p = Wm^{-1} p for every chain (one multifrontal solve with nChains right-hand sides)
-int mass_apply(hmcmt_plan* pl) {
-    if (!pl->massOn) return kOk;
-    const size_t n = (size_t)pl->nChains * pl->nAC;
-    k_real_to_cplx<<<(unsigned)((n + 255) / 256), 256, 0, pl->stream>>>(n, pl->p.p, pl->massBuf.p);
+// p = L^T z with the same banded factor (W = sqrt(beta) L^T V of hmcmt_gn_eig), times s.  grid (ceil(n/256), vectors)
+__global__ void k_bandLT_matvec(int n, int bw, const double* __restrict__ Lband, double s, const double* __restrict__ z, double* __restrict__ p) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const double* zz = z + (size_t)blockIdx.y * n;
+    double acc = 0.0;
+    for (int d = 0, e = min(bw, n - 1 - i); d <= e; ++d) acc += Lband[(size_t)(i + d) * (bw + 1) + d] * zz[i + d];
+    p[(size_t)blockIdx.y * n + i] = s * acc;
+}
+// y[ch][i] = s Re x[ch][i] for x [nChains][n], y with a leading dimension of its own.  grid (ceil(n/256), nChains)
+__global__ void k_cplx_to_col(int n, const cplx* __restrict__ x, double s, double* __restrict__ y, size_t ldy) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) y[(size_t)blockIdx.y * ldy + i] = s * x[(size_t)blockIdx.y * n + i].x;
+}
+// out[ch] = mlin[ch] + x[ch] (a Laplace draw), out with a leading dimension of its own.  grid (ceil(n/256), nChains)
+__global__ void k_shift_col(int n, const double* __restrict__ mlin, const double* __restrict__ x, double* __restrict__ out, size_t ldo) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    const size_t o = (size_t)blockIdx.y * n + i;
+    if (i < n) out[(size_t)blockIdx.y * ldo + i] = mlin[o] + x[o];
+}
+
+// X^T Y per chain for tall-skinny X (r1 columns) and Y (r2 columns) of length nAC: block partials, folded in block order.  The
+// block layout depends on nAC only, so a chain's result does not depend on the number of chains.
+int ts_rows(int n) { return (std::max(32 * kTsTile, (n + 127) / 128) + kTsTile - 1) / kTsTile * kTsTile; }
+int ts_blocks(int n) { return (n + ts_rows(n) - 1) / ts_rows(n); }
+int ts_dot(hmcmt_plan* pl, int r1, int r2, const double* X, size_t ldx, const double* Y, size_t ldy, double* part, double* out) {
+    const int n = pl->nAC, nb = ts_blocks(n);
+    k_ts_dot_part<<<dim3(nb, pl->nChains), kTsThreads, 0, pl->stream>>>(n, r1, r2, ts_rows(n), X, ldx, Y, ldy, part);
     LAUNCH_CHECK(pl);
-    int rc = pl->massSolver->solve(pl->stream, pl->nChains, pl->massBuf.p, pl->nAC, pl->massBuf.p, pl->nAC, &pl->launches);
-    if (rc) return rc;
-    k_cplx_to_real<<<(unsigned)((n + 255) / 256), 256, 0, pl->stream>>>(n, pl->massBuf.p, pl->gradK.p);
+    k_ts_dot_fold<<<dim3((r1 * r2 + 255) / 256, pl->nChains), 256, 0, pl->stream>>>(r1 * r2, nb, part, out);
     LAUNCH_CHECK(pl);
     return kOk;
 }
+// Y <- alpha Y + gamma X diag(w) C per chain (k_ts_update)
+int ts_update(hmcmt_plan* pl, int r1, int r2, double alpha, double gamma, const double* X, size_t ldx, const double* C, const double* w,
+              double* Y, size_t ldy) {
+    k_ts_update<<<dim3((pl->nAC + 255) / 256, r2, pl->nChains), 256, 0, pl->stream>>>(pl->nAC, r1, r2, alpha, gamma, X, ldx, C, w, Y, ldy);
+    LAUNCH_CHECK(pl);
+    return kOk;
+}
+
+// out = invM in for every chain, in and out [nChains][nAC] distinct: kind 1 Wm^{-1} in (one multifrontal solve with nChains
+// right-hand sides); kind 2 (beta Wm + H_k)^{-1} in = Wm^{-1} in / beta - V (d .* V^T in) (Woodbury, V^T beta Wm V = I)
+int mass_inv(hmcmt_plan* pl, int kind, const double* in, double* out) {
+    const size_t n = (size_t)pl->nChains * pl->nAC;
+    k_real_to_cplx<<<(unsigned)((n + 255) / 256), 256, 0, pl->stream>>>(n, in, pl->massBuf.p);
+    LAUNCH_CHECK(pl);
+    int rc = pl->massSolver->solve(pl->stream, pl->nChains, pl->massBuf.p, pl->nAC, pl->massBuf.p, pl->nAC, &pl->launches);
+    if (rc) return rc;
+    k_cplx_to_real<<<(unsigned)((n + 255) / 256), 256, 0, pl->stream>>>(n, pl->massBuf.p, out);
+    LAUNCH_CHECK(pl);
+    if (kind == 2) {
+        const size_t ld = (size_t)pl->eigK * pl->nAC;
+        if ((rc = ts_dot(pl, pl->eigK, 1, pl->eigV.p, ld, in, pl->nAC, pl->eigPart.p, pl->eigS.p))) return rc;
+        return ts_update(pl, pl->eigK, 1, 1.0 / pl->beta, -1.0, pl->eigV.p, ld, pl->eigS.p, pl->eigD.p, out, pl->nAC);
+    }
+    return kOk;
+}
+// out = S z for every chain (S S^T = M): kind 1 L z; kind 2 sqrt(beta) L (z + W (a .* W^T z)), which overwrites z with
+// sqrt(beta) (z + W (a .* W^T z)) first
+int mass_sqrt(hmcmt_plan* pl, int kind, double* z, double* out) {
+    if (kind == 2) {
+        const size_t ld = (size_t)pl->eigK * pl->nAC;
+        const double sb = std::sqrt(pl->beta);
+        int rc;
+        if ((rc = ts_dot(pl, pl->eigK, 1, pl->eigW.p, ld, z, pl->nAC, pl->eigPart.p, pl->eigS.p)) ||
+            (rc = ts_update(pl, pl->eigK, 1, sb, sb, pl->eigW.p, ld, pl->eigS.p, pl->eigA.p, z, pl->nAC)))
+            return rc;
+    }
+    k_bandL_matvec<<<dim3((pl->nAC + 255) / 256, pl->nChains), 256, 0, pl->stream>>>(pl->nAC, pl->massBw, pl->Lband.p, z, out);
+    LAUNCH_CHECK(pl);
+    return kOk;
+}
+
+// gradK = invM p for every chain
+int mass_apply(hmcmt_plan* pl) {
+    if (!pl->massKind) return kOk;
+    return mass_inv(pl, pl->massKind, pl->p.p, pl->gradK.p);
+}
 // p <- sqrtM p in place (p holds the clipped normal draws)
 int mass_sqrt_apply(hmcmt_plan* pl) {
-    if (!pl->massOn) return kOk;
-    k_bandL_matvec<<<dim3((pl->nAC + 255) / 256, pl->nChains), 256, 0, pl->stream>>>(pl->nAC, pl->massBw, pl->Lband.p, pl->p.p, pl->gradK.p);
-    LAUNCH_CHECK(pl);
+    if (!pl->massKind) return kOk;
+    int rc = mass_sqrt(pl, pl->massKind, pl->p.p, pl->gradK.p);
+    if (rc) return rc;
     HMCMT_CUDA_TRY(cudaMemcpyAsync(pl->p.p, pl->gradK.p, sizeof(double) * (size_t)pl->nChains * pl->nAC, cudaMemcpyDeviceToDevice, pl->stream));
     return kOk;
 }
@@ -805,7 +878,7 @@ int energies(hmcmt_plan* pl) {
     int mrc = mass_apply(pl);
     if (mrc) return mrc;
     k_energies<<<pl->nChains, kHmcThreads, 0, pl->stream>>>(pl->nAC, pl->m.p, pl->mref.p, pl->p.p, pl->wmPtr.p, pl->wmIdx.p, pl->wmVal.p,
-                                                            pl->beta, pl->energies.p, pl->massOn ? pl->gradK.p : nullptr);
+                                                            pl->beta, pl->energies.p, pl->massKind ? pl->gradK.p : nullptr);
     LAUNCH_CHECK(pl);
     return kOk;
 }
@@ -814,7 +887,7 @@ inline int kDriftBlocks(int nAC) { return std::max(1, std::min(128, (nAC + kHmcT
 int drift(hmcmt_plan* pl, double dt) {
     int mrc = mass_apply(pl);
     if (mrc) return mrc;
-    const double* gk = pl->massOn ? pl->gradK.p : nullptr;
+    const double* gk = pl->massKind ? pl->gradK.p : nullptr;
     const dim3 grid(kDriftBlocks(pl->nAC), pl->nChains);
     k_drift_max<<<grid, kHmcThreads, 0, pl->stream>>>(pl->nAC, dt, pl->p.p, gk, pl->driftPart.p);
     LAUNCH_CHECK(pl);
@@ -1208,7 +1281,7 @@ void hmcmt_destroy(hmcmt_plan* pl) {
     pl->driftFlag.release(); pl->packed2full.release(); pl->full2packed.release(); pl->Lsteps.release(); pl->obs.release(); pl->bc.release(); pl->bcs.release();
     pl->rhs.release(); pl->x.release(); pl->F.release(); pl->lam.release(); pl->Lam.release(); pl->srows.release(); pl->qrow.release();
     pl->scratch.release(); pl->predFull.release(); pl->ainvz.release(); pl->zadj.release(); pl->vin.release();
-    pl->predPacked.release(); pl->conCols.release(); pl->dbc.release(); pl->jvFull.release(); pl->dsigA.release(); pl->gnBuf.release(); pl->gnVec.release(); pl->gnPart.release(); pl->gnS.release(); pl->gnE.release(); pl->gnAct.release(); pl->gnI.release(); pl->xbuf.release(); pl->wexp.release(); pl->respFull.release(); pl->gradK.release(); pl->Lband.release(); pl->massBuf.release(); pl->massStatus.release(); delete pl->massSolver; pl->massSolver = nullptr; pl->mfSys.release(); delete pl->mfs; pl->mfs = nullptr; pl->fwdJobs.release(); pl->sysDesc.release(); pl->jobs.release();
+    pl->predPacked.release(); pl->conCols.release(); pl->dbc.release(); pl->jvFull.release(); pl->dsigA.release(); pl->gnBuf.release(); pl->gnVec.release(); pl->gnPart.release(); pl->gnS.release(); pl->gnE.release(); pl->gnAct.release(); pl->gnI.release(); pl->xbuf.release(); pl->wexp.release(); pl->respFull.release(); pl->gradK.release(); pl->Lband.release(); pl->eigV.release(); pl->eigW.release(); pl->eigLam.release(); pl->eigD.release(); pl->eigA.release(); pl->eigMlin.release(); pl->eigS.release(); pl->eigPart.release(); pl->massBuf.release(); pl->massStatus.release(); delete pl->massSolver; pl->massSolver = nullptr; pl->mfSys.release(); delete pl->mfs; pl->mfs = nullptr; pl->fwdJobs.release(); pl->sysDesc.release(); pl->jobs.release();
     if (pl->pin) cudaFreeHost(pl->pin);
     delete pl;
 }
@@ -1239,11 +1312,10 @@ int hmcmt_sync(hmcmt_plan* pl) {
     HMCMT_CUDA_TRY(cudaStreamSynchronize(pl->stream));
     return kOk;
 }
-int hmcmt_set_mass_matrix(hmcmt_plan* pl, int32_t kind) {
-    if (!pl || kind < 0 || kind > 1) return kErrArg;
-    HMCMT_CUDA_TRY(cudaSetDevice(pl->device));
-    if (kind == 0) { pl->massOn = false; return kOk; }
-    if (pl->massSolver) { pl->massOn = true; return kOk; }
+// The factors of Wm both non-identity mass matrices use, built on first use: invM p through a multifrontal factorisation of Wm,
+// sqrtM z through its banded Cholesky factor.  -40 if Wm is not positive definite.
+static int ensure_wm_factors(hmcmt_plan* pl) {
+    if (pl->massSolver) return kOk;
     const int n = pl->nAC;
     std::vector<int> ptr(n + 1), idx;
     std::vector<double> val;
@@ -1311,7 +1383,17 @@ int hmcmt_set_mass_matrix(hmcmt_plan* pl, int32_t kind) {
     if ((rc = pl->gradK.alloc((size_t)pl->nChains * n)) != kOk) return rc;
     if ((rc = pl->massBuf.alloc((size_t)pl->nChains * n)) != kOk) return rc;
     pl->massBw = bw;
-    pl->massOn = true;
+    return kOk;
+}
+
+int hmcmt_set_mass_matrix(hmcmt_plan* pl, int32_t kind) {
+    if (!pl || kind < 0 || kind > 2) return kErrArg;
+    HMCMT_CUDA_TRY(cudaSetDevice(pl->device));
+    if (kind == 0) { pl->massKind = 0; return kOk; }
+    if (kind == 2 && (!pl->eigV.p || !(pl->beta > 0.0))) return kErrArg;
+    int rc = ensure_wm_factors(pl);
+    if (rc) return rc;
+    pl->massKind = kind;
     return kOk;
 }
 
@@ -1607,6 +1689,16 @@ static int gn_partials(hmcmt_plan* pl, const double* v) {
     return adjoint_phase(pl, false);
 }
 
+// gnBuf, the Gauss-Newton product's [v | 0 | gsig | gdata | gtotal], allocated on first use
+static int ensure_gn_buf(hmcmt_plan* pl) {
+    if (pl->gnBuf.p) return kOk;
+    const size_t nA = (size_t)pl->nChains * pl->nAC;
+    int rc = pl->gnBuf.alloc(5 * nA);
+    if (rc) return rc;
+    HMCMT_CUDA_TRY(cudaMemsetAsync(pl->gnBuf.p + nA, 0, sizeof(double) * nA, pl->stream));      // m_ref = 0 of the prior term
+    return kOk;
+}
+
 int hmcmt_gn_hessvec(hmcmt_plan* pl, const double* v, int32_t with_prior, double* hv) {
     if (!pl || !v || !hv || !pl->haveForward) return kErrArg;
     HMCMT_CUDA_TRY(cudaSetDevice(pl->device));
@@ -1615,10 +1707,7 @@ int hmcmt_gn_hessvec(hmcmt_plan* pl, const double* v, int32_t with_prior, double
     const MeshDev& M = pl->M;
     cudaStream_t st = pl->stream;
     const size_t nA = (size_t)pl->nChains * pl->nAC;
-    if (!pl->gnBuf.p) {
-        if ((rc = pl->gnBuf.alloc(5 * nA))) return rc;
-        HMCMT_CUDA_TRY(cudaMemsetAsync(pl->gnBuf.p + nA, 0, sizeof(double) * nA, st));      // m_ref = 0 of the prior term
-    }
+    if ((rc = ensure_gn_buf(pl))) return rc;
     double *vD = pl->gnBuf.p, *zero = vD + nA, *gs = zero + nA, *gd = gs + nA, *gt = gd + nA;
     HMCMT_CUDA_TRY(cudaMemcpyAsync(vD, v, sizeof(double) * nA, cudaMemcpyHostToDevice, st));
     if ((rc = gn_partials(pl, vD))) return rc;
@@ -1825,6 +1914,148 @@ int hmcmt_gauss_newton(hmcmt_plan* pl, const double* m0, int32_t maxIter, int32_
     }
     cudaStreamSynchronize(st);
     hist.release();
+    return rc;
+}
+
+// Randomized generalized eigendecomposition H v = lambda beta Wm v at the resident state, every chain on its own (double pass,
+// Saibaba, Lee & Kitanidis 2016; include/hmcmt_b200.h, DESIGN.md 4.9).  H is the Gauss-Newton data Hessian: gn_partials reduced
+// by k_reduce_grad with (m, m_ref) = (v, 0), its data part gd.
+int hmcmt_gn_eig(hmcmt_plan* pl, int32_t k, int32_t r, const double* omega, double* lambda, double* V, int32_t* info) {
+    if (!pl || !omega || !lambda || !info || k < 1 || r < k || r > std::min(pl->nAC, kEigMaxR) || !(pl->beta > 0.0) || !pl->haveForward)
+        return kErrArg;
+    HMCMT_CUDA_TRY(cudaSetDevice(pl->device));
+    int rc;
+    if ((rc = ensure_wm_factors(pl)) || (rc = ensure_tangent(pl)) || (rc = ensure_gn_buf(pl))) return rc;
+    static PerDeviceOnce once;
+    if (once.need())
+        HMCMT_CUDA_TRY(cudaFuncSetAttribute(k_jacobi_eig, cudaFuncAttributeMaxDynamicSharedMemorySize, 2 * kEigMaxR * kEigMaxR * (int)sizeof(double)));
+    cudaStream_t st = pl->stream;
+    const int nCh = pl->nChains, n = pl->nAC;
+    const size_t nA = (size_t)nCh * n, ldr = (size_t)r * n, ldk = (size_t)k * n;
+    const MeshDev& M = pl->M;
+    double *vD = pl->gnBuf.p, *zero = vD + nA, *gs = zero + nA, *gd = gs + nA, *gt = gd + nA;
+    DevBuf<double> Y, Z, Q, G, P, sig, Cm, part, nV, nW, nLam, nD, nA_, nMlin, nS, nPart;
+    DevBuf<int> inf;
+    auto release = [&]() {
+        for (DevBuf<double>* b : {&Y, &Z, &Q, &G, &P, &sig, &Cm, &part, &nV, &nW, &nLam, &nD, &nA_, &nMlin, &nS, &nPart}) b->release();
+        inf.release();
+    };
+    const size_t rr = (size_t)nCh * r * r;
+    if ((rc = Y.alloc(nCh * ldr)) || (rc = Z.alloc(nCh * ldr)) || (rc = Q.alloc(nCh * ldr)) || (rc = G.alloc(rr)) || (rc = P.alloc(rr)) ||
+        (rc = sig.alloc((size_t)nCh * r)) || (rc = Cm.alloc(rr)) || (rc = part.alloc(rr * ts_blocks(n))) || (rc = nV.alloc(nCh * ldk)) ||
+        (rc = nW.alloc(nCh * ldk)) || (rc = nLam.alloc((size_t)nCh * k)) || (rc = nD.alloc((size_t)nCh * k)) || (rc = nA_.alloc((size_t)nCh * k)) ||
+        (rc = nMlin.alloc(nA)) || (rc = nS.alloc((size_t)nCh * k)) || (rc = nPart.alloc((size_t)nCh * k * ts_blocks(n))) ||
+        (rc = inf.alloc(2 * (size_t)nCh))) {
+        release();
+        return rc;
+    }
+    // gd <- H (column j of X) for every chain
+    auto gn_col = [&](const double* X, int j) -> int {
+        HMCMT_CUDA_TRY(cudaMemcpy2DAsync(vD, sizeof(double) * n, X + (size_t)j * n, sizeof(double) * ldr, sizeof(double) * n, nCh,
+                                         cudaMemcpyDeviceToDevice, st));
+        int e = gn_partials(pl, vD);
+        if (e) return e;
+        k_reduce_grad<<<dim3((n + 255) / 256, nCh), 256, 0, st>>>(n, M.nCell, pl->nSysPerChain, pl->act2cell.p, pl->Gpart.p, vD, zero,
+                                                                  pl->wmPtr.p, pl->wmIdx.p, pl->wmVal.p, pl->beta, pl->sigma.p, gs, gd, gt);
+        LAUNCH_CHECK(pl);
+        return kOk;
+    };
+    const size_t jsm = 2 * (size_t)r * r * sizeof(double);
+    // out <- X P Sigma^{-1/2} over the kept columns of X^T beta Wm X = P Sigma P^T; inf[2 ch] = columns kept
+    auto borth = [&](const double* X, double* out) -> int {
+        k_wm_cols<<<dim3((n + 255) / 256, r, nCh), 256, 0, st>>>(n, r, pl->wmPtr.p, pl->wmIdx.p, pl->wmVal.p, pl->beta, X, Z.p);
+        LAUNCH_CHECK(pl);
+        int e = ts_dot(pl, r, r, X, ldr, Z.p, ldr, part.p, G.p);
+        if (e) return e;
+        k_jacobi_eig<<<nCh, kJacobiThreads, jsm, st>>>(r, G.p, sig.p, P.p);
+        LAUNCH_CHECK(pl);
+        k_eig_whiten<<<nCh, 128, 0, st>>>(r, sig.p, P.p, Cm.p, inf.p);
+        LAUNCH_CHECK(pl);
+        return ts_update(pl, r, r, 0.0, 1.0, X, ldr, Cm.p, nullptr, out, ldr);
+    };
+    auto run = [&]() -> int {
+        int e;
+        // (1)-(2) Y = (beta Wm)^{-1} H Omega, one Gauss-Newton product and one Wm solve per column
+        HMCMT_CUDA_TRY(cudaMemcpyAsync(Q.p, omega, sizeof(double) * nCh * ldr, cudaMemcpyHostToDevice, st));
+        for (int j = 0; j < r; ++j) {
+            if ((e = gn_col(Q.p, j))) return e;
+            k_real_to_cplx<<<(unsigned)((nA + 255) / 256), 256, 0, st>>>(nA, gd, pl->massBuf.p);
+            LAUNCH_CHECK(pl);
+            if ((e = pl->massSolver->solve(st, nCh, pl->massBuf.p, n, pl->massBuf.p, n, &pl->launches))) return e;
+            k_cplx_to_col<<<dim3((n + 255) / 256, nCh), 256, 0, st>>>(n, pl->massBuf.p, 1.0 / pl->beta, Y.p + (size_t)j * n, ldr);
+            LAUNCH_CHECK(pl);
+        }
+        // (3) B-orthonormalise twice: Y -> Q -> Y
+        if ((e = borth(Y.p, Q.p)) || (e = borth(Q.p, Y.p))) return e;
+        std::vector<int> h(2 * nCh);
+        HMCMT_CUDA_TRY(cudaMemcpyAsync(h.data(), inf.p, sizeof(int) * 2 * nCh, cudaMemcpyDeviceToHost, st));
+        HMCMT_CUDA_TRY(cudaStreamSynchronize(st));
+        int rmax = 0;
+        for (int ch = 0; ch < nCh; ++ch) rmax = std::max(rmax, h[2 * ch]);
+        // (4) T = Q^T (H Q): the columns of Q beyond a chain's r' are zero, and so are those of H Q
+        HMCMT_CUDA_TRY(cudaMemsetAsync(Z.p, 0, sizeof(double) * nCh * ldr, st));
+        for (int j = 0; j < rmax; ++j) {
+            if ((e = gn_col(Y.p, j))) return e;
+            HMCMT_CUDA_TRY(cudaMemcpy2DAsync(Z.p + (size_t)j * n, sizeof(double) * ldr, gd, sizeof(double) * n, sizeof(double) * n, nCh,
+                                             cudaMemcpyDeviceToDevice, st));
+        }
+        if ((e = ts_dot(pl, r, r, Y.p, ldr, Z.p, ldr, part.p, G.p))) return e;
+        // (5) T = U Lambda U^T, the k' leading pairs with lambda > 0, V = Q U, signs; (6) W = sqrt(beta) L^T V
+        k_jacobi_eig<<<nCh, kJacobiThreads, jsm, st>>>(r, G.p, sig.p, P.p);
+        LAUNCH_CHECK(pl);
+        k_eig_select<<<nCh, 128, 0, st>>>(r, k, sig.p, P.p, inf.p, nLam.p, nD.p, nA_.p, Cm.p);
+        LAUNCH_CHECK(pl);
+        if ((e = ts_update(pl, r, k, 0.0, 1.0, Y.p, ldr, Cm.p, nullptr, nV.p, ldk))) return e;
+        k_col_sign<<<nCh * k, 256, 0, st>>>(n, nV.p);
+        LAUNCH_CHECK(pl);
+        k_bandLT_matvec<<<dim3((n + 255) / 256, nCh * k), 256, 0, st>>>(n, pl->massBw, pl->Lband.p, std::sqrt(pl->beta), nV.p, nW.p);
+        LAUNCH_CHECK(pl);
+        HMCMT_CUDA_TRY(cudaMemcpyAsync(nMlin.p, pl->m.p, sizeof(double) * nA, cudaMemcpyDeviceToDevice, st));
+        HMCMT_CUDA_TRY(cudaMemcpyAsync(lambda, nLam.p, sizeof(double) * nCh * k, cudaMemcpyDeviceToHost, st));
+        if (V) HMCMT_CUDA_TRY(cudaMemcpyAsync(V, nV.p, sizeof(double) * nCh * ldk, cudaMemcpyDeviceToHost, st));
+        HMCMT_CUDA_TRY(cudaMemcpyAsync(h.data(), inf.p, sizeof(int) * 2 * nCh, cudaMemcpyDeviceToHost, st));
+        HMCMT_CUDA_TRY(cudaStreamSynchronize(st));
+        for (int i = 0; i < 2 * nCh; ++i) info[i] = h[i];
+        return check_status(pl);
+    };
+    rc = run();
+    if (rc == kOk) {
+        // the new decomposition replaces the plan's (a failed call leaves the earlier one in place)
+        std::swap(pl->eigV, nV); std::swap(pl->eigW, nW); std::swap(pl->eigLam, nLam); std::swap(pl->eigD, nD);
+        std::swap(pl->eigA, nA_); std::swap(pl->eigMlin, nMlin); std::swap(pl->eigS, nS); std::swap(pl->eigPart, nPart);
+        pl->eigK = k;
+    }
+    cudaStreamSynchronize(st);
+    release();
+    return rc;
+}
+
+// Laplace draws m_lin + M^{-1} S z_i with M = beta Wm + H_k of the plan's decomposition, on scratch buffers: the chain state stays
+int hmcmt_laplace_sample(hmcmt_plan* pl, int32_t ns, const double* z, double* out) {
+    if (!pl || ns < 1 || !z || !out || !pl->eigV.p) return kErrArg;
+    HMCMT_CUDA_TRY(cudaSetDevice(pl->device));
+    cudaStream_t st = pl->stream;
+    const int nCh = pl->nChains, n = pl->nAC;
+    const size_t nA = (size_t)nCh * n, ld = (size_t)ns * n;
+    DevBuf<double> zs, a, b, res;
+    auto run = [&]() -> int {
+        int e;
+        if ((e = zs.alloc(nCh * ld)) || (e = res.alloc(nCh * ld)) || (e = a.alloc(nA)) || (e = b.alloc(nA))) return e;
+        HMCMT_CUDA_TRY(cudaMemcpyAsync(zs.p, z, sizeof(double) * nCh * ld, cudaMemcpyHostToDevice, st));
+        for (int i = 0; i < ns; ++i) {
+            HMCMT_CUDA_TRY(cudaMemcpy2DAsync(a.p, sizeof(double) * n, zs.p + (size_t)i * n, sizeof(double) * ld, sizeof(double) * n, nCh,
+                                             cudaMemcpyDeviceToDevice, st));
+            if ((e = mass_sqrt(pl, 2, a.p, b.p)) || (e = mass_inv(pl, 2, b.p, a.p))) return e;
+            k_shift_col<<<dim3((n + 255) / 256, nCh), 256, 0, st>>>(n, pl->eigMlin.p, a.p, res.p + (size_t)i * n, ld);
+            LAUNCH_CHECK(pl);
+        }
+        HMCMT_CUDA_TRY(cudaMemcpyAsync(out, res.p, sizeof(double) * nCh * ld, cudaMemcpyDeviceToHost, st));
+        HMCMT_CUDA_TRY(cudaStreamSynchronize(st));
+        return check_status(pl);
+    };
+    int rc = run();
+    cudaStreamSynchronize(st);
+    zs.release(); a.release(); b.release(); res.release();
     return rc;
 }
 

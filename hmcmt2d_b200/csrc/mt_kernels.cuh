@@ -1557,4 +1557,270 @@ k_gn_revert(int nAC, const double* __restrict__ mk, double* __restrict__ m, int*
     }
 }
 
+// ---------------------------------------------------------------------------------------------
+// Randomized generalized eigensolver H v = lambda beta Wm v (hmcmt_gn_eig) and the low-rank mass matrix it gives (kind 2).
+// Tall-skinny operands hold r columns of length n per chain, column a of chain ch at X + ch * ldx + a * n.  Every sum runs in a
+// fixed order (rows in order within a block, blocks folded in block order), so results repeat bit for bit and a chain's result
+// does not depend on the other chains.
+constexpr int kEigMaxR = 96;          // widest sketch: the Jacobi kernel keeps two kEigMaxR^2 matrices in shared memory
+constexpr int kTsThreads = 256, kTsTile = 16;
+constexpr int kJacobiThreads = 256, kJacobiSweeps = 30;
+constexpr double kJacobiTol = 1e-14;  // stop when the off-diagonal Frobenius norm is below kJacobiTol |A|_F
+
+// Block partials of X^T Y: part[ch][blk][a * r2 + b] = sum over the rows of block blk of X[ch][a][i] Y[ch][b][i], r1, r2 <=
+// kEigMaxR, rowsPerBlk a multiple of kTsTile.  grid (blocks, nChains), block kTsThreads
+__global__ void __launch_bounds__(kTsThreads)
+k_ts_dot_part(int n, int r1, int r2, int rowsPerBlk, const double* __restrict__ X, size_t ldx, const double* __restrict__ Y, size_t ldy,
+              double* __restrict__ part) {
+    constexpr int kQ = (kEigMaxR * kEigMaxR + kTsThreads - 1) / kTsThreads;
+    __shared__ double sx[kEigMaxR * kTsTile], sy[kEigMaxR * kTsTile];
+    const int ch = blockIdx.y, nOut = r1 * r2;
+    const int i0 = blockIdx.x * rowsPerBlk, i1 = min(n, i0 + rowsPerBlk);
+    const double* x = X + (size_t)ch * ldx;
+    const double* y = Y + (size_t)ch * ldy;
+    double acc[kQ];
+#pragma unroll
+    for (int q = 0; q < kQ; ++q) acc[q] = 0.0;
+    for (int t0 = i0; t0 < i1; t0 += kTsTile) {
+        const int nt = min(kTsTile, i1 - t0);
+        for (int e = threadIdx.x; e < r1 * kTsTile; e += blockDim.x) {
+            const int a = e / kTsTile, t = e % kTsTile;
+            sx[e] = t < nt ? x[(size_t)a * n + t0 + t] : 0.0;
+        }
+        for (int e = threadIdx.x; e < r2 * kTsTile; e += blockDim.x) {
+            const int b = e / kTsTile, t = e % kTsTile;
+            sy[e] = t < nt ? y[(size_t)b * n + t0 + t] : 0.0;
+        }
+        __syncthreads();
+#pragma unroll
+        for (int q = 0; q < kQ; ++q) {
+            const int o = threadIdx.x + q * kTsThreads;
+            if (o < nOut) {
+                const double* xa = sx + (o / r2) * kTsTile;
+                const double* yb = sy + (o % r2) * kTsTile;
+                double s = acc[q];
+                for (int t = 0; t < kTsTile; ++t) s = fma(xa[t], yb[t], s);
+                acc[q] = s;
+            }
+        }
+        __syncthreads();
+    }
+    double* out = part + ((size_t)ch * gridDim.x + blockIdx.x) * nOut;
+#pragma unroll
+    for (int q = 0; q < kQ; ++q) {
+        const int o = threadIdx.x + q * kTsThreads;
+        if (o < nOut) out[o] = acc[q];
+    }
+}
+
+// out[ch][o] = the nBlk partials of k_ts_dot_part summed in block order.  grid (ceil(nOut/256), nChains)
+__global__ void k_ts_dot_fold(int nOut, int nBlk, const double* __restrict__ part, double* __restrict__ out) {
+    const int o = blockIdx.x * blockDim.x + threadIdx.x, ch = blockIdx.y;
+    if (o >= nOut) return;
+    const double* p = part + (size_t)ch * nBlk * nOut + o;
+    double s = 0.0;
+    for (int b = 0; b < nBlk; ++b) s += p[(size_t)b * nOut];
+    out[(size_t)ch * nOut + o] = s;
+}
+
+// Y[ch][b] <- alpha Y[ch][b] + gamma sum_a X[ch][a] w[ch][a] C[ch][a][b]  (C row-major r1 x r2 per chain; w NULL: ones; alpha = 0
+// does not read Y).  Y must not overlap X.  grid (ceil(n/256), r2, nChains), block 256
+__global__ void k_ts_update(int n, int r1, int r2, double alpha, double gamma, const double* __restrict__ X, size_t ldx,
+                            const double* __restrict__ C, const double* __restrict__ w, double* __restrict__ Y, size_t ldy) {
+    __shared__ double sc[kEigMaxR];
+    const int i = blockIdx.x * blockDim.x + threadIdx.x, b = blockIdx.y, ch = blockIdx.z;
+    for (int a = threadIdx.x; a < r1; a += blockDim.x)
+        sc[a] = (w ? w[(size_t)ch * r1 + a] : 1.0) * C[(size_t)ch * r1 * r2 + (size_t)a * r2 + b];
+    __syncthreads();
+    if (i >= n) return;
+    const double* x = X + (size_t)ch * ldx + i;
+    double acc = 0.0;
+    for (int a = 0; a < r1; ++a) acc = fma(x[(size_t)a * n], sc[a], acc);
+    double* y = Y + (size_t)ch * ldy + (size_t)b * n + i;
+    *y = alpha == 0.0 ? gamma * acc : alpha * *y + gamma * acc;
+}
+
+// Z[ch][j] = beta Wm X[ch][j] for the r columns of every chain (CSR rows in order).  grid (ceil(n/256), r, nChains)
+__global__ void k_wm_cols(int n, int r, const int* __restrict__ wmPtr, const int* __restrict__ wmIdx, const double* __restrict__ wmVal,
+                          double beta, const double* __restrict__ X, double* __restrict__ Z) {
+    const int a = blockIdx.x * blockDim.x + threadIdx.x;
+    if (a >= n) return;
+    const size_t o = ((size_t)blockIdx.z * r + blockIdx.y) * n;
+    double s = 0.0;
+    for (int k = wmPtr[a]; k < wmPtr[a + 1]; ++k) s += wmVal[k] * X[o + wmIdx[k]];
+    Z[o + a] = beta * s;
+}
+
+// Eigendecomposition of A = (G + G^T) / 2, G [ch][r][r] row-major, r <= kEigMaxR, one CTA per chain: cyclic Jacobi in the parallel
+// (round-robin) order, r/2 disjoint rotations per round, at most kJacobiSweeps sweeps, stopped when the off-diagonal Frobenius
+// norm is at most kJacobiTol |A|_F.  lam [ch][r] descending (ties by index); eigenvector j at U[ch][j][:], with its
+// largest-magnitude entry (lowest index on ties) positive.  Dynamic shared memory 2 r^2 doubles (A, then the rotations V).
+// grid nChains, block kJacobiThreads
+__global__ void __launch_bounds__(kJacobiThreads)
+k_jacobi_eig(int r, const double* __restrict__ G, double* __restrict__ lam, double* __restrict__ U) {
+    extern __shared__ double jsm[];
+    double* A = jsm;
+    double* V = jsm + r * r;
+    __shared__ double cs[kEigMaxR / 2], sn[kEigMaxR / 2], red[kEigMaxR], dg[kEigMaxR];
+    __shared__ int ip[kEigMaxR / 2], iq[kEigMaxR / 2], rank[kEigMaxR];
+    __shared__ double sgn[kEigMaxR];
+    __shared__ int stop;
+    const int ch = blockIdx.x, tid = threadIdx.x, m = r + (r & 1), np = m / 2;
+    const double* g = G + (size_t)ch * r * r;
+    for (int e = tid; e < r * r; e += blockDim.x) {
+        const int i = e / r, j = e % r;
+        A[e] = 0.5 * (g[i * r + j] + g[j * r + i]);
+        V[e] = i == j ? 1.0 : 0.0;
+    }
+    __syncthreads();
+    // squared Frobenius norm (off = true: off-diagonal part), row sums in order, then the rows in order
+    auto sumsq = [&](bool off) {
+        if (tid < r) {
+            double s = 0.0;
+            for (int j = 0; j < r; ++j)
+                if (!off || j != tid) s += A[tid * r + j] * A[tid * r + j];
+            red[tid] = s;
+        }
+        __syncthreads();
+        double t = 0.0;
+        for (int i = 0; i < r; ++i) t += red[i];
+        __syncthreads();
+        return t;
+    };
+    const double tol2 = kJacobiTol * kJacobiTol * sumsq(false);
+    for (int sweep = 0; sweep < kJacobiSweeps; ++sweep) {
+        const double off2 = sumsq(true);
+        if (tid == 0) stop = !(off2 > tol2);
+        __syncthreads();
+        if (stop) break;
+        for (int rd = 0; rd < m - 1; ++rd) {
+            for (int k = tid; k < np; k += blockDim.x) {
+                int a = k == 0 ? m - 1 : (rd + k) % (m - 1), b = k == 0 ? rd : (rd - k + m - 1) % (m - 1);
+                const int p = min(a, b), q = max(a, b);
+                double c = 1.0, s = 0.0;
+                if (q < r) {
+                    const double apq = A[p * r + q];
+                    if (apq != 0.0) {
+                        const double tau = (A[q * r + q] - A[p * r + p]) / (2.0 * apq);
+                        const double t = (tau >= 0.0 ? 1.0 : -1.0) / (fabs(tau) + hypot(1.0, tau));
+                        c = 1.0 / sqrt(1.0 + t * t);
+                        s = t * c;
+                    }
+                }
+                ip[k] = p;
+                iq[k] = q < r ? q : -1;
+                cs[k] = c;
+                sn[k] = s;
+            }
+            __syncthreads();
+            for (int e = tid; e < r * np; e += blockDim.x) {          // columns: A <- A J, V <- V J
+                const int k = e / r, i = e % r, p = ip[k], q = iq[k];
+                if (q < 0 || sn[k] == 0.0) continue;
+                const double c = cs[k], s = sn[k];
+                const double ap = A[i * r + p], aq = A[i * r + q], vp = V[i * r + p], vq = V[i * r + q];
+                A[i * r + p] = c * ap - s * aq;
+                A[i * r + q] = s * ap + c * aq;
+                V[i * r + p] = c * vp - s * vq;
+                V[i * r + q] = s * vp + c * vq;
+            }
+            __syncthreads();
+            for (int e = tid; e < r * np; e += blockDim.x) {          // rows: A <- J^T A
+                const int k = e / r, j = e % r, p = ip[k], q = iq[k];
+                if (q < 0 || sn[k] == 0.0) continue;
+                const double c = cs[k], s = sn[k];
+                const double ap = A[p * r + j], aq = A[q * r + j];
+                A[p * r + j] = c * ap - s * aq;
+                A[q * r + j] = s * ap + c * aq;
+            }
+            __syncthreads();
+            for (int k = tid; k < np; k += blockDim.x)
+                if (iq[k] >= 0 && sn[k] != 0.0) A[ip[k] * r + iq[k]] = A[iq[k] * r + ip[k]] = 0.0;
+            __syncthreads();
+        }
+    }
+    if (tid < r) dg[tid] = A[tid * r + tid];
+    __syncthreads();
+    if (tid < r) {
+        const double d = dg[tid];
+        int rk = 0;
+        for (int j = 0; j < r; ++j) rk += dg[j] > d || (dg[j] == d && j < tid);
+        rank[tid] = rk;
+        int jm = 0;
+        double best = -1.0;
+        for (int j = 0; j < r; ++j)
+            if (fabs(V[j * r + tid]) > best) { best = fabs(V[j * r + tid]); jm = j; }
+        sgn[tid] = V[jm * r + tid] < 0.0 ? -1.0 : 1.0;
+        lam[(size_t)ch * r + rk] = d;
+    }
+    __syncthreads();
+    for (int e = tid; e < r * r; e += blockDim.x) {
+        const int i = e / r, j = e % r;
+        U[(size_t)ch * r * r + (size_t)rank[i] * r + j] = sgn[i] * V[j * r + i];
+    }
+}
+
+// B-orthonormalisation step: keep the r' leading columns with sigma_b > 1e-12 sigma_0 (sigma descending, k_jacobi_eig) and form
+// C[a][b] = P_b[a] / sqrt(sigma_b) for b < r', 0 beyond; info[2 ch] = r'.  grid nChains, block 128
+__global__ void k_eig_whiten(int r, const double* __restrict__ sig, const double* __restrict__ P, double* __restrict__ C,
+                             int* __restrict__ info) {
+    const int ch = blockIdx.x;
+    const double* s = sig + (size_t)ch * r;
+    int rk = 0;
+    while (rk < r && s[rk] > 1e-12 * s[0]) ++rk;
+    for (int e = threadIdx.x; e < r * r; e += blockDim.x) {
+        const int a = e / r, b = e % r;
+        C[(size_t)ch * r * r + e] = b < rk ? P[(size_t)ch * r * r + (size_t)b * r + a] / sqrt(s[b]) : 0.0;
+    }
+    if (threadIdx.x == 0) info[2 * ch] = rk;
+}
+
+// The eigenpairs kept: k' = the number of lambda_b > 0 among the first min(k, r') (lambda descending), C[a][b] = U_b[a] (r x k)
+// for b < k', lamOut = lambda, d = lambda / (1 + lambda), s = sqrt(1 + lambda) - 1 = lambda / (1 + sqrt(1 + lambda)); zero beyond
+// k'.  info [ch][2] = (r', k').  grid nChains, block 128
+__global__ void k_eig_select(int r, int k, const double* __restrict__ lamT, const double* __restrict__ U, int* __restrict__ info,
+                             double* __restrict__ lamOut, double* __restrict__ d, double* __restrict__ s, double* __restrict__ C) {
+    const int ch = blockIdx.x;
+    const double* l = lamT + (size_t)ch * r;
+    const int kmax = min(k, info[2 * ch]);
+    int kk = 0;
+    while (kk < kmax && l[kk] > 0.0) ++kk;
+    for (int e = threadIdx.x; e < r * k; e += blockDim.x) {
+        const int a = e / k, b = e % k;
+        C[(size_t)ch * r * k + e] = b < kk ? U[(size_t)ch * r * r + (size_t)b * r + a] : 0.0;
+    }
+    for (int b = threadIdx.x; b < k; b += blockDim.x) {
+        const double v = b < kk ? l[b] : 0.0;
+        lamOut[(size_t)ch * k + b] = v;
+        d[(size_t)ch * k + b] = v / (1.0 + v);
+        s[(size_t)ch * k + b] = v / (1.0 + sqrt(1.0 + v));
+    }
+    if (threadIdx.x == 0) info[2 * ch + 1] = kk;
+}
+
+// Sign of every column of V [nVec][n]: its largest-magnitude entry (lowest index on ties) made positive.  grid nVec, block 256
+__global__ void __launch_bounds__(256) k_col_sign(int n, double* __restrict__ V) {
+    __shared__ double bv[256];
+    __shared__ int bi[256];
+    double* v = V + (size_t)blockIdx.x * n;
+    double best = -1.0;
+    int at = 0;
+    for (int i = threadIdx.x; i < n; i += blockDim.x)
+        if (fabs(v[i]) > best) { best = fabs(v[i]); at = i; }
+    bv[threadIdx.x] = best;
+    bi[threadIdx.x] = at;
+    __syncthreads();
+    for (int h = blockDim.x / 2; h > 0; h >>= 1) {
+        if (threadIdx.x < h) {
+            const double ob = bv[threadIdx.x + h];
+            const int oi = bi[threadIdx.x + h];
+            if (ob > bv[threadIdx.x] || (ob == bv[threadIdx.x] && oi < bi[threadIdx.x])) { bv[threadIdx.x] = ob; bi[threadIdx.x] = oi; }
+        }
+        __syncthreads();
+    }
+    const bool flip = v[bi[0]] < 0.0;
+    __syncthreads();
+    if (flip)
+        for (int i = threadIdx.x; i < n; i += blockDim.x) v[i] = -v[i];
+}
+
 }  // namespace hmcmt

@@ -195,6 +195,33 @@ int hmcmt_gn_hessvec(hmcmt_plan* plan, const double* v, int32_t with_prior, doub
  * the device error flags (as hmcmt_status reports them) are checked once per outer iteration. */
 int hmcmt_gauss_newton(hmcmt_plan* plan, const double* m0, int32_t maxIter, int32_t maxCG, double cgTol, int32_t maxLS,
                        double maxStep, double tolRel, double* m_out, double* history, int32_t* info);
+/* Low-rank Gauss-Newton Hessian at the resident state: the k dominant pairs of the generalized eigenproblem
+ *   H v = lambda B v,  H = D Re(J^H Wd^2 J) D (hmcmt_gn_hessvec without the prior),  B = beta Wm = C C^T,  C = sqrt(beta) L
+ * (L the banded Cholesky factor of Wm), every chain on its own, by the double-pass randomized generalized eigensolver (Saibaba,
+ * Lee & Kitanidis 2016):
+ *   1-2. Y = B^{-1} H Omega: r Gauss-Newton products and r Wm solves;
+ *   3.   twice: G = Y^T B Y = P Sigma P^T (symmetrised, cyclic Jacobi), keep the columns with sigma_i > 1e-12 sigma_max,
+ *        Y <- Y P Sigma^{-1/2}: Q with Q^T B Q = I (r' = columns kept after the second pass; a sketch wider than the rank of H
+ *        loses columns instead of failing);
+ *   4.   T = Q^T (H Q): r' more Gauss-Newton products;
+ *   5.   T = U Lambda U^T, descending; the first min(k, r') pairs with lambda > 0 are kept (k'), V = Q U, each column of V with
+ *        its largest-magnitude entry (lowest index on ties) positive.  V^T B V = I.
+ * 1 <= k <= r <= min(nAC, 96).  omega: [nChains][r][nAC] standard-normal test vectors (drawn by the caller).  lambda: [nChains][k]
+ * descending; V: [nChains][k][nAC] or NULL; info: [nChains][2] = (r', k'); entries beyond k' are zero.
+ * The plan keeps V, W = C^T V, lambda, d = lambda / (1 + lambda), a = sqrt(1 + lambda) - 1 and m_lin (the model of the resident
+ * state), replacing an earlier decomposition: mass matrix kind 2 and hmcmt_laplace_sample use them.  It works at the state of the
+ * last forward evaluation (after hmcmt_gauss_newton: the mode) and leaves the fields, factors, predictions, misfit, gradient, m, p,
+ * m_ref and the current mass matrix kind as they were; it builds the factors of Wm on first use.  Results repeat bit for bit, and a
+ * chain's result does not depend on the other chains.  On a frequency-sharded plan the Gauss-Newton products are the rank's
+ * partial sums, so the result is not that of the whole problem.
+ * -3 without a forward evaluation, on NULL omega / lambda / info, bad k / r, or beta <= 0; -40 if Wm is not positive definite;
+ * the device error flags are checked once at the end. */
+int hmcmt_gn_eig(hmcmt_plan* plan, int32_t k, int32_t r, const double* omega, double* lambda, double* V, int32_t* info);
+/* Draws of the Laplace approximation N(m_lin, M^{-1}), M = beta Wm + H_k (mass matrix kind 2) of the plan's decomposition:
+ *   out_i = m_lin + M^{-1} S z_i,  S = C (I + W diag(a) W^T),  S S^T = M,  so M^{-1} S = S^{-T} and cov(out) = M^{-1}.
+ * z, out: [nChains][ns][nAC]; z standard normal, not clipped.  The bounds are not applied.  The chain state is untouched.
+ * -3 without a decomposition (hmcmt_gn_eig), ns < 1 or NULL z / out. */
+int hmcmt_laplace_sample(hmcmt_plan* plan, int32_t ns, const double* z, double* out);
 
 /* compDataGradient(mtMesh,mtData,invParam,hmcprior)  HMCSampler.jl:277-330:
  * m -> pred [nChains][nData] complex, phi_d [nChains], grad [nChains][nAC] (w.r.t. log conductivity,
@@ -252,7 +279,10 @@ int hmcmt_status(hmcmt_plan* plan);
  * non-diagonal M = Wm (setMassMatrix(invParam) HMCSampler.jl:478-489: dense Cholesky of Wm in the reference).  Here invM p is one
  * multifrontal solve with the sparse factor of Wm and sqrtM z the product with Wm's banded Cholesky factor (natural ordering,
  * identical to the reference's dense L).  Affects drift (getKineticGradient), kinetic energy and the momentum draws of
- * hmcmt_run_chain.  -40 if Wm is not positive definite. */
+ * hmcmt_run_chain.  -40 if Wm is not positive definite.
+ * Kind 2 = M = beta Wm + H_k = B + B V Lambda V^T B, the low-rank Gauss-Newton Hessian of hmcmt_gn_eig (a Hessian-preconditioned
+ * sampler): invM p = Wm^{-1} p / beta - V (d .* V^T p) (Woodbury with V^T B V = I: one Wm solve, one dot, one update) and
+ * sqrtM z = S z = sqrt(beta) L (z + W (a .* W^T z)), S S^T = M.  -3 without a decomposition or with beta <= 0. */
 int hmcmt_set_mass_matrix(hmcmt_plan* plan, int32_t kind);
 /* Response type of the forward evaluation of an impedance plan (compMTRespTE mt2DTE.jl:240-259, compMTRespTM mt2DTM.jl:224-242):
  * kind 0 = impedance, 1 = apparent resistivity rho_a = |Z|^2/(omega mu0) and phase atan2(Im Z, Re Z) in degrees (tipper slots keep

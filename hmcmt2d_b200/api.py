@@ -325,6 +325,17 @@ class Plan:
         _lib.check(self.L.hmcmt_laplace_sample(self.h, ns, _lib.f64(zz), _lib.f64(out)), "hmcmt_laplace_sample")
         return out
 
+    def posterior_variance(self, prior=True, posterior=True, resolution=True):
+        """Per-cell variances in ln sigma (hmcmt_posterior_variance): (prior_var [nAC] = diag((beta Wm)^-1), post_var [nChains, nAC]
+        = diag(M^-1) of the Laplace approximation with M = beta Wm + H_k of gn_eig, resolution [nChains, nAC] = diag(V D V^T beta Wm)).
+        An output not asked for is None; post_var and resolution need gn_eig first.  The bounds are not applied."""
+        pv = np.zeros(self.nAC) if prior else None
+        qv = np.zeros((self.nChains, self.nAC)) if posterior else None
+        rv = np.zeros((self.nChains, self.nAC)) if resolution else None
+        ptr = lambda a: _lib.f64(a) if a is not None else None  # noqa: E731
+        _lib.check(self.L.hmcmt_posterior_variance(self.h, ptr(pv), ptr(qv), ptr(rv)), "hmcmt_posterior_variance")
+        return pv, qv, rv
+
     def forward_gradient(self, m, total=False):
         """compDataGradient (HMCSampler.jl:277-330): predicted data, data misfit, gradient w.r.t. ln(sigma).  total=True adds the
         model-norm part beta Wm (m - m_ref) on the device (m_ref from set_state), as proposeLeapfrog does right afterwards."""
@@ -806,6 +817,25 @@ def getPosteriorModel(hmcmodel, mtMesh, invParam, hmcprior, outdir: str = "."):
     out.sigma = invParam.activeCell @ std + invParam.bgModel
     writeEMModel2D(os.path.join(outdir, "stdModel.model"), out)
     return mean, std
+
+
+def getLaplacePosteriorModel(plan, m_map, mtMesh, invParam, outdir: str = ".", chain: int = 0):
+    """The Laplace approximation's counterpart of getPosteriorModel: laplaceMeanModel.model holds exp(m_map) and
+    laplaceStdModel.model the posterior standard deviation in ln sigma, sqrt(diag(M^-1)) of Plan.posterior_variance (M = beta Wm
+    + H_k of the plan's gn_eig decomposition), in the same format and active-cell / background composition as meanModel.model /
+    stdModel.model, so the Laplace and HMC maps compare file to file.  m_map: [nAC] (or [nChains, nAC], row `chain` used);
+    `chain` selects the plan's chain.  Returns (m_map, std) of that chain."""
+    m = np.asarray(m_map, dtype=np.float64)
+    if m.ndim == 2:
+        m = m[chain]
+    _, post, _ = plan.posterior_variance(prior=False, posterior=True, resolution=False)
+    std = np.sqrt(np.maximum(post[chain], 0.0))
+    out = TensorMesh2D(mtMesh.yLen, mtMesh.zLen, mtMesh.airLayer, mtMesh.gridSize, mtMesh.origin, None)
+    out.sigma = invParam.activeCell @ np.exp(m) + invParam.bgModel
+    writeEMModel2D(os.path.join(outdir, "laplaceMeanModel.model"), out)
+    out.sigma = invParam.activeCell @ std + invParam.bgModel
+    writeEMModel2D(os.path.join(outdir, "laplaceStdModel.model"), out)
+    return m, std
 
 
 def outputHMCSamples(hmcmodel, hmcstats: HMCStatus, hmcdata, ichain: int = 1, cputime: float = 0.0, outdir: str = "."):

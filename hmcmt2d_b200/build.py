@@ -16,7 +16,7 @@ HDR = os.path.join("..", "..", "include", "hmcmt_b200.h")
 SOURCES = {
     "hmcmt_b200.cu": ["common.cuh", "band_factor.cuh", "band_solve.cuh", "mt_kernels.cuh", "mf_solver.cuh", "mf_symbolic.h", HDR],
     "mumps_shim.cu": ["common.cuh", "band_factor.cuh", "band_solve.cuh", "mf_solver.cuh", "mf_symbolic.h", HDR],
-    "mf_solver.cu": ["common.cuh", "band_factor.cuh", "mf_kernels.cuh", "mf_solver.cuh", "mf_symbolic.h"],
+    "mf_solver.cu": ["common.cuh", "band_factor.cuh", "mf_kernels.cuh", "mf_selinv.cuh", "mf_solver.cuh", "mf_symbolic.h"],
 }
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "-Xcompiler", "-fPIC"]
 

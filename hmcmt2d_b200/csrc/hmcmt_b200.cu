@@ -113,6 +113,7 @@ struct hmcmt_plan {
     // [nChains][nAC]; eigS [nChains][eigK] and eigPart (block partials of V^T p, W^T z) are the scratch of mass kind 2
     int eigK = 0;
     DevBuf<double> eigV, eigW, eigLam, eigD, eigA, eigMlin, eigS, eigPart;
+    DevBuf<double> wmInvDiag;                       // diag(Wm^{-1}) [nAC], hmcmt_posterior_variance, computed on first use
     // frequency-sharded steps: NCCL communicator over the ranks that share this chain (hmcmt_nccl_init)
     ncclComm_t comm = nullptr;
     int commWorld = 1;
@@ -1281,7 +1282,7 @@ void hmcmt_destroy(hmcmt_plan* pl) {
     pl->driftFlag.release(); pl->packed2full.release(); pl->full2packed.release(); pl->Lsteps.release(); pl->obs.release(); pl->bc.release(); pl->bcs.release();
     pl->rhs.release(); pl->x.release(); pl->F.release(); pl->lam.release(); pl->Lam.release(); pl->srows.release(); pl->qrow.release();
     pl->scratch.release(); pl->predFull.release(); pl->ainvz.release(); pl->zadj.release(); pl->vin.release();
-    pl->predPacked.release(); pl->conCols.release(); pl->dbc.release(); pl->jvFull.release(); pl->dsigA.release(); pl->gnBuf.release(); pl->gnVec.release(); pl->gnPart.release(); pl->gnS.release(); pl->gnE.release(); pl->gnAct.release(); pl->gnI.release(); pl->xbuf.release(); pl->wexp.release(); pl->respFull.release(); pl->gradK.release(); pl->Lband.release(); pl->eigV.release(); pl->eigW.release(); pl->eigLam.release(); pl->eigD.release(); pl->eigA.release(); pl->eigMlin.release(); pl->eigS.release(); pl->eigPart.release(); pl->massBuf.release(); pl->massStatus.release(); delete pl->massSolver; pl->massSolver = nullptr; pl->mfSys.release(); delete pl->mfs; pl->mfs = nullptr; pl->fwdJobs.release(); pl->sysDesc.release(); pl->jobs.release();
+    pl->predPacked.release(); pl->conCols.release(); pl->dbc.release(); pl->jvFull.release(); pl->dsigA.release(); pl->gnBuf.release(); pl->gnVec.release(); pl->gnPart.release(); pl->gnS.release(); pl->gnE.release(); pl->gnAct.release(); pl->gnI.release(); pl->xbuf.release(); pl->wexp.release(); pl->respFull.release(); pl->gradK.release(); pl->Lband.release(); pl->eigV.release(); pl->eigW.release(); pl->eigLam.release(); pl->eigD.release(); pl->eigA.release(); pl->eigMlin.release(); pl->eigS.release(); pl->eigPart.release(); pl->wmInvDiag.release(); pl->massBuf.release(); pl->massStatus.release(); delete pl->massSolver; pl->massSolver = nullptr; pl->mfSys.release(); delete pl->mfs; pl->mfs = nullptr; pl->fwdJobs.release(); pl->sysDesc.release(); pl->jobs.release();
     if (pl->pin) cudaFreeHost(pl->pin);
     delete pl;
 }
@@ -2056,6 +2057,61 @@ int hmcmt_laplace_sample(hmcmt_plan* pl, int32_t ns, const double* z, double* ou
     int rc = run();
     cudaStreamSynchronize(st);
     zs.release(); a.release(); b.release(); res.release();
+    return rc;
+}
+
+int hmcmt_posterior_variance(hmcmt_plan* pl, double* prior_var, double* post_var, double* resolution) {
+    if (!pl || !(pl->beta > 0.0) || (!prior_var && !post_var && !resolution)) return kErrArg;
+    if ((post_var || resolution) && !pl->eigV.p) return kErrArg;
+    HMCMT_CUDA_TRY(cudaSetDevice(pl->device));
+    cudaStream_t st = pl->stream;
+    const int nCh = pl->nChains, n = pl->nAC, k = pl->eigK;
+    int rc = ensure_wm_factors(pl);
+    if (rc) return rc;
+    if (!pl->wmInvDiag.p) {      // diag(Wm^{-1}) by a selected inversion of the resident factor of Wm (system 0, real values)
+        DevBuf<cplx> z;
+        DevBuf<double> w;
+        auto first = [&]() -> int {
+            int e;
+            if ((e = z.alloc(n)) || (e = w.alloc(n))) return e;
+            if ((e = pl->massSolver->inverse_diag(st, z.p, n, &pl->launches))) return e;
+            k_real_part<<<(n + 255) / 256, 256, 0, st>>>(n, z.p, w.p);
+            LAUNCH_CHECK(pl);
+            HMCMT_CUDA_TRY(cudaStreamSynchronize(st));
+            return kOk;
+        };
+        rc = first();
+        cudaStreamSynchronize(st);
+        z.release();
+        if (rc) { w.release(); return rc; }
+        std::swap(pl->wmInvDiag, w);
+    }
+    DevBuf<double> bv, post, res;
+    auto run = [&]() -> int {
+        int e;
+        if (prior_var) {
+            HMCMT_CUDA_TRY(cudaMemcpyAsync(prior_var, pl->wmInvDiag.p, sizeof(double) * n, cudaMemcpyDeviceToHost, st));
+            HMCMT_CUDA_TRY(cudaStreamSynchronize(st));
+            for (int a = 0; a < n; ++a) prior_var[a] /= pl->beta;
+        }
+        if (!post_var && !resolution) return kOk;
+        const size_t nA = (size_t)nCh * n;
+        if ((post_var && (e = post.alloc(nA))) || (resolution && (e = res.alloc(nA)))) return e;
+        if (resolution) {
+            if ((e = bv.alloc((size_t)nCh * k * n))) return e;
+            k_wm_cols<<<dim3((n + 255) / 256, k, nCh), 256, 0, st>>>(n, k, pl->wmPtr.p, pl->wmIdx.p, pl->wmVal.p, pl->beta, pl->eigV.p, bv.p);
+            LAUNCH_CHECK(pl);
+        }
+        k_post_var<<<dim3((n + 255) / 256, nCh), 256, 0, st>>>(n, k, pl->beta, pl->wmInvDiag.p, pl->eigV.p, bv.p, pl->eigD.p, post.p, res.p);
+        LAUNCH_CHECK(pl);
+        if (post_var) HMCMT_CUDA_TRY(cudaMemcpyAsync(post_var, post.p, sizeof(double) * nA, cudaMemcpyDeviceToHost, st));
+        if (resolution) HMCMT_CUDA_TRY(cudaMemcpyAsync(resolution, res.p, sizeof(double) * nA, cudaMemcpyDeviceToHost, st));
+        HMCMT_CUDA_TRY(cudaStreamSynchronize(st));
+        return check_status(pl);
+    };
+    rc = run();
+    cudaStreamSynchronize(st);
+    bv.release(); post.release(); res.release();
     return rc;
 }
 

@@ -6,6 +6,7 @@
 #include <cstdlib>
 
 #include "mf_kernels.cuh"
+#include "mf_selinv.cuh"
 
 namespace hmcmt {
 namespace mf {
@@ -547,6 +548,125 @@ int Solver::backward_pair(cudaStream_t st, cplx* Xa, cplx* Xb, int64_t ldx, int6
         if (D.nSolveCta) {
             mf_bwd_pair_kernel<<<dim3(D.nSolveCta, n), D.solveCtaThreads, pairSmem, st>>>(tb, sa, sb, P.pairCtaList[d], P.nPairCtaBoth[d]);
             ++nl;
+        }
+    }
+    HMCMT_CUDA_TRY(cudaGetLastError());
+    if (nLaunches) *nLaunches += nl;
+    return kOk;
+}
+
+// ------------------------------------------------------------------------------------------------------------------------
+// selected inversion (mf_selinv.cuh).  Tables from the symbolic analysis, on the first call only: the Z square of every front in
+// the arena of its depth parity, the gather tiles of every depth, and per chunk step the product jobs and their 64 x 64 tiles.
+// The schedule depends on the tree alone (no routing knob is read), so the result does not depend on how the factor was launched.
+int Solver::build_selinv() {
+    int rc;
+#define MF_TRY(x) do { rc = (x); if (rc) return rc; } while (0)
+    std::vector<int64_t> zOff(S.K, 0);
+    std::vector<std::vector<int>> byDepth(S.maxDepth + 1);
+    for (int d = 0; d <= S.maxDepth; ++d) {
+        byDepth[d] = S.byDepthBig[d];
+        byDepth[d].insert(byDepth[d].end(), S.byDepthSmall[d].begin(), S.byDepthSmall[d].end());
+        int64_t at = 0;
+        for (int k : byDepth[d]) {
+            zOff[k] = at;
+            at += 2 * (int64_t)S.fronts[k].fp() * S.fronts[k].fp();
+        }
+        zDoubles[d & 1] = std::max(zDoubles[d & 1], at);
+    }
+    MF_TRY(upload(zOff, &d_zOff));
+    for (int p = 0; p < 2; ++p) {
+        const size_t nb = std::max<size_t>((size_t)nsys * zDoubles[p] * sizeof(double), 16);
+        if (cudaMalloc(&d_zarena[p], nb) != cudaSuccess) return kErrAlloc;
+        owned.push_back(d_zarena[p]);
+        bytes += nb;
+    }
+    selSched.assign(S.maxDepth + 1, SelDepth());
+    for (int d = 0; d <= S.maxDepth; ++d) {
+        SelDepth& D = selSched[d];
+        std::vector<SelGatherTile> gt;
+        int maxChunk = 0;
+        for (int k : byDepth[d]) {
+            const Front& F = S.fronts[k];
+            maxChunk = std::max(maxChunk, F.nChunk);
+            const int nt = (F.up + 63) / 64;
+            if (F.u > 0)
+                for (int bi = 0; bi < nt; ++bi)
+                    for (int bj = 0; bj < nt; ++bj) gt.push_back(SelGatherTile{k, bi, bj});
+        }
+        SelGatherTile* pg = nullptr;
+        if (!gt.empty()) { MF_TRY(upload(gt, &pg)); D.gather = pg; D.nGather = (int)gt.size(); }
+        for (int s = 0; s < maxChunk; ++s) {
+            std::vector<SelJob> jobs;
+            std::vector<SelTile> t1, t2;
+            for (int k : byDepth[d]) {
+                const Front& F = S.fronts[k];
+                if (F.nChunk <= s) continue;
+                const Chunk& ch = S.chunks[F.chunkPtr + F.nChunk - 1 - s];
+                const int sc = ch.p1 - ch.p0, mr = F.fp() - ch.p1;
+                if (mr > 0) {      // Z(R, c) = -Z(R, R) M_c, and its transpose Z(c, R)
+                    SelJob j{};
+                    j.front = k; j.bOff = ch.mOff; j.ldB = mr; j.rA = ch.p1; j.kA = ch.p1; j.rC = ch.p1; j.cC = ch.p0;
+                    j.m = mr; j.n = sc; j.K = mr; j.transC = 1; j.alpha = -1.0;
+                    const int ji = (int)jobs.size();
+                    jobs.push_back(j);
+                    for (int bi = 0; bi < (mr + 63) / 64; ++bi)
+                        for (int bj = 0; bj < (sc + 63) / 64; ++bj) t1.push_back(SelTile{ji, bi, bj});
+                }
+                SelJob j{};      // Z(c, c) = G_c - Z(c, R) M_c, diagonal of the real pivots to out
+                j.front = k; j.bOff = ch.mOff; j.ldB = mr; j.sOff = ch.gOff; j.ldS = sc; j.hasS = 1; j.rA = ch.p0; j.kA = ch.p1;
+                j.rC = ch.p0; j.cC = ch.p0; j.m = sc; j.n = sc; j.K = mr; j.diag = 1; j.alpha = -1.0;
+                const int ji = (int)jobs.size();
+                jobs.push_back(j);
+                for (int bi = 0; bi < (sc + 63) / 64; ++bi)
+                    for (int bj = 0; bj < (sc + 63) / 64; ++bj) t2.push_back(SelTile{ji, bi, bj});
+            }
+            SelStep st;
+            SelJob* pj = nullptr;
+            SelTile* pt = nullptr;
+            MF_TRY(upload(jobs, &pj));
+            st.jobs = pj;
+            if (!t1.empty()) { MF_TRY(upload(t1, &pt)); st.tiles1 = pt; st.n1 = (int)t1.size(); }
+            if (!t2.empty()) { MF_TRY(upload(t2, &pt)); st.tiles2 = pt; st.n2 = (int)t2.size(); }
+            D.steps.push_back(st);
+        }
+    }
+#undef MF_TRY
+    selBuilt = true;
+    return kOk;
+}
+
+int Solver::inverse_diag(cudaStream_t st, cplx* out, int64_t ldo, int64_t* nLaunches, int sys0, int n) {
+    if (!out || ldo < S.N) return kErrArg;
+    if (n < 0) n = this->nsys - sys0;
+    if (sys0 < 0 || n < 1 || sys0 + n > this->nsys) return kErrArg;
+    if (!selBuilt) {
+        const int rc = build_selinv();
+        if (rc) return rc;
+    }
+    static PerDeviceOnceMf once;
+    if (once.need()) HMCMT_CUDA_TRY(cudaFuncSetAttribute(mf_selinv_gemm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kGemmSmemBytes));
+    SelTables tb{};
+    tb.fronts = d_fronts; tb.rel = d_rel; tb.pos2orig = d_pos2orig; tb.zOff = d_zOff;
+    tb.fac = d_fac + (size_t)sys0 * S.factorDoubles; tb.facStride = S.factorDoubles;
+    for (int p = 0; p < 2; ++p) { tb.zarena[p] = d_zarena[p] + (size_t)sys0 * zDoubles[p]; tb.zStride[p] = zDoubles[p]; }
+    tb.out = out + (size_t)sys0 * ldo; tb.ldo = ldo;
+    int64_t nl = 0;
+    for (int d = 0; d <= S.maxDepth; ++d) {
+        const SelDepth& D = selSched[d];
+        if (D.nGather) {
+            mf_selinv_gather_kernel<<<dim3(D.nGather, n), 256, 0, st>>>(tb, (const SelGatherTile*)D.gather);
+            ++nl;
+        }
+        for (const SelStep& s : D.steps) {
+            if (s.n1) {
+                mf_selinv_gemm_kernel<<<dim3(s.n1, n), kGemmThreads, kGemmSmemBytes, st>>>(tb, (const SelJob*)s.jobs, (const SelTile*)s.tiles1);
+                ++nl;
+            }
+            if (s.n2) {
+                mf_selinv_gemm_kernel<<<dim3(s.n2, n), kGemmThreads, kGemmSmemBytes, st>>>(tb, (const SelJob*)s.jobs, (const SelTile*)s.tiles2);
+                ++nl;
+            }
         }
     }
     HMCMT_CUDA_TRY(cudaGetLastError());

@@ -112,8 +112,13 @@ class Solver {
     int add_rhs_pattern(const std::vector<unsigned char>& nz);
     // fronts visited by the forward elimination of a pattern (0: all), for diagnostics
     int fwd_fronts(int pattern) const;
+    // diag(A^{-1}) of every system of the range, by a selected inversion of the resident factor (mf_selinv.cuh): system s at
+    // out + s*ldo, original numbering (out is the base of the whole batch, as in solve()).  Run after factor().  The launch lists
+    // and the two depth-parity arenas of the inverse's fronts are built on the first call; nothing else is touched.
+    int inverse_diag(cudaStream_t st, cplx* out, int64_t ldo, int64_t* nLaunches = nullptr, int sys0 = 0, int n = -1);
     size_t device_bytes() const { return bytes; }
     double factor_flops() const { return S.flops; }
+    double selinv_flops() const { return S.selinvFlops; }
     int64_t factor_doubles() const { return S.factorDoubles; }
 
   private:
@@ -127,6 +132,7 @@ class Solver {
     int set_solve_attributes();
     int clear_ws(cudaStream_t st, const SolveArgs& sa, int nvec);
     int fwd_sweep(cudaStream_t st, const Tables& tb, const SolveArgs& sa, int nvec, int pattern, int64_t& nl);
+    int build_selinv();
     Symbolic S;
     int nsys = 0, maxRhs = 1;
     int64_t valCount = 0;
@@ -155,6 +161,24 @@ class Solver {
     size_t solveSmem = 0;
     size_t pairSmem = 0;                       // mf_bwd_pair_kernel: two vectors of the largest front and their chunk stages
     unsigned long long* d_prof = nullptr;      // HMCMT_MF_PROF=1: phase cycle counters of mf_small_kernel
+    // selected inversion (inverse_diag), built on its first call: per depth (roots first) the gather tiles of Z(U, U), then per
+    // chunk step (every front's last chunk first) the tiles of Z(R, c) = -Z(R, R) M_c and of Z(c, c) = G_c - Z(c, R) M_c
+    struct SelStep {
+        const void* jobs = nullptr;            // SelJob[]
+        const void* tiles1 = nullptr;          // SelTile[n1]: Z(R, c)
+        const void* tiles2 = nullptr;          // SelTile[n2]: Z(c, c) and the diagonal
+        int n1 = 0, n2 = 0;
+    };
+    struct SelDepth {
+        const void* gather = nullptr;          // SelGatherTile[nGather]
+        int nGather = 0;
+        std::vector<SelStep> steps;
+    };
+    std::vector<SelDepth> selSched;
+    bool selBuilt = false;
+    int64_t* d_zOff = nullptr;
+    double* d_zarena[2] = {nullptr, nullptr};
+    int64_t zDoubles[2] = {0, 0};              // per system, depth parity
 };
 
 }  // namespace mf

@@ -115,6 +115,7 @@ struct Symbolic {
     int64_t updEntries = 0;             // per system: total update-vector entries (complex)
     int maxFpSmall = 0, maxFpBig = 0, maxFp = 0;
     double flops = 0.0;                 // real flops of one factorisation (padded sizes, sweep formulation)
+    double selinvFlops = 0.0;           // real flops of the selected inversion (Solver::inverse_diag): two products per chunk
 };
 
 // ------------------------------------------------------------------------------------------------------------------------
@@ -467,6 +468,7 @@ inline bool mf_symbolic(int N, const std::vector<std::vector<int>>& snodes, cons
             S.chunks.push_back(c);
             const double a = sc, b = fp - p1;
             S.flops += 8.0 * (0.5 * a * a * a + a * a * b + 0.5 * a * b * b);
+            S.selinvFlops += 8.0 * (a * b * b + a * a * b);      // Z(R, c) = -Z(R, R) M_c,  Z(c, c) = G_c - Z(c, R) M_c
         }
         F.nChunk = (int)S.chunks.size() - F.chunkPtr;
     }

@@ -1640,6 +1640,30 @@ __global__ void k_ts_update(int n, int r1, int r2, double alpha, double gamma, c
     *y = alpha == 0.0 ? gamma * acc : alpha * *y + gamma * acc;
 }
 
+// hmcmt_posterior_variance, one thread per (cell a, chain): post[ch][a] = wid[a] / beta - sum_j d_j V_ja^2 and
+// res[ch][a] = sum_j d_j V_ja (beta Wm V)_ja, j = 0 .. k-1 in order (V, BV: [nChains][k][n], d: [nChains][k]; either output may be
+// NULL).  wid: diag(Wm^{-1}).  grid (ceil(n/256), nChains)
+__global__ void k_post_var(int n, int k, double beta, const double* __restrict__ wid, const double* __restrict__ V,
+                           const double* __restrict__ BV, const double* __restrict__ d, double* __restrict__ post,
+                           double* __restrict__ res) {
+    const int a = blockIdx.x * blockDim.x + threadIdx.x, ch = blockIdx.y;
+    if (a >= n) return;
+    const size_t o = (size_t)ch * k * n + a;
+    double sv = 0.0, sr = 0.0;
+    for (int j = 0; j < k; ++j) {
+        const double dj = d[(size_t)ch * k + j], v = V[o + (size_t)j * n];
+        sv += dj * v * v;
+        if (res) sr += dj * v * BV[o + (size_t)j * n];
+    }
+    if (post) post[(size_t)ch * n + a] = wid[a] / beta - sv;
+    if (res) res[(size_t)ch * n + a] = sr;
+}
+// real part of a complex vector (the imaginary part of diag(Wm^{-1}) is exactly zero)
+__global__ void k_real_part(int n, const cplx* __restrict__ x, double* __restrict__ y) {
+    const int a = blockIdx.x * blockDim.x + threadIdx.x;
+    if (a < n) y[a] = x[a].x;
+}
+
 // Z[ch][j] = beta Wm X[ch][j] for the r columns of every chain (CSR rows in order).  grid (ceil(n/256), r, nChains)
 __global__ void k_wm_cols(int n, int r, const int* __restrict__ wmPtr, const int* __restrict__ wmIdx, const double* __restrict__ wmVal,
                           double beta, const double* __restrict__ X, double* __restrict__ Z) {

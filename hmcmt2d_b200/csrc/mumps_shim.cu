@@ -353,6 +353,34 @@ int64_t hmcmt_debug_get_factor(int64_t handle, double* panels, double* ainv, int
     if (ainv) cudaMemcpy(ainv, f->ainvz, (size_t)f->S * AZ * sizeof(cplx), cudaMemcpyDeviceToHost);
     return kOk;
 }
+int64_t hmcmt_factor_inverse_diag(const int64_t* handle, double* out) {
+    if (!handle || !out) return kErrArg;
+    Factor* f = lookup(*handle);
+    if (!f || !f->mfs) return kErrArg;
+    const size_t n = f->n;
+    cplx* d = nullptr;
+    if (cudaMalloc(&d, n * sizeof(cplx)) != cudaSuccess) return kErrAlloc;
+    int rc = f->mfs->inverse_diag(nullptr, d, (int64_t)n);
+    if (rc == kOk && cudaDeviceSynchronize() != cudaSuccess) rc = kErrCuda;
+    if (rc == kOk) {
+        std::vector<cplx> h(n);
+        if (cudaMemcpy(h.data(), d, n * sizeof(cplx), cudaMemcpyDeviceToHost) != cudaSuccess) rc = kErrCuda;
+        for (size_t i = 0; rc == kOk && i < n; ++i) {
+            if (f->isReal) out[i] = h[i].x;
+            else { out[2 * i] = h[i].x; out[2 * i + 1] = h[i].y; }
+        }
+    }
+    cudaFree(d);
+    return rc;
+}
+int64_t hmcmt_debug_factor_flops(const int64_t* handle, double* flops) {
+    if (!handle || !flops) return kErrArg;
+    Factor* f = lookup(*handle);
+    if (!f || !f->mfs) return kErrArg;
+    flops[0] = f->mfs->factor_flops();
+    flops[1] = f->mfs->selinv_flops();
+    return kOk;
+}
 int64_t destroy_mumps_(const int64_t* handle) { return handle ? destroy_common(*handle) : kErrArg; }
 int64_t destroy_mumps_cmplx_(const int64_t* handle) { return handle ? destroy_common(*handle) : kErrArg; }
 

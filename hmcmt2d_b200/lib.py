@@ -69,6 +69,7 @@ def load() -> C.CDLL:
                                        _f64p, _i32p]
     lib.hmcmt_gn_eig.argtypes = [vp, C.c_int32, C.c_int32, _f64p, _f64p, _f64p, _i32p]
     lib.hmcmt_laplace_sample.argtypes = [vp, C.c_int32, _f64p, _f64p]
+    lib.hmcmt_posterior_variance.argtypes = [vp, _f64p, _f64p, _f64p]
     lib.hmcmt_status.argtypes = [vp]
     lib.hmcmt_set_mass_matrix.argtypes = [vp, C.c_int32]
     lib.hmcmt_set_response_kind.argtypes = [vp, C.c_int32]
@@ -105,6 +106,10 @@ def load() -> C.CDLL:
         fn = getattr(lib, name)
         fn.argtypes = [_i64p, _i64p, _i64p, _f64p, _i64p, _i64p, _f64p, _i64p]
         fn.restype = None
+    lib.hmcmt_factor_inverse_diag.argtypes = [_i64p, _f64p]
+    lib.hmcmt_factor_inverse_diag.restype = C.c_int64
+    lib.hmcmt_debug_factor_flops.argtypes = [_i64p, _f64p]
+    lib.hmcmt_debug_factor_flops.restype = C.c_int64
     for name in ("destroy_mumps_", "destroy_mumps_cmplx_"):
         fn = getattr(lib, name)
         fn.argtypes = [_i64p]
@@ -115,9 +120,9 @@ def load() -> C.CDLL:
 
 EXPORTED_SYMBOLS = [
     "factor_mumps_cmplx_", "factor_mumps_", "solve_mumps_cmplx_", "solve_mumps_", "solve_mumps_sparse_rhs_",
-    "solve_mumps_cmplx_sparse_rhs_", "destroy_mumps_", "destroy_mumps_cmplx_",
+    "solve_mumps_cmplx_sparse_rhs_", "destroy_mumps_", "destroy_mumps_cmplx_", "hmcmt_factor_inverse_diag", "hmcmt_debug_factor_flops",
     "hmcmt_plan_create", "hmcmt_plan_create_rho_phase", "hmcmt_destroy", "hmcmt_plan_info", "hmcmt_forward", "hmcmt_forward_sigma", "hmcmt_jtvec",
-    "hmcmt_forward_gradient", "hmcmt_forward_gradient_total", "hmcmt_jacobian", "hmcmt_jvec", "hmcmt_gn_hessvec", "hmcmt_gauss_newton", "hmcmt_gn_eig", "hmcmt_laplace_sample", "hmcmt_status", "hmcmt_set_mass_matrix", "hmcmt_set_response_kind", "hmcmt_get_responses",
+    "hmcmt_forward_gradient", "hmcmt_forward_gradient_total", "hmcmt_jacobian", "hmcmt_jvec", "hmcmt_gn_hessvec", "hmcmt_gauss_newton", "hmcmt_gn_eig", "hmcmt_laplace_sample", "hmcmt_posterior_variance", "hmcmt_status", "hmcmt_set_mass_matrix", "hmcmt_set_response_kind", "hmcmt_get_responses",
     "hmcmt_set_state", "hmcmt_get_state", "hmcmt_leapfrog_trajectory", "hmcmt_leapfrog_steps_device", "hmcmt_sync",
     "hmcmt_step_partial", "hmcmt_exchange_buffer", "hmcmt_step_finish", "hmcmt_nccl_unique_id", "hmcmt_nccl_init",
     "hmcmt_leapfrog_steps_sharded",
@@ -187,6 +192,16 @@ def applyMUMPS(factor: MUMPSfactorization, rhs, tr: int = 0):
     rc = fn(C.byref(h), C.byref(nr), b.ctypes.data_as(_f64p), x.ctypes.data_as(_f64p), C.byref(t))
     check(rc, "applyMUMPS")
     return x[:, 0].copy() if rhs.ndim == 1 else np.ascontiguousarray(x)
+
+
+def inverse_diag(factor: MUMPSfactorization):
+    """diag(A^-1) of a factorised matrix (selected inversion of the multifrontal factor on the device): complex128 for a
+    complex factor, float64 for a real one.  Raises HmcmtError(-3) for a band-routed or destroyed handle."""
+    lib = load()
+    out = np.zeros(factor.n, dtype=np.complex128 if factor.is_complex else np.float64)
+    h = C.c_int64(factor.ptr)
+    check(lib.hmcmt_factor_inverse_diag(C.byref(h), out.ctypes.data_as(_f64p)), "inverse_diag")
+    return out
 
 
 def destroyMUMPS(factor: MUMPSfactorization):

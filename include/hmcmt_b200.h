@@ -60,6 +60,15 @@ void solve_mumps_cmplx_sparse_rhs_(const int64_t* handle, const int64_t* nzrhs, 
 /* destroyMUMPS  MUMPSfuncs.jl:148-176 */
 int64_t destroy_mumps_(const int64_t* handle);
 int64_t destroy_mumps_cmplx_(const int64_t* handle);
+/* Diagonal of the inverse of a factorised matrix (MUMPS offers entries of A^-1; here the diagonal only): a selected
+ * inversion of the multifrontal factor on the device, no extra factorisation.  out: n complex values (interleaved) for a
+ * handle of factor_mumps_cmplx_, n doubles for one of factor_mumps_.  Returns 0, or -3 for an unknown handle or a handle
+ * routed to the band kernels (half-bandwidth <= 104 without HMCMT_SHIM_SOLVER=mf: they keep no multifrontal factor).
+ * Repeated calls give bit-identical results; later solves with the handle are unchanged. */
+int64_t hmcmt_factor_inverse_diag(const int64_t* handle, double* out);
+/* debug: real flop counts of a multifrontal handle (padded front sizes, Symbolic::flops / selinvFlops): flops[0] the
+ * factorisation, flops[1] the selected inversion of hmcmt_factor_inverse_diag.  -3 for an unknown or band-routed handle. */
+int64_t hmcmt_debug_factor_flops(const int64_t* handle, double* flops);
 
 /* ----------------------------------------------------------------------------------------------
  * Level 2: fused MT2D forward + adjoint + HMC entry points
@@ -222,6 +231,16 @@ int hmcmt_gn_eig(hmcmt_plan* plan, int32_t k, int32_t r, const double* omega, do
  * z, out: [nChains][ns][nAC]; z standard normal, not clipped.  The bounds are not applied.  The chain state is untouched.
  * -3 without a decomposition (hmcmt_gn_eig), ns < 1 or NULL z / out. */
 int hmcmt_laplace_sample(hmcmt_plan* plan, int32_t ns, const double* z, double* out);
+/* Variances of the prior and of the Laplace approximation, and the resolution diagonal, per cell (in ln sigma):
+ *   prior_var  [nAC]          diag((beta Wm)^{-1});
+ *   post_var   [nChains][nAC] diag(M^{-1}) = diag(Wm^{-1}) / beta - sum_j d_j V_ij^2   (M = beta Wm + H_k of hmcmt_gn_eig);
+ *   resolution [nChains][nAC] diag(V D V^T beta Wm) = sum_j d_j V_ij (beta Wm V)_ij      (R = M^{-1} H_k, d = lambda / (1 + lambda)).
+ * diag(Wm^{-1}) is computed once per plan by a selected inversion of the resident multifrontal factor of Wm and kept on the plan
+ * (nAC doubles); j is summed in order, so results repeat bit for bit and a chain's result does not depend on the other chains.
+ * Any of the three pointers may be NULL.  The chain state, mass matrix kind, fields, factors and predictions are untouched; the
+ * bounds are not applied.  On a frequency-sharded plan the decomposition inherits hmcmt_gn_eig's caveat (the rank's partial sums).
+ * -3 for beta <= 0, all three pointers NULL, or post_var / resolution without a decomposition; -40 if Wm is not positive definite. */
+int hmcmt_posterior_variance(hmcmt_plan* plan, double* prior_var, double* post_var, double* resolution);
 
 /* compDataGradient(mtMesh,mtData,invParam,hmcprior)  HMCSampler.jl:277-330:
  * m -> pred [nChains][nData] complex, phi_d [nChains], grad [nChains][nAC] (w.r.t. log conductivity,
